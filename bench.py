@@ -2,6 +2,7 @@
 """Headline benchmark: Leduc transitions/sec of the fused NFSP rollout (env step + NFSP act + memories).
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
+    python bench.py --steps K --warmup W --dump-outputs DIR  # the same, and what its last timed step computed -> DIR/*.npy
     python bench.py --impl reference --steps K --warmup W    # CPU arm: the REFERENCE's own Python (leduc.newenv +
                                                              # main.train + Agent.play + both memories) on all host cores
 
@@ -235,6 +236,72 @@ def parity_check(nfsp_b200, dev, game0):
                               "debug and production launch"}
 
 
+DUMP_RL_ROWS, DUMP_SL_ROWS, DUMP_GAMES, DUMP_SEED = 1 << 18, 1 << 17, 1 << 18, 7  # 42 MB of float64 in all
+DUMP_MAX_BYTES = 64 << 20
+
+
+def mark_last_step(sp):
+    """Called before the last timed step, outside its timer.  Notes where the step's tickets start in every memory, and
+    fills the SL staging areas with -1 (no record has that first word: an observation is a 30-bit mask), because the
+    step's insert launch clears the per-segment counts that would otherwise tell its staged records from older ones."""
+    for st in sp.stage_sl:
+        st.fill_(-1)
+    return {"rl": [int(m.total.item()) for m in sp.rl], "sl": [int(m.total.item()) for m in sp.sl]}
+
+
+def canonical_sample(recs, rows, seed):
+    """int32 [m, 4] records -> a host array of at most `rows` of them, independent of the order the kernels appended them
+    in: sorted by their four words, then a fixed, seeded choice of positions."""
+    import torch
+
+    order = torch.arange(recs.shape[0], device=recs.device)
+    for k in (3, 2, 1, 0):  # least significant word first: stable passes give the lexicographic order
+        key = recs[order, k].to(torch.int64) & 0xFFFFFFFF
+        order = order[torch.sort(key, stable=True).indices]
+    if order.numel() > rows:
+        pick = torch.randperm(order.numel(), generator=torch.Generator().manual_seed(seed))[:rows].sort().values
+        order = order[pick.to(order.device)]
+    return recs[order].cpu().numpy()
+
+
+def dump_outputs(sp, mark, out_dir):
+    """What the last timed step handed its caller, as float64 .npy files (every field is exact in float64):
+      rl_records_p{0,1}  [rows, 7] s, s2, r, a, t, player, flags of the RL records the step wrote into player p's ring
+      sl_records_p{0,1}  [rows, 4] s, a[0..2] of the SL records the step moved into player p's reservoir
+      game_words         [DUMP_GAMES, 3] game id, low and high 32 bits of its packed state after the step
+      stats              [16] the rollout counters (cumulative since the SelfPlay was built)
+    Records are sorted and sampled by canonical_sample: the order in which warps append them changes from run to run,
+    the set does not.  Which of the SL records a reservoir keeps depends on that order, so the reservoirs' slots are not
+    dumped."""
+    import numpy as np
+    import torch
+
+    from nfsp_b200.batched import RL_DT, SL_DT
+
+    os.makedirs(out_dir, exist_ok=True)
+    out = {}
+    for p in range(2):
+        ring = sp.rl[p]
+        slots = torch.arange(mark["rl"][p], int(ring.total.item()), device=ring.store.device) % ring.capacity
+        r = canonical_sample(ring.data[slots], DUMP_RL_ROWS, DUMP_SEED + p).view(RL_DT).reshape(-1)
+        out["rl_records_p%d" % p] = np.stack([r[f].astype(np.float64) for f in RL_DT.names], axis=1)
+        st = sp.stage_sl[p]
+        staged = st[st[:, 0] != -1]
+        if staged.shape[0] != int(sp.sl[p].total.item()) - mark["sl"][p]:
+            raise RuntimeError("staged SL records of the last step do not match the reservoir's ticket count")
+        s = canonical_sample(staged, DUMP_SL_ROWS, DUMP_SEED + 2 + p).view(SL_DT).reshape(-1)
+        out["sl_records_p%d" % p] = np.concatenate([s["s"].astype(np.float64)[:, None], s["a"].astype(np.float64)], axis=1)
+    words = sp.env.state_words().cpu().numpy().view(np.uint32).reshape(-1, 2)
+    games = np.sort(np.random.default_rng(DUMP_SEED).choice(len(words), min(DUMP_GAMES, len(words)), replace=False))
+    out["game_words"] = np.concatenate([games[:, None], words[games]], axis=1).astype(np.float64)
+    out["stats"] = sp.stats.cpu().numpy().astype(np.float64)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError("dump of %d bytes exceeds %d" % (total, DUMP_MAX_BYTES))
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def workload_config():
     return {"workload": "nfsp_rollout: %d games/GPU x %d decisions per step, eta=%.2f eps=%.2f, 4 acting nets 30-64-3, "
                         "ring %d + reservoir %d records per player, sample %d" %
@@ -378,7 +445,14 @@ def run_gpu(args):
     if rank == 0:
         sampler.start()
     barrier()
-    tot_ms, ker_ms = timed_steps(args.steps, False)
+    if args.dump_outputs and rank == 0:  # every step ends in a synchronise: timing the last one on its own changes nothing
+        tot_ms, ker_ms = timed_steps(args.steps - 1, False)
+        mark = mark_last_step(sp)
+        last_tot, last_ker = timed_steps(1, False)
+        tot_ms, ker_ms = tot_ms + last_tot, ker_ms + last_ker
+        dump_outputs(sp, mark, args.dump_outputs)  # before the e2e steps write into the same memories
+    else:
+        tot_ms, ker_ms = timed_steps(args.steps, False)
     barrier()
     t_e2e, _ = timed_steps(max(1, min(args.warmup, 2)), True)  # e2e warm-up (pinned buffers, sample kernels)
     barrier()
@@ -680,7 +754,11 @@ def main():
     ap.add_argument("--variant", default="default", choices=["default", "states", "cuda", "pairs", "sorted", "tcgen05", "tcgen05_ws"],
                     help="rollout kernel: table of the nets' outputs per decision state (default), per-decision CUDA-core row sums, "
                          "net-sorted warp groups, tcgen05 tensor-core tiles")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float64; rank 0's games)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)

@@ -1,6 +1,6 @@
-"""-m "not gpu": the CPU legs of bench.py run the REFERENCE'S OWN files (oracle/ref_timing.py).  Here: the copy that travels
-to the GPU box (baseline/_ref) is byte-identical to /root/reference where that tree exists, and both drivers play hands and
-count transitions as the reference's own counters do."""
+"""-m "not gpu": the CPU legs of bench.py run the REFERENCE'S OWN files (oracle/ref_timing.py).  Here: materialise() copies
+the files the drivers execute verbatim (into the git-ignored baseline/_ref), and, where the reference's files are present,
+both drivers play hands and count transitions as the reference's own counters do."""
 import filecmp
 import os
 
@@ -9,13 +9,16 @@ import pytest
 from oracle import ref_timing
 
 
-def test_travelling_copy_is_verbatim():
-    src = "/root/reference"
-    if not os.path.isfile(os.path.join(src, "leduc", "newenv.py")):
-        pytest.skip("no reference tree on this machine (the GPU box): the copy under baseline/_ref is all there is")
-    assert ref_timing.materialise()
+def test_travelling_copy_is_verbatim(tmp_path):
+    src, dst = tmp_path / "reference", tmp_path / "copy"
+    for i, rel in enumerate(ref_timing.FILES):  # a stand-in tree: distinct bytes per file, every byte value present
+        (src / rel).parent.mkdir(parents=True, exist_ok=True)
+        (src / rel).write_bytes(bytes((i + k) % 256 for k in range(256 * (i + 1))))
+    assert ref_timing.materialise(str(src), str(dst))
     for rel in ref_timing.FILES:
-        assert filecmp.cmp(os.path.join(src, rel), os.path.join(ref_timing.REF_COPY, rel), shallow=False), rel
+        assert filecmp.cmp(os.path.join(src, rel), os.path.join(dst, rel), shallow=False), rel
+    assert not ref_timing.materialise(str(tmp_path / "absent"), str(tmp_path / "copy2"))
+    assert not (tmp_path / "copy2").exists()
 
 
 @pytest.mark.parametrize("kind", ["legacy", "nfsp"])

@@ -1,6 +1,7 @@
 """world_size-2 gloo test (CPU) of the multi-GPU host logic: contiguous game sharding, the counter
 all-reduce and max-over-ranks timing.  The data path itself has no collective (SURVEY 8e)."""
 import os
+import socket
 import sys
 
 import pytest
@@ -29,7 +30,10 @@ def _worker(rank, world, port, q):
 
 
 def test_sharding_two_ranks():
-    world, port = 2, 29611
+    with socket.socket() as s:  # a port nobody holds now: suites running side by side on one host must not collide
+        s.bind(("127.0.0.1", 0))
+        port = s.getsockname()[1]
+    world = 2
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     ps = [ctx.Process(target=_worker, args=(r, world, port, q)) for r in range(world)]
