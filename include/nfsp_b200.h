@@ -98,6 +98,9 @@ int nfsp_fsm_image(uint32_t *out, int capacity_words);
 /* The same for the legacy rules (leduc/env.py README iteration; layout in csrc/legacy_fsm.cuh); *n_rows receives the
  * number of states a rollout can reach. */
 int nfsp_legacy_fsm_image(uint32_t *out, int capacity_words, int *n_rows);
+/* The image the default rollout (variant 6) steps its games on (layout in csrc/nfsp_fsm.cuh, "the fused rollout's
+ * image"; addresses are byte offsets from the state table it follows); returns its size in words. */
+int nfsp_rollout_image(uint32_t *out, int capacity_words);
 /* newenv.Env.do_action (newenv.py:131-178) called on its own, for callers that drive the pieces of step() themselves:
  * raise->call coercions, history bit, round_raises, chips, last_action -- no snapshot, no round change, no showdown,
  * `terminated` untouched.  d_actions int8[n]: np.argmax(action), 3 = all-zero vector (argmax 0 = fold), negative =

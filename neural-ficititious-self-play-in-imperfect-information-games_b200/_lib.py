@@ -21,7 +21,7 @@ SYMBOLS = [
     "nfsp_version", "nfsp_last_error", "nfsp_device_info",
     "nfsp_env_create", "nfsp_env_destroy", "nfsp_env_num_games", "nfsp_env_rules", "nfsp_env_step_counter",
     "nfsp_env_set_step_counter", "nfsp_env_state_ptr", "nfsp_env_kernel_error", "nfsp_env_save_state", "nfsp_env_load_state",
-    "nfsp_env_reset", "nfsp_env_set_hands", "nfsp_env_step", "nfsp_env_do_action", "nfsp_fsm_image", "nfsp_legacy_fsm_image", "nfsp_env_observe", "nfsp_env_export",
+    "nfsp_env_reset", "nfsp_env_set_hands", "nfsp_env_step", "nfsp_env_do_action", "nfsp_fsm_image", "nfsp_legacy_fsm_image", "nfsp_rollout_image", "nfsp_env_observe", "nfsp_env_export",
     "nfsp_legacy_reset", "nfsp_legacy_set_hands", "nfsp_legacy_step", "nfsp_legacy_get_new_state",
     "nfsp_legacy_rollout", "nfsp_legacy_export",
     "nfsp_expand_obs",
@@ -111,6 +111,7 @@ def lib():
     L.nfsp_env_do_action.argtypes = [vp, i8p, i8p, i8p, vp]
     L.nfsp_fsm_image.argtypes = [vp, C.c_int]
     L.nfsp_legacy_fsm_image.argtypes = [vp, C.c_int, vp]
+    L.nfsp_rollout_image.argtypes = [vp, C.c_int]
     L.nfsp_env_observe.argtypes = [vp, i8p, C.c_int, vp, vp, vp, vp, vp, vp]
     L.nfsp_env_export.argtypes = [vp, vp, vp]
     L.nfsp_legacy_reset.argtypes = [vp, vp]

@@ -203,6 +203,8 @@ extern "C" int nfsp_act_set_weights(nfsp_env_t h, const float *d_weights, void *
         if (rc != NFSP_OK) return rc;
         rc = nfsp_rollout_states_configure();
         if (rc != NFSP_OK) return rc;
+        rc = nfsp_states_upload_image(h->d_states);
+        if (rc != NFSP_OK) return rc;
     }
     pack_images_kernel<<<(kPackFloats + kTabImageFloats + 4 * NFSP_NET_PARAMS + 255) / 256, 256, 0, (cudaStream_t)stream>>>(d_weights, h->d_wpack);
     NFSP_LAUNCH_CHECK();

@@ -89,43 +89,67 @@ __host__ __device__ inline uint32_t p_word(uint32_t p, uint32_t c0, uint32_t c1,
 
 // The whole image; addresses (nx, the first row of a hand) are byte offsets into it -- a CTA adds the shared-memory
 // address of its copy (is_address() says which words).
+// newenv.Env.step from (dealer, sigma, raw action): what both images (K1's and the rollout's) are built from
+struct Move {
+    uint32_t s, r, t, q, av, kind, add, hbit, tt_new, sigma_new;
+    uint32_t fin0;  // the round-0 sequence a step into round 1 finishes (0 otherwise)
+    bool term, pass;
+};
+inline Move move_of(uint32_t d, uint32_t sigma, uint32_t raw) {
+    Move m;
+    m.r = sigma >= 9u ? 1u : 0u;
+    m.s = sigma - 9u * m.r;
+    const uint32_t k = seq_actions(m.s);
+    m.t = 3u * m.r + k;
+    m.q = d ^ (k & 1u);
+    m.av = raw;
+    if (m.av == A_RAISE && m.s >= 3u) m.av = A_CALL;  // newenv.py:141-145: s in {4,6} are the two coercion cases
+    m.add = 0u;
+    m.hbit = 0u;
+    m.tt_new = m.t;
+    m.sigma_new = sigma;
+    m.fin0 = 0u;
+    if (m.av == A_FOLD) {
+        m.kind = KIND_FOLD;
+    } else {
+        const uint32_t s = m.s, t = m.t;
+        const bool prev_raise = s != 0u && !(s & 1u);                                        // s in {2,4,6}
+        m.add = (m.av == A_RAISE ? 2u : 0u) + (prev_raise ? 2u : 0u) + (t == 0u ? 1u : 0u);  // newenv.py:157-176
+        m.hbit = 1u << (12u * m.q + 2u * t + m.av - 1u);
+        const uint32_t sn = s < 3u ? 2u * s + m.av : 5u + (s >> 1);
+        const bool over = s >= 3u || (s != 0u && m.av == A_CALL);                             // newenv.py:180-190
+        if (!over) { m.kind = KIND_PASS; m.tt_new = t + 1u; m.sigma_new = 9u * m.r + sn; }
+        else if (m.r == 0u) { m.kind = KIND_ROUND; m.tt_new = 3u; m.sigma_new = 9u; }         // newenv.py:215-242
+        else { m.kind = KIND_SHOWDOWN; m.tt_new = t + 1u; }                                   // newenv.py:261-298
+        if (m.kind == KIND_ROUND) m.fin0 = (sn >> 1) - 1u;  // 0 CC, 1 RC, 2 CRC, 3 RRC
+    }
+    m.term = m.kind >= KIND_SHOWDOWN;
+    m.pass = !m.term && (m.kind == KIND_PASS || m.q != d);  // round 1 opens with the dealer
+    return m;
+}
+
+// The whole image; addresses (nx, the first row of a hand) are byte offsets into it -- a CTA adds the shared-memory
+// address of its copy (is_address() says which words).
 inline void build_image(uint32_t *img) {
     for (int i = 0; i < kImageWords; ++i) img[i] = 0u;
     for (uint32_t d = 0; d < 2; ++d)
         for (uint32_t sigma = 0; sigma < 18; ++sigma) {
-            const uint32_t r = sigma >= 9u ? 1u : 0u, s = sigma - 9u * r;
             uint32_t *row = img + (kFsmOff + (int)(d * 18u + sigma) * kRowBytes) / 4;
-            if (s >= 7u) continue;  // [C,R,C] / [R,R,C] end the round: never a state to act in
-            const uint32_t k = seq_actions(s), t = 3u * r + k, q = d ^ (k & 1u);
-            row[kInfoOff / 4] = t | (q << 4);
+            if (sigma % 9u >= 7u) continue;  // [C,R,C] / [R,R,C] end the round: never a state to act in
+            const Move m0 = move_of(d, sigma, 0u);
+            row[kInfoOff / 4] = m0.t | (m0.q << 4);
             for (uint32_t raw = 0; raw < 3; ++raw) {
+                const Move m = move_of(d, sigma, raw);
                 uint32_t *e = row + raw * (kEntryBytes / 4);
-                uint32_t av = raw;
-                if (av == A_RAISE && s >= 3u) av = A_CALL;  // newenv.py:141-145: s in {4,6} are the two coercion cases
-                uint32_t kind, add = 0u, hbit = 0u, tt_new = t, sigma_new = sigma;
-                if (av == A_FOLD) {
-                    kind = KIND_FOLD;
-                } else {
-                    const bool prev_raise = s != 0u && !(s & 1u);                                  // s in {2,4,6}
-                    add = (av == A_RAISE ? 2u : 0u) + (prev_raise ? 2u : 0u) + (t == 0u ? 1u : 0u);  // newenv.py:157-176
-                    hbit = 1u << (12u * q + 2u * t + av - 1u);
-                    const uint32_t sn = s < 3u ? 2u * s + av : 5u + (s >> 1);
-                    const bool over = s >= 3u || (s != 0u && av == A_CALL);                         // newenv.py:180-190
-                    if (!over) { kind = KIND_PASS; tt_new = t + 1u; sigma_new = 9u * r + sn; }
-                    else if (r == 0u) { kind = KIND_ROUND; tt_new = 3u; sigma_new = 9u; }             // newenv.py:215-242
-                    else { kind = KIND_SHOWDOWN; tt_new = t + 1u; }                                   // newenv.py:261-298
-                }
-                const bool term = kind >= KIND_SHOWDOWN;
-                const bool pass = !term && (kind == KIND_PASS || q != d);  // round 1 opens with the dealer
-                const uint32_t r_new = tt_new >= 3u ? 1u : 0u;
-                e[0] = hbit | ((r == 1u || kind == KIND_ROUND) ? kCm1 : kCm0) | ((uint32_t)term << 30) | (q << 31);
-                e[1] = (add << 2) | (add << 8) | (raw << 13) | (1u << 15) | (t << 16);
-                e[2] = pass ? 0xFFFFFFFFu : 0u;
-                e[3] = (uint32_t)(kFsmOff + (int)(term ? term_row(kind, tt_new, q) : d * 18u + sigma_new) * kRowBytes);
-                e[4] = raw | (av << 2) | (r_new << 4) | (r_new << 12);
-                e[5] = add << (13u + 4u * q);
-                e[6] = kind == KIND_FOLD ? 0x3Cu : (kind == KIND_SHOWDOWN ? 0xC0u : 0u);
-                e[7] = kind == KIND_SHOWDOWN ? 0xF00u : 0u;
+                const uint32_t r_new = m.tt_new >= 3u ? 1u : 0u;
+                e[0] = m.hbit | ((m.r == 1u || m.kind == KIND_ROUND) ? kCm1 : kCm0) | ((uint32_t)m.term << 30) | (m.q << 31);
+                e[1] = (m.add << 2) | (m.add << 8) | (raw << 13) | (1u << 15) | (m.t << 16);
+                e[2] = m.pass ? 0xFFFFFFFFu : 0u;
+                e[3] = (uint32_t)(kFsmOff + (int)(m.term ? term_row(m.kind, m.tt_new, m.q) : d * 18u + m.sigma_new) * kRowBytes);
+                e[4] = raw | (m.av << 2) | (r_new << 4) | (r_new << 12);
+                e[5] = m.add << (13u + 4u * m.q);
+                e[6] = m.kind == KIND_FOLD ? 0x3Cu : (m.kind == KIND_SHOWDOWN ? 0xC0u : 0u);
+                e[7] = m.kind == KIND_SHOWDOWN ? 0xF00u : 0u;
             }
         }
     for (uint32_t kind = KIND_SHOWDOWN; kind <= KIND_FOLD; ++kind)
@@ -168,6 +192,104 @@ __host__ __device__ inline bool is_address(int w) {
     return v >= kPolOff / 4 && (v & 3) == 3;
 }
 
+// ---- the fused rollout's image (rollout_states_kernel) ---------------------------------------------------------------
+// The same rows (dealer, sigma) and entries (row, raw action), every word used as loaded, with what a decision of the
+// rollout needs beside the game step (32 bytes an entry):
+//   hc, pm, nx  as above
+//   pa     as above without the non-zero flag: the decision sets it (bit 15 of the state table's fourth word)
+//   ds     change of the state-table offset 16 * (fin0 * 18 + sigma), fin0 = the finished round-0 sequence (round 1)
+//   mx     raw | effective action << 2 | round after the step << 4 | 1 << 8 | the same round << 12 | q << 16: & 0x10103 is
+//          the last word of the actor's terminal RL record, & 0x101F the per-step part of trace word 3
+//   rm     mask of (PA & 0xFF) | (PO & 0xF00) giving the reward word's byte offset: fold 0x3C, showdown 0xFFC, else 0
+//   inc    1 << 5 * (3q + raw): the step's count in the action histogram
+// Terminal pseudo-rows keep only their info word, 16 bytes apart (a row address is its info word's minus kInfoOff).
+// A deal entry holds both players' P words (bit 23 set in player 1's) and both state-table offsets without the policy,
+// 16 * (2 * player * 1296 + card * 432 + pub * 144 + dealer * 72); a policy entry the policy bits and 16 * 1296 * policy
+// per player.  A dealer's deal table is as long as its rows, so its first row is at dl - kRDealOff.  Reward word: index
+// fold chips | showdown result << 4 | opponent chips << 6, the actor's half chips in byte 0 and the other player's in
+// byte 1 (int8).
+// Addresses are byte offsets from the state table, which the image follows `at` bytes later in shared memory.
+constexpr uint32_t kPPlayer = 1u << 23;  // rollout P words: this is player 1
+constexpr int kNetSlots = 72 * 18;       // state-table slots per net (rollout_states.cu)
+constexpr int kRTermOff = kLiveRows * kRowBytes;                // 4032
+constexpr int kRDealOff = kRTermOff + kTermRows * 16;           // 4288
+constexpr int kRDealHalf = 18 * kRowBytes;                      // 2016
+constexpr int kRRewardOff = kRDealOff + 2 * kRDealHalf;         // 8320
+constexpr int kRImageBytes = kRRewardOff + 4 * kRewardWords;    // 12416
+constexpr int kRImageWords = kRImageBytes / 4;
+static_assert(kPolOff + 4 * 16 <= kRDealHalf, "a dealer's deal and policy entries fit beside its rows' stride");
+
+__host__ __device__ inline uint32_t state_offset(uint32_t net, uint32_t card, uint32_t pub, uint32_t dealer, uint32_t fin0,
+                                                 uint32_t sigma) {
+    return 16u * (net * (uint32_t)kNetSlots + ((((card * 3u + pub) * 2u + dealer) * 4u + fin0) * 18u + sigma));
+}
+
+inline void build_rollout_image(uint32_t *img, uint32_t at) {
+    for (int i = 0; i < kRImageWords; ++i) img[i] = 0u;
+    for (uint32_t d = 0; d < 2; ++d)
+        for (uint32_t sigma = 0; sigma < 18; ++sigma) {
+            uint32_t *row = img + (int)(d * 18u + sigma) * kRowBytes / 4;
+            if (sigma % 9u >= 7u) continue;
+            const Move m0 = move_of(d, sigma, 0u);
+            row[kInfoOff / 4] = m0.t | (m0.q << 4);
+            for (uint32_t raw = 0; raw < 3; ++raw) {
+                const Move m = move_of(d, sigma, raw);
+                uint32_t *e = row + raw * (kEntryBytes / 4);
+                const uint32_t r_new = m.tt_new >= 3u ? 1u : 0u;
+                const uint32_t g_new = m.term ? sigma : m.fin0 * 18u + m.sigma_new;  // fin0 is 0 until round 1 starts
+                e[0] = m.hbit | ((m.r == 1u || m.kind == KIND_ROUND) ? kCm1 : kCm0) | ((uint32_t)m.term << 30) | (m.q << 31);
+                e[1] = (m.add << 2) | (m.add << 8) | (raw << 13) | (m.t << 16);
+                e[2] = m.pass ? 0xFFFFFFFFu : 0u;
+                e[3] = at + (m.term ? (uint32_t)(kRTermOff + 16 * ((int)term_row(m.kind, m.tt_new, m.q) - kLiveRows) - kInfoOff)
+                                    : (d * 18u + m.sigma_new) * (uint32_t)kRowBytes);
+                e[4] = 16u * (g_new - sigma);  // within round 1 fin0 does not change
+                e[5] = raw | (m.av << 2) | (r_new << 4) | (1u << 8) | (r_new << 12) | (m.q << 16);
+                e[6] = m.kind == KIND_FOLD ? 0x3Cu : (m.kind == KIND_SHOWDOWN ? 0xFFCu : 0u);
+                e[7] = 1u << (5u * (3u * m.q + raw));
+            }
+        }
+    for (uint32_t kind = KIND_SHOWDOWN; kind <= KIND_FOLD; ++kind)
+        for (uint32_t tt = (kind == KIND_FOLD ? 0u : 5u); tt <= (kind == KIND_FOLD ? 5u : 6u); ++tt)
+            for (uint32_t q = 0; q < 2; ++q)
+                img[(kRTermOff + 16 * ((int)term_row(kind, tt, q) - kLiveRows)) / 4] = tt | (q << 4) | (kind << 8) | (1u << 16);
+    for (uint32_t d = 0; d < 2; ++d) {
+        uint32_t *half = img + (kRDealOff + (int)d * kRDealHalf) / 4;
+        for (uint32_t idx = 0; idx < (uint32_t)kDealEntries; ++idx) {
+            const uint32_t c = deal_ranks_h(idx), c0 = c & 3u, c1 = (c >> 2) & 3u, pub = (c >> 4) & 3u;
+            const uint32_t b0 = d == 0u ? 1u : 2u, b1 = d == 0u ? 2u : 1u;
+            const uint32_t P0 = p_word(0, c0, c1, pub, b0, 0, 0, 0, 7), P1 = p_word(1, c0, c1, pub, b1, 0, 0, 0, 7) | kPPlayer;
+            half[4 * idx + 0] = d ? P1 : P0;
+            half[4 * idx + 1] = d ? P0 : P1;
+            half[4 * idx + 2] = state_offset(2u * d, d ? c1 : c0, pub, d, 0u, 0u);
+            half[4 * idx + 3] = state_offset(2u * (d ^ 1u), d ? c0 : c1, pub, d, 0u, 0u);
+        }
+        for (uint32_t pw = 0; pw < 4; ++pw) {
+            uint32_t *e = half + kPolOff / 4 + 4 * pw;
+            const uint32_t pol0 = pw & 1u, pol1 = pw >> 1, pa = d ? pol1 : pol0, po = d ? pol0 : pol1;
+            e[0] = pa << 12;
+            e[1] = po << 12;
+            e[2] = pa * 16u * (uint32_t)kNetSlots;
+            e[3] = po * 16u * (uint32_t)kNetSlots;
+        }
+    }
+    uint32_t *rew = img + kRRewardOff / 4;
+    for (int i = 0; i < kRewardWords; ++i) {
+        const int ba = i & 15, sd = (i >> 4) & 3, bo = i >> 6;
+        int ra = 0, ro = 0;
+        if (bo == 0 && sd == 0) { ra = -ba; ro = ba; }      // fold: newenv.py:252-255
+        else if (sd == 1) { ra = bo; ro = -ba; }            // showdown won by the actor
+        else if (sd == 2) { ra = -bo; ro = ba; }            // lost; drawn: 0
+        rew[i] = (uint32_t)(uint8_t)(int8_t)ra | (uint32_t)(uint8_t)(int8_t)ro << 8;
+    }
+}
+// word w of the rollout image holds an offset that becomes a shared-memory address
+__host__ __device__ inline bool is_rollout_address(int w) {
+    if (w < kRTermOff / 4) return (w % (kRowBytes / 4)) < 24 && ((w % (kRowBytes / 4)) & 7) == 3;
+    if (w < kRDealOff / 4 || w >= kRRewardOff / 4) return false;
+    const int v = (w - kRDealOff / 4) % (kRDealHalf / 4);
+    return v < kPolOff / 4 && (v & 3) >= 2;
+}
+
 #ifdef __CUDACC__
 __device__ __forceinline__ uint4 lds128(uint32_t a) {
     uint4 v;
@@ -179,8 +301,9 @@ __device__ __forceinline__ uint32_t lds32(uint32_t a) {
     asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a));
     return v;
 }
-// One game in registers for the steps of a launch.
-struct Game {
+// One game in registers for the steps of a launch; kDeal / kHalf: where the image keeps the deal tables.
+template <int kDeal, int kHalf>
+struct GameAt {
     uint32_t HX;   // history (0-23) | card mask of the round (24-29) | hand over (30) | actor of the last step (31)
     uint32_t PA, PO;  // words of the player to act / the other one; swap when the turn passes
     uint32_t ms;   // trace word 3: dealer, cards, policies, both players' chips
@@ -204,13 +327,13 @@ struct Game {
         ms = (d << 5) | (c0 << 6) | (c1 << 8) | (pub << 10) | (g.bets(0) << 13) | (g.bets(1) << 17) | (g.policy(0) << 22) |
              (g.policy(1) << 23);
         tix = base + (uint32_t)kFsmOff + (d * 18u + (over ? 0u : 9u * r + seq)) * (uint32_t)kRowBytes;
-        dl = base + (uint32_t)kDealOff + d * (uint32_t)kDealHalf;
+        dl = base + (uint32_t)kDeal + d * (uint32_t)kHalf;
     }
 
     __device__ __forceinline__ uint64_t pack(uint32_t base) const {
         const uint32_t info = lds32(tix + (uint32_t)kInfoOff);
         const uint32_t tt = info & 7u, q = (info >> 4) & 1u, kind = (info >> 8) & 3u, over = (info >> 16) & 1u;
-        const uint32_t d = dl != base + (uint32_t)kDealOff ? 1u : 0u;
+        const uint32_t d = dl != base + (uint32_t)kDeal ? 1u : 0u;
         const uint32_t P0 = q ? PO : PA, P1 = q ? PA : PO;
         const uint32_t r = tt >= 3u ? 1u : 0u, k = tt - 3u * r;
         const uint32_t sd = (PA >> 6) & 3u;  // PA is the actor of the terminating step
@@ -222,6 +345,31 @@ struct Game {
                             (((P1 >> 13) & 3u) << 16) | (((P0 >> 15) & 1u) << 18) | (((P1 >> 15) & 1u) << 19) |
                             (((P0 >> 16) & 7u) << 20) | (((P1 >> 16) & 7u) << 23) | ((over ? q : 0u) << 26) | (oc << 27);
         return (uint64_t)lo | ((uint64_t)hi << 32);
+    }
+};
+using Game = GameAt<kDealOff, kDealHalf>;
+
+// The rollout's game: the snapshots s[p] (newenv.py:200-202) and the players' state-table addresses at the current row
+// (FA + 16 * slot of this row's (fin0, sigma) is added as the game moves: entry word ds) beside the words of Game; all
+// per-player registers swap with the turn.  ibase / sbase: shared-memory addresses of the image / the state table.
+struct RolloutGame : GameAt<kRDealOff, kRDealHalf> {
+    uint32_t SA, SO, FA, FO;
+
+    __device__ __forceinline__ void unpack(uint64_t w, uint32_t ibase, uint32_t sbase) {
+        GameAt<kRDealOff, kRDealHalf>::unpack(w, ibase);
+        const NfspW g{w};
+        const uint32_t H = g.hist(), both = H | (H >> 12), r = g.round(), d = g.dealer(), q = (uint32_t)g.to_act();
+        const auto seq = [](uint32_t rnd) {
+            const uint32_t s0 = rnd & 3u, s1 = (rnd >> 2) & 3u, s2 = (rnd >> 4) & 3u;
+            return s2 ? 6u + s0 : (s1 ? 2u * s0 + s1 : s0);
+        };
+        const uint32_t fin0 = r ? (seq(both & 63u) >> 1) - 1u : 0u, sigma = r ? 9u + seq((both >> 6) & 63u) : seq(both & 63u);
+        PA |= q ? kPPlayer : 0u;
+        PO |= q ? 0u : kPPlayer;
+        FA = sbase + state_offset(2u * q + g.policy((int)q), g.card((int)q), g.pub(), d, fin0, sigma);
+        FO = sbase + state_offset(2u * (q ^ 1u) + g.policy((int)(q ^ 1u)), g.card((int)(q ^ 1u)), g.pub(), d, fin0, sigma);
+        SA = g.snapshot((int)q);
+        SO = g.snapshot((int)(q ^ 1u));
     }
 };
 #endif  // __CUDACC__

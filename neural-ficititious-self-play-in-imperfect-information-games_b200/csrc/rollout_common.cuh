@@ -26,6 +26,7 @@ int nfsp_rollout_pairs_configure();
 int nfsp_rollout_states_launch(nfsp_env_t h, const nfsp::RolloutArgs &A, const nfsp_rollout_io *io, bool debug, cudaStream_t st);
 int nfsp_states_ensure(nfsp_env_t h, const float *d_tab, float *d_states, cudaStream_t st);
 int nfsp_states_floats();
+int nfsp_states_upload_image(float *d_states);
 int nfsp_rollout_states_configure();
 
 namespace nfsp {

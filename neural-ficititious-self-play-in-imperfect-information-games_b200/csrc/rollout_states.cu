@@ -6,15 +6,16 @@
 // pure function of the observation, so its three outputs on all of them -- computed by states_pack_kernel from the SAME
 // table image and with the same operations as variant 1 (two rows added, relu, FFMA2 second layer, head; the 16
 // hidden-unit quads summed in four interleaved groups) every time the weights change -- stand for the 8.4 M forwards
-// of a 2^20-game x 8-step launch.  A decision then costs ONE 16-byte shared-memory read instead of variant 1's 80 (32
-// row quads + 48 W2 quads, which bound that kernel: an LDS.128 holds the pipe for four cycles), and what is left is the
-// game logic, Philox and the record append.
+// of a 2^20-game x 8-step launch.  A decision then costs ONE 16-byte shared-memory read instead of variant 1's 80.
 //
-// The decision logic around the forward -- fast_begin / fast_decide, block ownership, the counters -- is variant 1's, so
-// the records, game words and counters are those of variant 1 run on the same score vectors; the score vectors differ
-// from variant 1's only by the summation order of a lane's rotation (held to 1e-5 of the CPU restatement in
-// tests/test_gpu_act.py and tests/test_gpu_baseline_sizes.py).  The append is this kernel's own: warp-private buffers
-// in shared memory (below).
+// What is left is the game logic, Philox and the record append, and the game logic runs on the state machine of the
+// env-only kernel (nfsp_fsm.cuh, the rollout image): a step is two 16-byte reads of the entry (row, raw action) whose
+// words are used as loaded -- no field extraction, no index formula for the state table (each player carries its
+// address, moved by the entry).  The records, game words and counters are those of variant 1 run on the same score
+// vectors; the score vectors differ from variant 1's only by the summation order of a lane's rotation (held to 1e-5 of
+// the CPU restatement in tests/test_gpu_act.py and tests/test_gpu_baseline_sizes.py).  The append is this kernel's own:
+// warp-private buffers in shared memory (below).
+#include "nfsp_fsm.cuh"
 #include "rollout_fast.cuh"
 #include "rollout_tables.cuh"
 #include "ptx_helpers.cuh"
@@ -26,9 +27,18 @@ namespace nfsp {
 // the public card and has no finished sequence yet (f = 0), so its 54 states are stored once per public card; slots with
 // round 0 and f != 0 are never read.  702 distinct states in 72 * 18 = 1 296 slots per net.
 constexpr int kNetStates = 72 * 18;
-constexpr int kStateQuads = 4 * kNetStates;      // one float4 {o0, o1, o2, argmax | non-zero << 2} per net and slot
+constexpr int kStateQuads = 4 * kNetStates;      // one float4 {o0, o1, o2, action word} per net and slot
 constexpr int kStateBytes = kStateQuads * 16;    // 82 944
 static_assert(kStateBytes % 16 == 0, "bulk copies move multiples of 16 bytes");
+static_assert(kNetStates == fsm::kNetSlots, "the rollout image addresses this table");
+
+// action word of a score vector: np.argmax (first maximum) * the entry size (the entry's offset in its row) | the
+// non-zero flag (np.average != 0, agent.py:134) at its bit in the P word
+__device__ __forceinline__ uint32_t score_word(float v0, float v1, float v2) {
+    const uint32_t an = score_action(v0, v1, v2);
+    return (an & 3u) * (uint32_t)fsm::kEntryBytes | (an >> 2) << 15;
+}
+constexpr uint32_t kWordEntry = 0x60u, kWordNz = 1u << 15;
 
 // table slot -> rows of the factorised first layer (the inverse of the index the rollout computes)
 __device__ __forceinline__ void state_rows(int s, uint32_t &xrow, uint32_t &yrow) {
@@ -65,7 +75,7 @@ __global__ void states_pack_kernel(const float *__restrict__ tab, float4 *__rest
     if (valid && j == 0) {
         float o0, o1, o2;
         Layer2Acc::head_of_sums(s0, s1, s2, reinterpret_cast<const float4 *>(tab + kTabFloats + kTabW2Floats)[net], net & 1u, o0, o1, o2);
-        states[e] = make_float4(o0, o1, o2, __uint_as_float(score_action(o0, o1, o2)));
+        states[e] = make_float4(o0, o1, o2, __uint_as_float(score_word(o0, o1, o2)));
     }
 }
 
@@ -79,11 +89,14 @@ constexpr int kStatesThreads = 1024, kStatesThreadsSmall = 512;
 // warp's critical path, and with the direct ring append every one of the launch's 262 144 warp-steps hits the SAME two
 // words (the rings' totals): same-address atomics retire at ~1.4 ns each, 0.37 ms per launch -- invisible beside variant
 // 1's 0.37 ms of shared-memory traffic, the bound of this kernel once the forward is a table read.  Here a warp collects
-// its records in shared memory (the table leaves 180 KB free) and claims slots for a whole buffer at a time: one atomic
-// and one coalesced copy (512 B per warp instruction) per ~100 records.
-constexpr int kBufRL = 104, kBufSL = 32;                 // records per player and warp; >= a step's worst case (64, 32)
-constexpr int kWarpBufQuads = 2 * kBufRL + 2 * kBufSL;   // 272 uint4 = 4 352 B per warp
-constexpr int states_smem_bytes(int threads) { return kStateBytes + (threads / 32) * kWarpBufQuads * 16; }
+// its records in shared memory (beside the table and the image) and claims slots for a whole buffer at a time: one
+// atomic and one coalesced copy (512 B per warp instruction) per ~100 records.  100 RL records is what the 227 KB of a
+// CTA leave at 32 warps.
+constexpr int kBufRL = 100, kBufSL = 32;                 // records per player and warp; >= a step's worst case (64, 32)
+constexpr int kWarpBufQuads = 2 * kBufRL + 2 * kBufSL;   // 264 uint4 = 4 224 B per warp
+constexpr int kImageQuads = fsm::kRImageBytes / 16;
+constexpr int states_smem_bytes(int threads) { return kStateBytes + fsm::kRImageBytes + (threads / 32) * kWarpBufQuads * 16; }
+static_assert(fsm::kRImageBytes % 16 == 0, "the warps' buffers follow the image 16-byte aligned");
 static_assert(kBufRL >= 64 && kBufSL >= 32, "a buffer must take the records of one step");
 
 // quad offsets of the four lists in a warp's buffer: RL of player 0 / 1, SL of player 0 / 1
@@ -150,19 +163,21 @@ __device__ __forceinline__ void buf_flush(WarpBuf &B, const RolloutArgs &A, cons
     __syncwarp();
 }
 
-// a step's records into the warp's buffers (what warp_append does with global atomics).  All lanes call it.
+// a step's records into the warp's buffers (what warp_append does with global atomics): the actor q's RL records A (the
+// transition it remembered before acting) and B (its terminal observation), the other player's RL record C and the
+// actor's SL record S.  All lanes call it.
 template <bool kDirect>
-__device__ __forceinline__ void buf_append(WarpBuf &B, const RolloutArgs &A, const WarpStage &W, const FastDecision &d,
-                                           const FastRecords &R, float v0, float v1, float v2, FastCounters &c) {
-    const uint32_t q = R.q;
+__device__ __forceinline__ void buf_append(WarpBuf &B, const RolloutArgs &A, const WarpStage &W, FastCounters &c, uint32_t q,
+                                           bool vA, bool vB, bool vC, bool vS, const uint4 &recA, const uint4 &recB,
+                                           const uint4 &recC, const uint4 &recS) {
     // actor-relative counts: own ring | other ring << 8 | own reservoir << 16; swapping the bytes of each half makes them
     // absolute (rl0 | rl1 << 8 | sl0 << 16 | sl1 << 24) for player 1
-    const uint32_t rel = ((uint32_t)R.vA + (uint32_t)R.vB) | (uint32_t)R.vC << 8 | (uint32_t)R.vS << 16;
+    const uint32_t rel = ((uint32_t)vA + (uint32_t)vB) | (uint32_t)vC << 8 | (uint32_t)vS << 16;
     const uint32_t mine = q ? __byte_perm(rel, 0u, 0x2301u) : rel;
     const uint32_t incl = warp_scan_bytes_p(mine);
     const uint32_t tot = __shfl_sync(0xFFFFFFFFu, incl, 31);
     // a list that cannot take this step's records is flushed first (warp-uniform, rare): byte > cap <=> bit 7 of
-    // byte + 127 - cap (no byte carries: <= 104 + 64 and <= 32 + 32)
+    // byte + 127 - cap (no byte carries: <= 100 + 64 and <= 32 + 32)
     constexpr uint32_t kOverRL = 127u - (uint32_t)kBufRL, kOverSL = 127u - (uint32_t)kBufSL;
     const uint32_t over = (B.cnt + tot + (kOverRL | kOverRL << 8 | kOverSL << 16 | kOverSL << 24)) & 0x80808080u;
     if (over) {
@@ -173,23 +188,27 @@ __device__ __forceinline__ void buf_append(WarpBuf &B, const RolloutArgs &A, con
     const uint32_t pos = B.cnt + (incl - mine);                       // absolute positions, bytewise
     const uint32_t prel = q ? __byte_perm(pos, 0u, 0x2301u) : pos;    // own ring | other ring | own reservoir
     uint32_t own = q * kOffRL1 + (prel & 0xFFu);
-    if (R.vA) B.b[own++] = make_uint4(d.snap_a, d.obs, 0u, d.meta_a);
-    if (R.vB) B.b[own] = R.recB;
-    if (R.vC) B.b[(q ^ 1u) * kOffRL1 + ((prel >> 8) & 0xFFu)] = R.recC;
-    if (R.vS) B.b[kOffSL0 + q * (uint32_t)kBufSL + ((prel >> 16) & 0xFFu)] = make_uint4(d.obs, __float_as_uint(v0), __float_as_uint(v1), __float_as_uint(v2));
+    if (vA) B.b[own++] = recA;
+    if (vB) B.b[own] = recB;
+    if (vC) B.b[(q ^ 1u) * kOffRL1 + ((prel >> 8) & 0xFFu)] = recC;
+    if (vS) B.b[kOffSL0 + q * (uint32_t)kBufSL + ((prel >> 16) & 0xFFu)] = recS;
     B.cnt += tot;
 }
 
 template <bool kDebug, bool kDirect, int kThreads>
 __global__ void __launch_bounds__(kThreads, 1)
 rollout_states_kernel(const RolloutArgs A) {
-    extern __shared__ __align__(128) float4 s_tab[];  // kStateQuads, then the warps' record buffers
+    extern __shared__ __align__(128) float4 s_tab[];  // kStateQuads, the rollout image, then the warps' record buffers
     __shared__ unsigned long long s_stats[NFSP_STATS_FIELDS];
     __shared__ __align__(8) uint64_t s_bar;
-    __shared__ FastLuts s_lut;
     __shared__ uint32_t s_next;  // blocks of games this CTA has handed to its warps
     if (threadIdx.x < NFSP_STATS_FIELDS) s_stats[threadIdx.x] = 0ull;
-    s_lut.fill();
+    const uint32_t sbase = smem_u32(s_tab), ibase = sbase + (uint32_t)kStateBytes;
+    {
+        const uint32_t *img = reinterpret_cast<const uint32_t *>(A.pack) + 4 * kStateQuads;
+        uint32_t *dst = reinterpret_cast<uint32_t *>(s_tab + kStateQuads);
+        for (int w = threadIdx.x; w < fsm::kRImageWords; w += kThreads) dst[w] = img[w] + (fsm::is_rollout_address(w) ? sbase : 0u);
+    }
     const uint32_t bar = smem_u32(&s_bar);
     if (threadIdx.x == 0) {
         s_next = 0u;
@@ -202,10 +221,12 @@ rollout_states_kernel(const RolloutArgs A) {
         constexpr uint32_t kChunk = 32768;
         for (uint32_t off = 0; off < (uint32_t)kStateBytes; off += kChunk) {
             const uint32_t len = (uint32_t)kStateBytes - off < kChunk ? (uint32_t)kStateBytes - off : kChunk;
-            bulk_g2s(smem_u32(s_tab) + off, reinterpret_cast<const uint8_t *>(A.pack) + off, len, bar);
+            bulk_g2s(sbase + off, reinterpret_cast<const uint8_t *>(A.pack) + off, len, bar);
         }
     }
     bool image_ready = false;
+    const uint32_t dl_sum = 2u * (ibase + (uint32_t)fsm::kRDealOff) + (uint32_t)fsm::kRDealHalf;
+    const uint32_t rew_base = ibase + (uint32_t)fsm::kRRewardOff;
 
     FastCounters c;
     const int64_t plane = (int64_t)A.n_steps * A.n;
@@ -213,7 +234,7 @@ rollout_states_kernel(const RolloutArgs A) {
     WarpBuf B;
     // the warp's offset goes through a shuffle so that it lives in a register: left as arithmetic on threadIdx.x, it was
     // recomputed at each of the step's four buffer stores (16 instructions per warp-step in ncu's source view)
-    B.b = reinterpret_cast<uint4 *>(s_tab) + kStateQuads + __shfl_sync(0xFFFFFFFFu, (threadIdx.x >> 5) * (uint32_t)kWarpBufQuads, 0);
+    B.b = reinterpret_cast<uint4 *>(s_tab) + kStateQuads + kImageQuads + __shfl_sync(0xFFFFFFFFu, (threadIdx.x >> 5) * (uint32_t)kWarpBufQuads, 0);
     WarpStage W;
     W.init(A, 0u, kDirect);
     const int64_t n_blocks = (A.n + 31) >> 5;  // CTA c owns blocks c, c + grid, ...; its warps take them dynamically
@@ -227,28 +248,97 @@ rollout_states_kernel(const RolloutArgs A) {
         const bool live = i < A.n;
         const uint64_t game = A.game0 + (uint64_t)i;
         W.init(A, (uint32_t)(base >> 5) & (A.n_seg - 1u), kDirect);
-        NfspFast g;
-        g.unpack(live ? A.state[i] : 0ull);
+        fsm::RolloutGame g;
+        g.unpack(live ? A.state[i] : 0ull, ibase, sbase);
         if (!image_ready) {  // the table's copy ran beside the set-up and the first loads of the game words
             mbar_wait(bar, 0);
             image_ready = true;
         }
         for (int t = 0; t < A.n_steps; ++t) {
-            FastDecision d;
-            fast_begin(g, s_lut, A, game, A.step0 + (uint64_t)t, live, d, c);
-            const uint32_t ca = (g.PA >> 11) & 3u;
-            const uint32_t x = (((ca * 3u + g.pub()) * 2u + g.dealer()) << 2) | g.fin0();
-            const float4 o = s_tab[(g.p() * 2u + (uint32_t)d.pol) * (uint32_t)kNetStates + x * 18u + g.sigma()];
-            float v0 = o.x, v1 = o.y, v2 = o.z;
-            uint32_t pre = __float_as_uint(o.w);
-            if (d.random) { v0 = d.r0; v1 = d.r1; v2 = d.r2; pre = score_action(v0, v1, v2); }
-            FastRecords R;
-            fast_decide<kDebug>(g, s_lut, A, d, v0, v1, v2, live, (int64_t)t * A.n + i, plane, c, R, pre);
-            buf_append<kDirect>(B, A, W, d, R, v0, v1, v2, c);
+            const uint64_t step = A.step0 + (uint64_t)t;
+            const Philox4 x = game_block(A.keys, game, step, STREAM_STEP);
+            uint32_t started = 0u;
+            if (g.HX & fsm::kHxOver) {  // newenv.py:76-114 + main.py:28-45: the other player deals
+                g.dl = dl_sum - g.dl;
+                const uint4 D = fsm::lds128(g.dl + __umulhi(x.y, 120u) * 16u);
+                uint32_t pa = g.dl + (uint32_t)fsm::kPolOff;
+                if (x.z < A.eta_u32) pa += 16u;
+                if (x.w < A.eta_u32) pa += 32u;
+                const uint4 P = fsm::lds128(pa);
+                g.PA = D.x | P.x;
+                g.PO = D.y | P.y;
+                g.FA = D.z + P.z;
+                g.FO = D.w + P.w;
+                g.SA = 0u;
+                g.SO = 0u;
+                g.tix = g.dl - (uint32_t)fsm::kRDealOff;
+                g.HX = fsm::kCm0;
+                started = 1u;
+                c.wide.hands += live;
+            }
+            // agent.py:130-141: the observation, the transition to remember, the policy of the hand, the epsilon branch
+            const uint32_t q = (g.PA >> 23) & 1u;
+            const uint32_t obs = g.HX & (g.PA | 0x00FFFFFFu);
+            const bool vA = (g.PA & kWordNz) != 0u, pol = (g.PA & (1u << 12)) != 0u;
+            const uint4 recA = make_uint4(g.SA, obs, 0u, ((g.PA >> 13) & 3u) | (q << 16));
+            const uint4 o = fsm::lds128(g.FA);
+            float v0 = __uint_as_float(o.x), v1 = __uint_as_float(o.y), v2 = __uint_as_float(o.z);
+            uint32_t aw = o.w;
+            if (pol && x.x < (q ? A.eps1_u32 : A.eps_u32)) {  // np.random.rand(1,1,3): rare, so it has its own Philox block
+                const Philox4 y = game_block(A.keys, game, step, STREAM_VECTOR);
+                v0 = (float)(y.x >> 8) * (1.0f / 16777216.0f);
+                v1 = (float)(y.y >> 8) * (1.0f / 16777216.0f);
+                v2 = (float)(y.z >> 8) * (1.0f / 16777216.0f);
+                aw = score_word(v0, v1, v2);
+            }
+            const int64_t at = (int64_t)t * A.n + i;
+            if (kDebug && live) {
+                if (A.vec) { A.vec[3 * at] = v0; A.vec[3 * at + 1] = v1; A.vec[3 * at + 2] = v2; }
+                if (A.forced) { v0 = A.forced[3 * at]; v1 = A.forced[3 * at + 1]; v2 = A.forced[3 * at + 2]; }
+                aw = score_word(v0, v1, v2);
+            }
+            // newenv.py:192-349: the entry (row, raw action)
+            const uint32_t ea = g.tix + (aw & kWordEntry);
+            const uint4 E = fsm::lds128(ea);        // hc, pa, pm, nx
+            const uint4 M = fsm::lds128(ea + 16u);  // ds, mx, rm, inc
+            g.PA = ((g.PA & ~fsm::kPClear) | (aw & kWordNz)) + E.y;
+            g.HX = (g.HX & 0xFFFFFFu) | E.x;
+            c.small += live ? M.w : 0u;
+            // main.py:55-67: at the end of the hand both players observe the terminal state once (no swap happens then)
+            const bool term = (g.HX & fsm::kHxOver) != 0u;
+            const uint32_t rw = fsm::lds32(rew_base + (M.z & ((g.PA & 0xFFu) | (g.PO & 0xF00u))));  // 0 while the hand is live
+            const int ra = (int)(int8_t)(rw & 0xFFu), ro = (int)(int8_t)((rw >> 8) & 0xFFu);
+            c.wide.rew0 += live ? (q ? ro : ra) : 0;
+            c.wide.rew1 += live ? (q ? ra : ro) : 0;
+            const float fa = 0.5f * (float)ra;
+            const uint4 recB = make_uint4(obs, g.HX & (g.PA | 0x00FFFFFFu), __float_as_uint(fa), M.y & 0x10103u);
+            const uint4 recC = make_uint4(g.SO, g.HX & (g.PO | 0x00FFFFFFu), __float_as_uint(0.5f * (float)ro),
+                                          ((g.PO >> 13) & 3u) | ((M.y & 0x10100u) ^ 0x10000u));
+            const bool vB = term && (aw & kWordNz) && live, vC = term && (g.PO & kWordNz) && live;
+            if (kDebug && live && A.trace) {
+                const uint32_t P0 = q ? g.PO : g.PA, P1 = q ? g.PA : g.PO;
+                const uint32_t d = g.dl != ibase + (uint32_t)fsm::kRDealOff ? 1u : 0u;
+                A.trace[at] = g.HX & (g.PA | 0xC0FFFFFFu);  // observation of the actor | hand over << 30 | actor << 31
+                A.trace[plane + at] = __float_as_uint(fa);
+                A.trace[2 * plane + at] = (M.y & 0x101Fu) | (d << 5) | (((P0 >> 19) & 3u) << 6) | (((P1 >> 19) & 3u) << 8) |
+                                          (((P0 >> 21) & 3u) << 10) | (((P0 >> 2) & 15u) << 13) | (((P1 >> 2) & 15u) << 17) |
+                                          (started << 21) | (((P0 >> 12) & 1u) << 22) | (((P1 >> 12) & 1u) << 23);
+            }
+            // the turn passes: swap the per-player registers
+            const uint32_t pm = E.z, pa = g.PA, sa = obs, fa_ = g.FA + M.x, fo = g.FO + M.x;
+            g.PA = (g.PO & pm) | (pa & ~pm);
+            g.PO = (pa & pm) | (g.PO & ~pm);
+            g.SA = (g.SO & pm) | (sa & ~pm);
+            g.SO = (sa & pm) | (g.SO & ~pm);
+            g.FA = (fo & pm) | (fa_ & ~pm);
+            g.FO = (fa_ & pm) | (fo & ~pm);
+            g.tix = E.w;
+            buf_append<kDirect>(B, A, W, c, q, vA && live, vB, vC, pol && live, recA, recB, recC,
+                                make_uint4(obs, __float_as_uint(v0), __float_as_uint(v1), __float_as_uint(v2)));
             if ((t & 15) == 15) c.spill();
         }
         c.spill();
-        if (live) A.state[i] = g.pack();
+        if (live) A.state[i] = g.pack(ibase);
         c.wide.trans += live ? A.n_steps : 0;
         // a block's staged records belong to the block's segment; the rings have no segments, their records stay buffered
         buf_flush<kDirect>(B, A, W, c, kDirect ? 12u : 15u);
@@ -263,7 +353,24 @@ rollout_states_kernel(const RolloutArgs A) {
 
 using namespace nfsp;
 
-int nfsp_states_floats() { return kStateQuads * 4; }
+// the state table, then the rollout image (uploaded once, nfsp_states_upload_image)
+int nfsp_states_floats() { return kStateQuads * 4 + fsm::kRImageWords; }
+
+static void build_states_image(uint32_t *img) { fsm::build_rollout_image(img, (uint32_t)kStateBytes); }
+
+int nfsp_states_upload_image(float *d_states) {
+    static uint32_t image[fsm::kRImageWords];
+    static const bool built = (build_states_image(image), true);
+    (void)built;
+    NFSP_CUDA(cudaMemcpy(d_states + 4 * kStateQuads, image, sizeof(image), cudaMemcpyHostToDevice));
+    return NFSP_OK;
+}
+
+// the rollout image for inspection on the host (addresses: byte offsets from the state table, which it follows)
+extern "C" int nfsp_rollout_image(uint32_t *out, int capacity_words) {
+    if (out && capacity_words >= fsm::kRImageWords) build_states_image(out);
+    return fsm::kRImageWords;
+}
 
 template <int kThreads>
 static int configure_states() {
