@@ -214,6 +214,21 @@ int nfsp_rollout(nfsp_env_t h, int n_steps, double eta, double epsilon, const nf
  * nfsp_act_set_weights(h, d_weights, stream) followed by nfsp_rollout(...). */
 int nfsp_rollout_with_weights(nfsp_env_t h, const float *h_weights, float *d_weights, int n_steps, double eta, double epsilon,
                               const nfsp_rollout_io *io, void *stream);
+/* Independent runs side by side: n_runs handles, each with its own games, step counter, seed, weight images, state table,
+ * memories and counters, whose hot launches are shared.  Run r does exactly what it would do alone, bit for bit.
+ * The same as n_runs calls nfsp_rollout(h[r], n_steps, eta[r], epsilon[r], &io[r], stream) -- preceded by
+ * nfsp_act_set_weights(h[r], d_weights[r], stream) when d_weights is not NULL -- with variant 6 and no debug outputs
+ * (io[r].variant 0 or 6; d_trace, d_vec, d_forced_vec NULL; player 1's epsilon through io[r].epsilon_p1 as there).
+ *   - d_weights (float[4][2179] per run) or NULL: the weight images and state tables of all runs are rebuilt first, in one
+ *     launch each (the run on blockIdx.y); every handle is then left as nfsp_act_set_weights leaves it.
+ *   - the rollout is ONE launch: the CTAs are split into contiguous ranges of floor((SMs - reserve_sms) / n_runs) or
+ *     fewer, one range per run, and a CTA serves its run as the run's own launch on that many CTAs would.
+ * The runs must share their shape: device, game count, direct or staged records, n_segments, ring_cap and reserve_sms;
+ * otherwise, or with n_runs outside [1, min(NFSP_MAX_RUNS, SMs - reserve_sms)], the call returns NFSP_E_ARG before
+ * anything is launched.  Every handle's step counter advances by n_steps. */
+#define NFSP_MAX_RUNS 32
+int nfsp_rollout_runs(const nfsp_env_t *h, int n_runs, int n_steps, const double *eta, const double *epsilon,
+                      const nfsp_rollout_io *io, float *const *d_weights, void *stream);
 /* Tuning of variant 3: SM cycles a partly filled tile of an average-policy / a best-response net may wait for more rows
  * before its MMAs are issued anyway (defaults 1500 / 700). */
 int nfsp_rollout_tune(nfsp_env_t h, int patience_avg, int patience_br);
@@ -279,7 +294,7 @@ int nfsp_sample_indices(uint64_t seed, uint64_t call_idx, const uint64_t *d_tota
  * reservoir (SL)  s[batch][30] a[batch][3]  = 33 * batch floats.  d_idx int64[n_reqs][batch] (storage slots, -1 beyond
  * the records held) and d_n_out uint32[n_reqs] (rows sampled) may be NULL.  A request with d_out = NULL only reports its
  * positions in d_idx (the learner kernels read the packed records themselves). */
-#define NFSP_MAX_SAMPLE_REQS 8
+#define NFSP_MAX_SAMPLE_REQS 128 /* 4 * NFSP_MAX_RUNS: the four memories of every run of a batch */
 typedef struct {
     const void *d_mem;        /* ring (16-byte records) / reservoir (32-byte slots, the record first) storage */
     const uint64_t *d_total;  /* records ever inserted (device) */
@@ -332,6 +347,12 @@ int nfsp_learner_grads(const nfsp_learner_io *io, void *stream);
 #define NFSP_MAX_FIT_STEPS 64
 int nfsp_learner_fit(const nfsp_learner_io *io, int minibatch, int fit_batch, int epochs, const float lr[4],
                      float *d_weights_out, void *stream);
+/* The fits of n_runs independent runs in ONE launch of 4 * n_runs CTAs (blockIdx.x = 4 * run + net): the same as n_runs
+ * calls nfsp_learner_fit(&io[r], minibatch, fit_batch, epochs, lr + 4 * r, d_weights_out[r], stream), each with its own
+ * memories, sampled slots, net_mask, gamma, flags, target nets, statistics and output weights (d_weights_out[r] may be
+ * io[r].d_weights).  The SGD step schedule (minibatch, fit_batch, epochs) is shared; 1 <= n_runs <= NFSP_MAX_RUNS. */
+int nfsp_learner_fit_runs(const nfsp_learner_io *io, int n_runs, int minibatch, int fit_batch, int epochs, const float *lr,
+                          float *const *d_weights_out, void *stream);
 /* The same fit when several GPUs of one box train together (SURVEY 8e, C1 + C2): the all-reduce of every SGD step runs
  * INSIDE the kernel over peer memory (NVLink).  Each rank owns an exchange buffer of NFSP_PEER_BUF_FLOATS floats, zeroed
  * once, that every other rank can address (CUDA IPC / torch symmetric memory); d_buf[r] is rank r's buffer as THIS

@@ -25,9 +25,9 @@ SYMBOLS = [
     "nfsp_legacy_reset", "nfsp_legacy_set_hands", "nfsp_legacy_step", "nfsp_legacy_get_new_state",
     "nfsp_legacy_rollout", "nfsp_legacy_export",
     "nfsp_expand_obs",
-    "nfsp_act_set_weights", "nfsp_act_set_weights_from_host", "nfsp_act_forward", "nfsp_act_forward_tc", "nfsp_rollout", "nfsp_rollout_with_weights", "nfsp_rollout_tune", "nfsp_rollout_profile",
+    "nfsp_act_set_weights", "nfsp_act_set_weights_from_host", "nfsp_act_forward", "nfsp_act_forward_tc", "nfsp_rollout", "nfsp_rollout_with_weights", "nfsp_rollout_runs", "nfsp_rollout_tune", "nfsp_rollout_profile",
     "nfsp_ring_insert", "nfsp_reservoir_insert", "nfsp_insert_multi", "nfsp_ring_insert_multi", "nfsp_reservoir_insert_multi", "nfsp_sample_indices", "nfsp_sample_minibatches", "nfsp_gather_rl", "nfsp_gather_sl",
-    "nfsp_learner_grads", "nfsp_learner_fit", "nfsp_learner_fit_peers", "nfsp_sgd_apply",
+    "nfsp_learner_grads", "nfsp_learner_fit", "nfsp_learner_fit_runs", "nfsp_learner_fit_peers", "nfsp_sgd_apply",
     "nfsp_peer_buffer_create", "nfsp_peer_buffer_open", "nfsp_peer_buffer_close", "nfsp_peer_buffer_destroy",
 ]
 
@@ -55,6 +55,9 @@ MAX_PEERS, PEER_BUF_FLOATS = 8, 279552  # NFSP_MAX_PEERS, NFSP_PEER_BUF_FLOATS
 class Peers(C.Structure):
     _fields_ = [("world", C.c_int32), ("rank", C.c_int32), ("d_buf", C.c_void_p * MAX_PEERS), ("epoch0", C.c_uint32),
                 ("d_err", C.c_void_p), ("d_mc", C.c_void_p)]
+
+
+MAX_RUNS, MAX_SAMPLE_REQS = 32, 128  # NFSP_MAX_RUNS, NFSP_MAX_SAMPLE_REQS (= 4 * NFSP_MAX_RUNS)
 
 
 class SampleReq(C.Structure):
@@ -127,6 +130,8 @@ def lib():
     L.nfsp_act_forward_tc.argtypes = [vp, vp, i8p, C.c_int64, vp, vp]
     L.nfsp_rollout.argtypes = [vp, C.c_int, C.c_double, C.c_double, C.POINTER(RolloutIO), vp]
     L.nfsp_rollout_with_weights.argtypes = [vp, vp, vp, C.c_int, C.c_double, C.c_double, C.POINTER(RolloutIO), vp]
+    L.nfsp_rollout_runs.argtypes = [C.POINTER(vp), C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double),
+                                    C.POINTER(RolloutIO), C.POINTER(vp), vp]
     L.nfsp_ring_insert.argtypes = [vp, C.c_int64, vp, vp, vp, C.c_int, C.c_int64, vp, vp]
     L.nfsp_reservoir_insert.argtypes = [vp, C.c_int64, vp, vp, vp, C.c_int, C.c_int64, C.c_uint64, C.c_int, vp, vp]
     L.nfsp_insert_multi.argtypes = [C.POINTER(InsertReq), C.c_int, vp]
@@ -138,6 +143,8 @@ def lib():
     L.nfsp_gather_sl.argtypes = [vp, vp, C.c_int, vp, vp, vp]
     L.nfsp_learner_grads.argtypes = [C.POINTER(LearnerIO), vp]
     L.nfsp_learner_fit.argtypes = [C.POINTER(LearnerIO), C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float), vp, vp]
+    L.nfsp_learner_fit_runs.argtypes = [C.POINTER(LearnerIO), C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float),
+                                        C.POINTER(vp), vp]
     L.nfsp_learner_fit_peers.argtypes = [C.POINTER(LearnerIO), C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float), vp,
                                          C.POINTER(Peers), vp]
     L.nfsp_sgd_apply.argtypes = [vp, vp, C.POINTER(C.c_float * 4), C.c_float, vp]

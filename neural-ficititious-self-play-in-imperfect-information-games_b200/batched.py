@@ -496,19 +496,7 @@ class SelfPlay:
         if n_steps > self.max_steps:
             raise ValueError("n_steps %d exceeds max_steps_per_call %d" % (n_steps, self.max_steps))
         want_debug = debug or forced_vec is not None
-        io = None if want_debug else getattr(self, "_io", None)  # the production argument block is built once
-        if io is None:
-            io = _lib.RolloutIO()
-            for p in range(2):
-                io.d_rl[p], io.d_sl[p] = self.stage_rl[p].data_ptr(), self.stage_sl[p].data_ptr()
-            io.cap_rl, io.cap_sl, io.n_segments = self.cap_rl, self.cap_sl, self.n_seg
-            io.d_counts, io.d_stats = self.counts.data_ptr(), self.stats.data_ptr()
-            if self.direct_rings:
-                for p in range(2):
-                    io.d_ring[p], io.d_ring_total[p] = self.rl[p].store.data_ptr(), self.rl[p].total.data_ptr()
-                io.ring_cap = self.rl[0].capacity
-            if not want_debug:
-                self._io = io
+        io = self._rollout_io(cache=not want_debug)
         io.variant = self.VARIANTS[variant or self.variant]
         io.epsilon_per_player, io.epsilon_p1 = int(self.epsilons[0] != self.epsilons[1]), self.epsilons[1]
         if self.direct_rings and io.variant not in (0, 1, 4, 5, 6):
@@ -547,6 +535,24 @@ class SelfPlay:
             self.flush()
         return out
 
+    def _rollout_io(self, cache=True):
+        """The rollout's argument block: staging arrays, counters and (direct_rings) the rings.  The production block is
+        built once (cache=True); a debug call gets a fresh one."""
+        io = getattr(self, "_io", None) if cache else None
+        if io is None:
+            io = _lib.RolloutIO()
+            for p in range(2):
+                io.d_rl[p], io.d_sl[p] = self.stage_rl[p].data_ptr(), self.stage_sl[p].data_ptr()
+            io.cap_rl, io.cap_sl, io.n_segments = self.cap_rl, self.cap_sl, self.n_seg
+            io.d_counts, io.d_stats = self.counts.data_ptr(), self.stats.data_ptr()
+            if self.direct_rings:
+                for p in range(2):
+                    io.d_ring[p], io.d_ring_total[p] = self.rl[p].store.data_ptr(), self.rl[p].total.data_ptr()
+                io.ring_cap = self.rl[0].capacity
+            if cache:
+                self._io = io
+        return io
+
     def staged(self):
         """Host copies of the staged records in batch order (segment by segment): ([rl0, rl1], [sl0, sl1])."""
         c = self.counts.cpu().numpy()
@@ -572,20 +578,30 @@ class SelfPlay:
         if hasattr(self, "_flush_reqs") and any(m._scratch is None or m._scratch.data_ptr() != p_ for m, p_ in zip(mems_now, self._flush_scratch)):
             del self._flush_reqs  # somebody inserted into a memory with a larger geometry: its scratch block moved
         if not hasattr(self, "_flush_reqs"):  # pointers and geometry never change: the request block is built once
-            mems = [(self.sl[p], self.stage_sl[p], 2 + p, self.cap_sl) for p in range(2)]
-            if not self.direct_rings:
-                mems += [(self.rl[p], self.stage_rl[p], p, self.cap_rl) for p in range(2)]
+            mems = self._insert_mems()
             arr = (_lib.InsertReq * len(mems))()
-            for r, (mem, stage, row, seg_cap) in zip(arr, mems):
-                r.d_mem, r.cap, r.d_total = mem.store.data_ptr(), mem.capacity, mem.total.data_ptr()
-                r.d_scratch = mem.scratch(self.n_seg).data_ptr()
-                r.d_recs, r.d_counts = stage.data_ptr(), self.counts[row].data_ptr()
-                r.n_segments, r.seg_cap, r.seed, r.mode = self.n_seg, seg_cap, mem.seed, getattr(mem, "mode", 0)
-                r.reservoir = 0 if mem.is_ring else 1
+            for r, m in zip(arr, mems):
+                self._insert_req(r, *m)
             self._flush_reqs = (arr, len(mems))
             self._flush_scratch = [m[0]._scratch.data_ptr() for m in mems]
         arr, n = self._flush_reqs
         check(lib().nfsp_insert_multi(arr, n, _stream(self.device)))
+
+    def _insert_mems(self):
+        """What flush() moves: (memory, staging array, counts row, segment capacity) -- both reservoirs, then the rings
+        unless the rollout writes them directly."""
+        mems = [(self.sl[p], self.stage_sl[p], 2 + p, self.cap_sl) for p in range(2)]
+        if not self.direct_rings:
+            mems += [(self.rl[p], self.stage_rl[p], p, self.cap_rl) for p in range(2)]
+        return mems
+
+    def _insert_req(self, r, mem, stage, row, seg_cap):
+        """Fills the nfsp_insert_req r of one entry of _insert_mems()."""
+        r.d_mem, r.cap, r.d_total = mem.store.data_ptr(), mem.capacity, mem.total.data_ptr()
+        r.d_scratch = mem.scratch(self.n_seg).data_ptr()
+        r.d_recs, r.d_counts = stage.data_ptr(), self.counts[row].data_ptr()
+        r.n_segments, r.seg_cap, r.seed, r.mode = self.n_seg, seg_cap, mem.seed, getattr(mem, "mode", 0)
+        r.reservoir = 0 if mem.is_ring else 1
 
     def sample_minibatches(self, batch=256, to_host=False, with_stats=False):
         """sample_batch(batch) of all four memories (replay_buffer.py:46-59, ReservoirBuffer.py:33-43) into ONE

@@ -48,13 +48,13 @@ __device__ __forceinline__ float pack_weights_value(const float *__restrict__ w,
 }
 
 static_assert((kPackFloats + kTabImageFloats + 4 * NFSP_NET_PARAMS) % 4 == 0, "the state table behind the images must be 16-byte aligned (bulk copy)");
-// both images in one launch: pack = [batched-forward image (kPackFloats) | rollout table image (kTabImageFloats)]
-// ... followed by a plain copy of the four nets (what the tensor-core variants' images are built from, on demand)
-__global__ void pack_images_kernel(const float *__restrict__ w, float *__restrict__ pack) {
+// both images in one launch: pack = [batched-forward image (kPackFloats) | rollout table image (kTabImageFloats)] + a plain copy of the four nets (what the tensor-core variants' images are built from, on demand)
+__device__ __forceinline__ void pack_images(const float *__restrict__ w, float *__restrict__ pack) {
     constexpr int kImages = kPackFloats + kTabImageFloats;
     for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < kImages + 4 * NFSP_NET_PARAMS; e += gridDim.x * blockDim.x)
         pack[e] = e < kPackFloats ? pack_weights_value(w, e) : (e < kImages ? pack_tables_value(w, e - kPackFloats) : w[e - kImages]);
 }
+__global__ void pack_images_kernel(const float *__restrict__ w, float *__restrict__ pack) { pack_images(w, pack); }
 
 // forward of one net on one observation mask; sw = packed image in shared memory.  The first layer is the sum of the
 // <= 10 weight rows of the set input bits (+ the bias row), accumulated in the thread's ROTATED quad order.
@@ -178,6 +178,13 @@ rollout_kernel(const RolloutArgs A) {
     if (A.stats) c.wide.commit(s_stats, A.stats);
 }
 
+// the images of several handles in one launch (nfsp_rollout_runs): blockIdx.y = run
+struct ImageRuns {
+    const float *w[NFSP_MAX_RUNS];
+    float *pack[NFSP_MAX_RUNS];
+};
+__global__ void pack_images_runs_kernel(const __grid_constant__ ImageRuns P) { pack_images(P.w[blockIdx.y], P.pack[blockIdx.y]); }
+
 }  // namespace nfsp
 
 using namespace nfsp;
@@ -270,8 +277,10 @@ int nfsp_rollout_direct_args(const nfsp_rollout_io *io, RolloutArgs &A, bool *di
     return NFSP_OK;
 }
 
-extern "C" int nfsp_rollout(nfsp_env_t h, int n_steps, double eta, double epsilon, const nfsp_rollout_io *io,
-                            void *stream) {
+// validates the arguments of a rollout of handle h and fills A (nothing is launched): the variant to run (0 resolved),
+// whether the call has debug outputs, whether it appends to the rings directly
+static int rollout_args(nfsp_env_t h, int n_steps, double eta, double epsilon, const nfsp_rollout_io *io, RolloutArgs &A,
+                        int *variant_out, bool *debug_out, bool *direct_out) {
     NFSP_CHECK_ARG(h != nullptr && io != nullptr, "null argument");
     NFSP_CHECK_ARG(h->rules == NFSP_RULES_NFSP, "rollout needs NFSP rules");
     NFSP_CHECK_ARG(n_steps >= 1 && n_steps <= 4096, "n_steps must be in [1,4096]");
@@ -281,9 +290,6 @@ extern "C" int nfsp_rollout(nfsp_env_t h, int n_steps, double eta, double epsilo
     NFSP_CHECK_ARG(io->n_segments >= 1 && io->n_segments <= 65536 && (io->n_segments & (io->n_segments - 1)) == 0,
                    "n_segments must be a power of two in [1,65536]");
     if (!h->has_weights) return set_error(NFSP_E_STATE, "nfsp_act_set_weights has not been called");
-    DeviceGuard guard(h->device);
-    if (!guard.ok) return set_error(NFSP_E_CUDA, "cannot select device %d", h->device);
-    RolloutArgs A;
     A.keys = philox_keys(h->seed);
     A.state = h->d_state; A.n = h->n; A.seed = h->seed; A.game0 = h->game0; A.step0 = h->step; A.n_steps = n_steps;
     A.eta_u32 = frac_u32(eta); A.eps_u32 = frac_u32(epsilon);
@@ -305,6 +311,23 @@ extern "C" int nfsp_rollout(nfsp_env_t h, int n_steps, double eta, double epsilo
         if (rc != NFSP_OK) return rc;
     }
     NFSP_CHECK_ARG(!direct || variant == 1 || variant >= 4, "the direct ring append (d_ring) exists in variants 1, 4, 5 and 6 only");
+    *variant_out = variant;
+    *debug_out = debug;
+    *direct_out = direct;
+    return NFSP_OK;
+}
+
+extern "C" int nfsp_rollout(nfsp_env_t h, int n_steps, double eta, double epsilon, const nfsp_rollout_io *io,
+                            void *stream) {
+    RolloutArgs A;
+    int variant = 0;
+    bool debug = false, direct = false;
+    {
+        const int rc = rollout_args(h, n_steps, eta, epsilon, io, A, &variant, &debug, &direct);
+        if (rc != NFSP_OK) return rc;
+    }
+    DeviceGuard guard(h->device);
+    if (!guard.ok) return set_error(NFSP_E_CUDA, "cannot select device %d", h->device);
     if (variant == 6) {
         int rc = nfsp_states_ensure(h, h->d_wpack + kPackFloats, h->d_states, (cudaStream_t)stream);
         if (rc != NFSP_OK) return rc;
@@ -357,4 +380,58 @@ extern "C" int nfsp_rollout_with_weights(nfsp_env_t h, const float *h_weights, f
     const int rc = h_weights ? nfsp_act_set_weights_from_host(h, h_weights, d_weights, stream) : nfsp_act_set_weights(h, d_weights, stream);
     if (rc != NFSP_OK) return rc;
     return nfsp_rollout(h, n_steps, eta, epsilon, io, stream);
+}
+
+extern "C" int nfsp_rollout_runs(const nfsp_env_t *h, int n_runs, int n_steps, const double *eta, const double *epsilon,
+                                 const nfsp_rollout_io *io, float *const *d_weights, void *stream) {
+    NFSP_CHECK_ARG(h != nullptr && eta != nullptr && epsilon != nullptr && io != nullptr, "null argument");
+    NFSP_CHECK_ARG(n_runs >= 1 && n_runs <= NFSP_MAX_RUNS, "n_runs must be in [1, %d]", NFSP_MAX_RUNS);
+    RolloutArgs A[NFSP_MAX_RUNS];
+    for (int r = 0; r < n_runs; ++r) {
+        NFSP_CHECK_ARG(h[r] != nullptr, "null handle of run %d", r);
+        for (int q = 0; q < r; ++q) NFSP_CHECK_ARG(h[q] != h[r], "runs %d and %d share a handle", q, r);
+        NFSP_CHECK_ARG(io[r].variant == 0 || io[r].variant == 6, "runs play variant 6 (run %d asks for %d)", r, io[r].variant);
+        NFSP_CHECK_ARG(!io[r].d_trace && !io[r].d_vec && !io[r].d_forced_vec, "runs have no debug outputs (run %d)", r);
+        NFSP_CHECK_ARG(!d_weights || d_weights[r], "null weights of run %d", r);
+        int variant = 0;
+        bool debug = false, direct = false;
+        const int rc = rollout_args(h[r], n_steps, eta[r], epsilon[r], &io[r], A[r], &variant, &debug, &direct);
+        if (rc != NFSP_OK) return rc;
+        A[r].pack = h[r]->d_states;
+        // the shape every run shares: one thread count and one CTA count per run for the whole launch
+        NFSP_CHECK_ARG(h[r]->device == h[0]->device, "run %d is on device %d, run 0 on %d", r, h[r]->device, h[0]->device);
+        NFSP_CHECK_ARG(h[r]->n == h[0]->n, "run %d has %lld games, run 0 %lld", r, (long long)h[r]->n, (long long)h[0]->n);
+        NFSP_CHECK_ARG((A[r].ring[0] != nullptr) == (A[0].ring[0] != nullptr), "runs 0 and %d differ in the record mode (direct rings)", r);
+        NFSP_CHECK_ARG(io[r].n_segments == io[0].n_segments, "runs 0 and %d differ in n_segments", r);
+        NFSP_CHECK_ARG(io[r].ring_cap == io[0].ring_cap, "runs 0 and %d differ in ring_cap", r);
+        NFSP_CHECK_ARG(io[r].reserve_sms == io[0].reserve_sms, "runs 0 and %d differ in reserve_sms", r);
+    }
+    const int sms = h[0]->sm_count - io[0].reserve_sms;
+    NFSP_CHECK_ARG(n_runs <= sms, "%d runs need as many SMs (%d free)", n_runs, sms);
+    DeviceGuard guard(h[0]->device);
+    if (!guard.ok) return set_error(NFSP_E_CUDA, "cannot select device %d", h[0]->device);
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (d_weights) {  // nfsp_act_set_weights of every run: the images, then the state tables, one launch each
+        ImageRuns P;
+        const float *tab[NFSP_MAX_RUNS];
+        for (int r = 0; r < n_runs; ++r) {
+            P.w[r] = d_weights[r];
+            P.pack[r] = h[r]->d_wpack;
+            tab[r] = h[r]->d_wpack + kPackFloats;
+        }
+        pack_images_runs_kernel<<<dim3((kPackFloats + kTabImageFloats + 4 * NFSP_NET_PARAMS + 255) / 256, (unsigned)n_runs), 256, 0, st>>>(P);
+        NFSP_LAUNCH_CHECK();
+        for (int r = 0; r < n_runs; ++r) h[r]->tc_dirty = h[r]->tq_dirty = h[r]->st_dirty = true;
+        const int rc = nfsp_states_pack_runs(h, tab, n_runs, st);
+        if (rc != NFSP_OK) return rc;
+    } else {
+        for (int r = 0; r < n_runs; ++r) {
+            const int rc = nfsp_states_ensure(h[r], h[r]->d_wpack + kPackFloats, h[r]->d_states, st);
+            if (rc != NFSP_OK) return rc;
+        }
+    }
+    const int rc = nfsp_rollout_states_runs_launch(h[0], A, n_runs, sms, st);
+    if (rc != NFSP_OK) return rc;
+    for (int r = 0; r < n_runs; ++r) h[r]->step += (uint64_t)n_steps;
+    return NFSP_OK;
 }

@@ -378,16 +378,22 @@ __device__ __forceinline__ void expand_sl(const uint4 rec, int row, int col, flo
 // its share of the sampled records once (one random 16-byte read per row, all in flight together) and expands them
 // into out[m] -- an RL block is s[b][30] a[b][3] r[b] s2[b][30] t[b], an SL block s[b][30] a[b][3] (b = batch).  The
 // rows of a memory are split over gridDim.y CTAs; each repeats the (cheap) draw.
-struct SampleReqs {
-    const uint4 *mem[NFSP_MAX_SAMPLE_REQS];
-    const uint64_t *total[NFSP_MAX_SAMPLE_REQS];
-    uint64_t cap[NFSP_MAX_SAMPLE_REQS], seed[NFSP_MAX_SAMPLE_REQS], call_idx[NFSP_MAX_SAMPLE_REQS];
-    float *out[NFSP_MAX_SAMPLE_REQS];
-    uint4 *rec_out[NFSP_MAX_SAMPLE_REQS];  // packed copies of the sampled slots (ring: 16 bytes, reservoir: 32), or null
-    int is_ring[NFSP_MAX_SAMPLE_REQS];
+// Up to kSmallSampleReqs requests travel in the kernel's parameters as they always have; a larger table (the four memories
+// of every run of a batch) in a __grid_constant__ copy of the wide table -- the same draws and rows either way.
+constexpr int kSmallSampleReqs = 8;
+template <int kReqs>
+struct SampleTable {
+    const uint4 *mem[kReqs];
+    const uint64_t *total[kReqs];
+    uint64_t cap[kReqs], seed[kReqs], call_idx[kReqs];
+    float *out[kReqs];
+    uint4 *rec_out[kReqs];  // packed copies of the sampled slots (ring: 16 bytes, reservoir: 32), or null
+    int is_ring[kReqs];
 };
-__global__ void __launch_bounds__(kBufThreads)
-sample_gather_kernel(const SampleReqs R, int batch, int64_t *__restrict__ idx_out, uint32_t *__restrict__ n_out) {
+struct SampleReqs : SampleTable<kSmallSampleReqs> {};
+struct SampleReqsWide : SampleTable<NFSP_MAX_SAMPLE_REQS> {};
+template <class Reqs>
+__device__ __forceinline__ void sample_gather(const Reqs &R, int batch, int64_t *__restrict__ idx_out, uint32_t *__restrict__ n_out) {
     __shared__ uint64_t draw[kMaxBatch];
     __shared__ uint64_t pick[kMaxBatch];
     __shared__ int64_t slot[kMaxBatch];
@@ -426,6 +432,14 @@ sample_gather_kernel(const SampleReqs R, int batch, int64_t *__restrict__ idx_ou
             expand_sl(s_rec[row], row, col, s, a);
         }
     }
+}
+__global__ void __launch_bounds__(kBufThreads)
+sample_gather_kernel(const SampleReqs R, int batch, int64_t *__restrict__ idx_out, uint32_t *__restrict__ n_out) {
+    sample_gather(R, batch, idx_out, n_out);
+}
+__global__ void __launch_bounds__(kBufThreads)
+sample_gather_wide_kernel(const __grid_constant__ SampleReqsWide R, int batch, int64_t *__restrict__ idx_out, uint32_t *__restrict__ n_out) {
+    sample_gather(R, batch, idx_out, n_out);
 }
 
 __global__ void __launch_bounds__(kBufThreads)
@@ -572,11 +586,8 @@ extern "C" int nfsp_sample_indices(uint64_t seed, uint64_t call_idx, const uint6
     return NFSP_OK;
 }
 
-extern "C" int nfsp_sample_minibatches(const nfsp_sample_req *reqs, int n_reqs, int batch, int64_t *d_idx, uint32_t *d_n_out,
-                                       void *stream) {
-    NFSP_CHECK_ARG(reqs && n_reqs >= 1 && n_reqs <= NFSP_MAX_SAMPLE_REQS, "1..%d requests", NFSP_MAX_SAMPLE_REQS);
-    NFSP_CHECK_ARG(batch >= 1 && batch <= kMaxBatch, "batch must be in [1,%d]", kMaxBatch);
-    SampleReqs R;
+template <int kReqs>
+static int fill_sample_table(const nfsp_sample_req *reqs, int n_reqs, const int64_t *d_idx, SampleTable<kReqs> &R) {
     for (int m = 0; m < n_reqs; ++m) {
         NFSP_CHECK_ARG(reqs[m].d_mem && reqs[m].d_total && reqs[m].cap > 0, "bad request %d", m);
         NFSP_CHECK_ARG(reqs[m].d_out || reqs[m].d_rec_out || d_idx, "request %d has neither an output block nor an index array", m);
@@ -589,7 +600,25 @@ extern "C" int nfsp_sample_minibatches(const nfsp_sample_req *reqs, int n_reqs, 
         R.rec_out[m] = (uint4 *)reqs[m].d_rec_out;
         R.is_ring[m] = reqs[m].is_ring;
     }
-    sample_gather_kernel<<<dim3((unsigned)n_reqs, 8u, 1u), kBufThreads, 0, (cudaStream_t)stream>>>(R, batch, d_idx, d_n_out);
+    return NFSP_OK;
+}
+
+extern "C" int nfsp_sample_minibatches(const nfsp_sample_req *reqs, int n_reqs, int batch, int64_t *d_idx, uint32_t *d_n_out,
+                                       void *stream) {
+    NFSP_CHECK_ARG(reqs && n_reqs >= 1 && n_reqs <= NFSP_MAX_SAMPLE_REQS, "1..%d requests", NFSP_MAX_SAMPLE_REQS);
+    NFSP_CHECK_ARG(batch >= 1 && batch <= kMaxBatch, "batch must be in [1,%d]", kMaxBatch);
+    const dim3 grid((unsigned)n_reqs, 8u, 1u);
+    if (n_reqs <= kSmallSampleReqs) {
+        SampleReqs R;
+        const int rc = fill_sample_table(reqs, n_reqs, d_idx, R);
+        if (rc != NFSP_OK) return rc;
+        sample_gather_kernel<<<grid, kBufThreads, 0, (cudaStream_t)stream>>>(R, batch, d_idx, d_n_out);
+    } else {
+        SampleReqsWide R;
+        const int rc = fill_sample_table(reqs, n_reqs, d_idx, R);
+        if (rc != NFSP_OK) return rc;
+        sample_gather_wide_kernel<<<grid, kBufThreads, 0, (cudaStream_t)stream>>>(R, batch, d_idx, d_n_out);
+    }
     NFSP_LAUNCH_CHECK();
     return NFSP_OK;
 }

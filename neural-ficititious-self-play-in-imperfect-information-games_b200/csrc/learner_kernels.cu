@@ -325,15 +325,24 @@ __device__ __forceinline__ float ld_volatile_f32(const float *p) {
     asm volatile("ld.volatile.global.f32 %0, [%1];" : "=f"(v) : "l"(p) : "memory");
     return v;
 }
-__global__ void __launch_bounds__(kLearnThreads)
-learner_fit_kernel(const FitArgs F) {
+// What a fit reads per run: the learner's arguments, the output weights and the four learning rates.  FitArgs carries the
+// same members for the single-run kernels; the step schedule (and the peers) always come from a FitArgs.
+struct FitRun {
+    LearnerArgs A;
+    float *w_out;
+    float lr[4];
+};
+
+// the register kernel's work on net `net` of run P
+template <class Run>
+__device__ __forceinline__ void fit_regs_net(const FitArgs &F, const Run &P, int net) {
     __shared__ float red_all[kRowGroups][4][2][4];
     __shared__ float part[kRowGroups][40][64];
-    const LearnerArgs &A = F.A;
-    const int net = blockIdx.x, j = threadIdx.x & 63;
+    const LearnerArgs &A = P.A;
+    const int j = threadIdx.x & 63;
     if (!((A.net_mask >> net) & 1)) {
-        if (F.w_out != A.w)
-            for (int e = threadIdx.x; e < NFSP_NET_PARAMS; e += kLearnThreads) F.w_out[net * NFSP_NET_PARAMS + e] = A.w[net * NFSP_NET_PARAMS + e];
+        if (P.w_out != A.w)
+            for (int e = threadIdx.x; e < NFSP_NET_PARAMS; e += kLearnThreads) P.w_out[net * NFSP_NET_PARAMS + e] = A.w[net * NFSP_NET_PARAMS + e];
         return;
     }
     __shared__ uint4 s_rec[kMaxFitRows];
@@ -341,7 +350,7 @@ learner_fit_kernel(const FitArgs F) {
     if (pre) prefetch_rows(A, net, 0, F.minibatch, s_rec);
     NetState N;
     N.load(A, net, j);
-    const float lr = F.lr[net];
+    const float lr = P.lr[net];
     for (int k = 0; k < F.n_steps; ++k) {
         step_sums(A, N, net, F.row0[k], F.rows[k], red_all, part, pre ? s_rec : nullptr, 0);
         if (k == 0) write_stats(A.stats, net, F.rows[k], part);
@@ -358,7 +367,7 @@ learner_fit_kernel(const FitArgs F) {
         __syncthreads();  // part[] is rewritten by the next step
     }
     if (threadIdx.x >= 64) return;
-    float *w = F.w_out + net * NFSP_NET_PARAMS;
+    float *w = P.w_out + net * NFSP_NET_PARAMS;
 #pragma unroll
     for (int i = 0; i < 30; ++i) w[i * 64 + j] = N.W.w1[i];
     w[1920 + j] = N.W.b1;
@@ -366,6 +375,8 @@ learner_fit_kernel(const FitArgs F) {
     for (int c = 0; c < 3; ++c) w[1984 + j * 3 + c] = N.W.w2[c];
     if (j < 3) w[2176 + j] = N.b2[j];
 }
+__global__ void __launch_bounds__(kLearnThreads)
+learner_fit_kernel(const FitArgs F) { fit_regs_net(F, F, blockIdx.x); }
 
 // ---- fit(), the row-parallel formulation ------------------------------------------------------------
 // The register kernel above is bound by instruction latency: a CTA of 256 threads per net, eight rows one after the
@@ -390,17 +401,18 @@ __device__ __forceinline__ void warp_sum9(float (&v)[9]) {
         for (int k = 0; k < 9; ++k) v[k] += __shfl_xor_sync(0xFFFFFFFFu, v[k], o);
     }
 }
-__global__ void __launch_bounds__(kRowThreads, 1)
-learner_fit_rows_kernel(const FitArgs F) {
+// the row-parallel kernel's work on net `net` of run P
+template <class Run>
+__device__ __forceinline__ void fit_rows_net(const FitArgs &F, const Run &P, int net) {
     extern __shared__ __align__(16) unsigned char fit_smem_raw[];
     RowFitSmem &S = *reinterpret_cast<RowFitSmem *>(fit_smem_raw);
     __shared__ int s_peer_lost;  // a peer did not answer within the time limit of the gradient exchange
-    const LearnerArgs &A = F.A;
-    const int net = blockIdx.x, player = net >> 1, is_br = net & 1, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const LearnerArgs &A = P.A;
+    const int player = net >> 1, is_br = net & 1, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (threadIdx.x == 0) s_peer_lost = 0;
     if (!((A.net_mask >> net) & 1)) {
-        if (F.w_out != A.w)
-            for (int e = threadIdx.x; e < NFSP_NET_PARAMS; e += kRowThreads) F.w_out[net * NFSP_NET_PARAMS + e] = A.w[net * NFSP_NET_PARAMS + e];
+        if (P.w_out != A.w)
+            for (int e = threadIdx.x; e < NFSP_NET_PARAMS; e += kRowThreads) P.w_out[net * NFSP_NET_PARAMS + e] = A.w[net * NFSP_NET_PARAMS + e];
         return;
     }
     for (int e = threadIdx.x; e < NFSP_NET_PARAMS; e += kRowThreads) {
@@ -408,7 +420,7 @@ learner_fit_rows_kernel(const FitArgs F) {
         if (is_br) S.wt[e] = A.w_target[player * NFSP_NET_PARAMS + e];
     }
     prefetch_rows(A, net, 0, F.minibatch, S.rec);  // ends with a CTA barrier
-    const float lr = F.lr[net];
+    const float lr = P.lr[net];
     for (int k = 0; k < F.n_steps; ++k) {
         const int row0 = F.row0[k], rows = F.rows[k];
         // phase 1: forward, loss, dz and dh of one row per warp
@@ -590,8 +602,20 @@ learner_fit_rows_kernel(const FitArgs F) {
         }
         __syncthreads();
     }
-    for (int e = threadIdx.x; e < NFSP_NET_PARAMS; e += kRowThreads) F.w_out[net * NFSP_NET_PARAMS + e] = S.w[e];
+    for (int e = threadIdx.x; e < NFSP_NET_PARAMS; e += kRowThreads) P.w_out[net * NFSP_NET_PARAMS + e] = S.w[e];
 }
+__global__ void __launch_bounds__(kRowThreads, 1)
+learner_fit_rows_kernel(const FitArgs F) { fit_rows_net(F, F, blockIdx.x); }
+
+// ---- the fits of independent runs in one launch (nfsp_learner_fit_runs): CTA 4 r + k = net k of run r ------------------
+struct FitRuns {
+    FitArgs F;  // the shared step schedule (world = 1); its A, w_out and lr are not read
+    FitRun run[NFSP_MAX_RUNS];
+};
+__global__ void __launch_bounds__(kLearnThreads)
+learner_fit_runs_kernel(const __grid_constant__ FitRuns R) { fit_regs_net(R.F, R.run[blockIdx.x >> 2], blockIdx.x & 3); }
+__global__ void __launch_bounds__(kRowThreads, 1)
+learner_fit_rows_runs_kernel(const __grid_constant__ FitRuns R) { fit_rows_net(R.F, R.run[blockIdx.x >> 2], blockIdx.x & 3); }
 
 // w[k] -= lr[k] * scale * grad[k]   (keras.optimizers.SGD without momentum, agent.py:45-46)
 __global__ void sgd_apply_kernel(float *__restrict__ w, const float *__restrict__ grad, float lr0, float lr1, float lr2,
@@ -636,6 +660,24 @@ extern "C" int nfsp_learner_grads(const nfsp_learner_io *io, void *stream) {
 static int learner_fit_impl(const nfsp_learner_io *io, int minibatch, int fit_batch, int epochs, const float lr[4],
                             float *d_weights_out, const nfsp_peers *peers, void *stream);
 
+// the SGD steps of Keras' fit(batch_size = fit_batch, epochs): slices [0, fit_batch), [fit_batch, 2 fit_batch), ... of the
+// minibatch, `epochs` times; one GPU, no peers
+static int fit_schedule(int minibatch, int fit_batch, int epochs, FitArgs &F) {
+    NFSP_CHECK_ARG(minibatch >= 1 && fit_batch >= 1 && epochs >= 1, "bad fit geometry");
+    F.minibatch = minibatch;
+    F.n_steps = 0;
+    for (int e = 0; e < epochs; ++e)
+        for (int row0 = 0; row0 < minibatch; row0 += fit_batch) {
+            NFSP_CHECK_ARG(F.n_steps < NFSP_MAX_FIT_STEPS, "more than %d SGD steps per fit", NFSP_MAX_FIT_STEPS);
+            F.row0[F.n_steps] = row0;
+            F.rows[F.n_steps] = minibatch - row0 < fit_batch ? minibatch - row0 : fit_batch;
+            ++F.n_steps;
+        }
+    F.world = 1; F.rank = 0; F.epoch0 = 0u; F.err = nullptr; F.mc = nullptr;
+    for (int r = 0; r < NFSP_MAX_PEERS; ++r) F.peer[r] = nullptr;
+    return NFSP_OK;
+}
+
 extern "C" int nfsp_learner_fit(const nfsp_learner_io *io, int minibatch, int fit_batch, int epochs, const float lr[4],
                                 float *d_weights_out, void *stream) {
     return learner_fit_impl(io, minibatch, fit_batch, epochs, lr, d_weights_out, nullptr, stream);
@@ -656,23 +698,13 @@ extern "C" int nfsp_learner_fit_peers(const nfsp_learner_io *io, int minibatch, 
 static int learner_fit_impl(const nfsp_learner_io *io, int minibatch, int fit_batch, int epochs, const float lr[4],
                             float *d_weights_out, const nfsp_peers *peers, void *stream) {
     NFSP_CHECK_ARG(lr && d_weights_out, "null argument");
-    NFSP_CHECK_ARG(minibatch >= 1 && fit_batch >= 1 && epochs >= 1, "bad fit geometry");
     FitArgs F;
-    const int rc = make_learner_args(io, F.A);
+    int rc = fit_schedule(minibatch, fit_batch, epochs, F);
+    if (rc != NFSP_OK) return rc;
+    rc = make_learner_args(io, F.A);
     if (rc != NFSP_OK) return rc;
     F.w_out = d_weights_out;
-    F.minibatch = minibatch;
-    F.n_steps = 0;
-    for (int e = 0; e < epochs; ++e)
-        for (int row0 = 0; row0 < minibatch; row0 += fit_batch) {
-            NFSP_CHECK_ARG(F.n_steps < NFSP_MAX_FIT_STEPS, "more than %d SGD steps per fit", NFSP_MAX_FIT_STEPS);
-            F.row0[F.n_steps] = row0;
-            F.rows[F.n_steps] = minibatch - row0 < fit_batch ? minibatch - row0 : fit_batch;
-            ++F.n_steps;
-        }
     for (int k = 0; k < 4; ++k) F.lr[k] = lr[k];
-    F.world = 1; F.rank = 0; F.epoch0 = 0u; F.err = nullptr; F.mc = nullptr;
-    for (int r = 0; r < NFSP_MAX_PEERS; ++r) F.peer[r] = nullptr;
     if (peers) {
         F.world = peers->world; F.rank = peers->rank; F.epoch0 = peers->epoch0; F.err = peers->d_err;
         F.mc = (float *)peers->d_mc;
@@ -684,6 +716,33 @@ static int learner_fit_impl(const nfsp_learner_io *io, int minibatch, int fit_ba
         learner_fit_rows_kernel<<<4, kRowThreads, sizeof(RowFitSmem), (cudaStream_t)stream>>>(F);
     } else {  // large batches: the register kernel
         learner_fit_kernel<<<4, kLearnThreads, 0, (cudaStream_t)stream>>>(F);
+    }
+    NFSP_LAUNCH_CHECK();
+    return NFSP_OK;
+}
+
+extern "C" int nfsp_learner_fit_runs(const nfsp_learner_io *io, int n_runs, int minibatch, int fit_batch, int epochs, const float *lr,
+                                     float *const *d_weights_out, void *stream) {
+    NFSP_CHECK_ARG(io && lr && d_weights_out, "null argument");
+    NFSP_CHECK_ARG(n_runs >= 1 && n_runs <= NFSP_MAX_RUNS, "n_runs must be in [1, %d]", NFSP_MAX_RUNS);
+    FitRuns R;
+    int rc = fit_schedule(minibatch, fit_batch, epochs, R.F);
+    if (rc != NFSP_OK) return rc;
+    R.F.A = LearnerArgs{};
+    R.F.w_out = nullptr;
+    for (int k = 0; k < 4; ++k) R.F.lr[k] = 0.f;
+    for (int r = 0; r < n_runs; ++r) {
+        NFSP_CHECK_ARG(d_weights_out[r], "null output weights of run %d", r);
+        rc = make_learner_args(io + r, R.run[r].A);
+        if (rc != NFSP_OK) return rc;
+        R.run[r].w_out = d_weights_out[r];
+        for (int k = 0; k < 4; ++k) R.run[r].lr[k] = lr[4 * r + k];
+    }
+    if (minibatch <= kMaxFitRows && fit_batch <= kMaxStepRows) {  // the same choice of kernel as nfsp_learner_fit
+        NFSP_CUDA(cudaFuncSetAttribute(learner_fit_rows_runs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RowFitSmem)));
+        learner_fit_rows_runs_kernel<<<4 * n_runs, kRowThreads, sizeof(RowFitSmem), (cudaStream_t)stream>>>(R);
+    } else {
+        learner_fit_runs_kernel<<<4 * n_runs, kLearnThreads, 0, (cudaStream_t)stream>>>(R);
     }
     NFSP_LAUNCH_CHECK();
     return NFSP_OK;

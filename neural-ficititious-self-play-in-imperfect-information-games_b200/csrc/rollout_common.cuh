@@ -28,6 +28,10 @@ int nfsp_states_ensure(nfsp_env_t h, const float *d_tab, float *d_states, cudaSt
 int nfsp_states_floats();
 int nfsp_states_upload_image(float *d_states);
 int nfsp_rollout_states_configure();
+// independent runs of one shape in one launch of the same rollout (nfsp_rollout_runs); A[r].pack = handle r's state table
+int nfsp_rollout_states_runs_launch(nfsp_env_t h, const nfsp::RolloutArgs *A, int n_runs, int sms, cudaStream_t st);
+// rebuilds the state tables of n handles from their table images in one launch and clears their st_dirty
+int nfsp_states_pack_runs(const nfsp_env_t *h, const float *const *tab, int n, cudaStream_t st);
 
 namespace nfsp {
 

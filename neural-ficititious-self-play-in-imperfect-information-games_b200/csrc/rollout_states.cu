@@ -50,7 +50,7 @@ __device__ __forceinline__ void state_rows(int s, uint32_t &xrow, uint32_t &yrow
 // One table slot per FOUR lanes: lane j of a quad takes hidden-unit quads j, j + 4, j + 8, j + 12 of mlp_forward_tables'
 // loop (two table rows added, relu, FFMA2 second layer), the three partial sums are combined with two shuffles, lane 0
 // applies the head.  All 20 loads of a lane are in flight at once: the launch is ~3 us on the step path.
-__global__ void states_pack_kernel(const float *__restrict__ tab, float4 *__restrict__ states) {
+__device__ __forceinline__ void states_pack(const float *__restrict__ tab, float4 *__restrict__ states) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x, e = t >> 2, j = t & 3;
     const bool valid = e < kStateQuads;  // the grid is a whole number of warps: every lane reaches the shuffles
     uint32_t xrow, yrow;
@@ -78,6 +78,14 @@ __global__ void states_pack_kernel(const float *__restrict__ tab, float4 *__rest
         states[e] = make_float4(o0, o1, o2, __uint_as_float(score_word(o0, o1, o2)));
     }
 }
+__global__ void states_pack_kernel(const float *__restrict__ tab, float4 *__restrict__ states) { states_pack(tab, states); }
+
+// the tables of several handles in one launch: blockIdx.y = run
+struct StatesRuns {
+    const float *tab[NFSP_MAX_RUNS];
+    float4 *states[NFSP_MAX_RUNS];
+};
+__global__ void states_pack_runs_kernel(const __grid_constant__ StatesRuns P) { states_pack(P.tab[blockIdx.y], P.states[blockIdx.y]); }
 
 // 1 024 threads per CTA for launches that keep every warp busy with several blocks of games; 512 (16 warps, 90 registers)
 // when the launch has no more blocks than that gives warps -- a warp then plays one block, and what counts is the latency
@@ -195,9 +203,21 @@ __device__ __forceinline__ void buf_append(WarpBuf &B, const RolloutArgs &A, con
     B.cnt += tot;
 }
 
-template <bool kDebug, bool kDirect, int kThreads>
-__global__ void __launch_bounds__(kThreads, 1)
-rollout_states_kernel(const RolloutArgs A) {
+// Which of the CTAs that serve A's games this CTA is: CTA c of n owns the blocks of 32 games c, c + n, c + 2 n, ... (every
+// SM gets its share however few games there are) and its warps take them dynamically.  A launch of one run: the grid.
+struct WholeGrid {
+    __device__ __forceinline__ uint32_t cta() const { return blockIdx.x; }
+    __device__ __forceinline__ uint32_t ctas() const { return gridDim.x; }
+};
+// one of several runs in a launch: a contiguous range of the grid
+struct RunRange {
+    uint32_t c, n;
+    __device__ __forceinline__ uint32_t cta() const { return c; }
+    __device__ __forceinline__ uint32_t ctas() const { return n; }
+};
+
+template <bool kDebug, bool kDirect, int kThreads, class Grid>
+__device__ __forceinline__ void rollout_states_cta(const RolloutArgs &A, const Grid &G) {
     extern __shared__ __align__(128) float4 s_tab[];  // kStateQuads, the rollout image, then the warps' record buffers
     __shared__ unsigned long long s_stats[NFSP_STATS_FIELDS];
     __shared__ __align__(8) uint64_t s_bar;
@@ -240,7 +260,7 @@ rollout_states_kernel(const RolloutArgs A) {
     const int64_t n_blocks = (A.n + 31) >> 5;  // CTA c owns blocks c, c + grid, ...; its warps take them dynamically
     for (;;) {
         uint32_t blk = 0;
-        if (lane == 0) blk = blockIdx.x + gridDim.x * atomicAdd(&s_next, 1u);
+        if (lane == 0) blk = G.cta() + G.ctas() * atomicAdd(&s_next, 1u);
         blk = __shfl_sync(0xFFFFFFFFu, blk, 0);
         if ((int64_t)blk >= n_blocks) break;
         const int64_t base = (int64_t)blk << 5;
@@ -349,6 +369,40 @@ rollout_states_kernel(const RolloutArgs A) {
     if (A.stats) c.wide.commit(s_stats, A.stats);
 }
 
+template <bool kDebug, bool kDirect, int kThreads>
+__global__ void __launch_bounds__(kThreads, 1)
+rollout_states_kernel(const RolloutArgs A) {
+    rollout_states_cta<kDebug, kDirect, kThreads>(A, WholeGrid{});
+}
+
+// ---- independent runs in one launch (nfsp_rollout_runs) -------------------------------------------
+// Runs of the same shape (game count, record mode) each get the same number of CTAs, in contiguous ranges of the grid:
+// CTA b serves run b / ctas_per_run as CTA b % ctas_per_run of ctas_per_run, with that run's state table, keys,
+// thresholds, game words, records and counters -- exactly what the run's own launch on ctas_per_run CTAs would do.
+// The run dimension is a compile-time bound on the argument table, which lives in the parameter space (~10 KB); a CTA
+// copies its run's entry to shared memory first (fewer registers than indexing the parameter space at every use).
+template <int kRuns>
+struct RolloutRuns {
+    RolloutArgs run[kRuns];
+    uint32_t ctas_per_run;
+};
+
+template <bool kDebug, bool kDirect, int kThreads, int kRuns>
+__global__ void __launch_bounds__(kThreads, 1)
+rollout_states_kernel(const __grid_constant__ RolloutRuns<kRuns> R) {
+    static_assert(!kDebug, "runs have no debug outputs");
+    static_assert(sizeof(RolloutArgs) % 4 == 0, "copied in words");
+    __shared__ __align__(16) RolloutArgs s_args;  // the run's arguments, read by the steps from shared memory
+    const uint32_t r = blockIdx.x / R.ctas_per_run;
+    {
+        const uint32_t *src = reinterpret_cast<const uint32_t *>(&R.run[r]);
+        uint32_t *dst = reinterpret_cast<uint32_t *>(&s_args);
+        for (int w = threadIdx.x; w < (int)(sizeof(RolloutArgs) / 4); w += kThreads) dst[w] = src[w];
+    }
+    __syncthreads();
+    rollout_states_cta<false, kDirect, kThreads>(s_args, RunRange{blockIdx.x - r * R.ctas_per_run, R.ctas_per_run});
+}
+
 }  // namespace nfsp
 
 using namespace nfsp;
@@ -405,6 +459,43 @@ static int launch_states(const RolloutArgs &A, int grid, bool debug, bool direct
     else rollout_states_kernel<false, false, kThreads><<<grid, kThreads, kBytes, st>>>(A);
     NFSP_LAUNCH_CHECK();
     return NFSP_OK;
+}
+
+// the state tables of n handles from their table images (tab[r] = handle r's, in its d_wpack), one launch
+int nfsp_states_pack_runs(const nfsp_env_t *h, const float *const *tab, int n, cudaStream_t st) {
+    StatesRuns P;
+    for (int r = 0; r < n; ++r) {
+        P.tab[r] = tab[r];
+        P.states[r] = reinterpret_cast<float4 *>(h[r]->d_states);
+    }
+    states_pack_runs_kernel<<<dim3((4 * kStateQuads + 127) / 128, (unsigned)n), 128, 0, st>>>(P);
+    NFSP_LAUNCH_CHECK();
+    for (int r = 0; r < n; ++r) h[r]->st_dirty = false;
+    return NFSP_OK;
+}
+
+template <bool kDirect, int kThreads>
+static int launch_states_runs(const RolloutArgs *A, int n_runs, int ctas_per_run, cudaStream_t st) {
+    constexpr int kBytes = states_smem_bytes(kThreads);
+    using Kernel = void (*)(RolloutRuns<NFSP_MAX_RUNS>);
+    const Kernel k = rollout_states_kernel<false, kDirect, kThreads, NFSP_MAX_RUNS>;
+    // per call: the attribute belongs to the current device's context
+    NFSP_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, kBytes));
+    RolloutRuns<NFSP_MAX_RUNS> R;
+    for (int r = 0; r < n_runs; ++r) R.run[r] = A[r];
+    R.ctas_per_run = (uint32_t)ctas_per_run;
+    k<<<n_runs * ctas_per_run, kThreads, kBytes, st>>>(R);
+    NFSP_LAUNCH_CHECK();
+    return NFSP_OK;
+}
+
+// n_runs runs of h->n games each, of one record mode (A[r].ring[0] != null for all or none); sms = SMs the grid may use.
+// Always 512 threads per CTA: a run's arguments are no longer constant-bank operands (the 20 Philox round keys alone), and
+// at 1 024 threads' 64 registers that spilled; at 512 the kernel holds them without spills (ptxas log).
+int nfsp_rollout_states_runs_launch(nfsp_env_t h, const RolloutArgs *A, int n_runs, int sms, cudaStream_t st) {
+    const int ctas = grid_for(h->n, 32, sms / n_runs, 1);  // at least one block of 32 games per CTA
+    return A[0].ring[0] != nullptr ? launch_states_runs<true, kStatesThreadsSmall>(A, n_runs, ctas, st)
+                                   : launch_states_runs<false, kStatesThreadsSmall>(A, n_runs, ctas, st);
 }
 
 int nfsp_rollout_states_launch(nfsp_env_t h, const RolloutArgs &A, const nfsp_rollout_io *io, bool debug, cudaStream_t st) {

@@ -114,6 +114,22 @@ class Learner:
         snapshot: the launch also copies the sampled slots out of the memories; the fit then reads those copies.
         which = "rl" / "sl": only the two rings / the two reservoirs (the pipelined trainer samples the rings as soon as
         the rollout has written them and the reservoirs after the insert launch); "rl" returns nothing."""
+        b = self.minibatch
+        lo, hi = self._sample_requests(snapshot, which)
+        g_rl, g_sl, rows = self._snapshot_buffers() if snapshot else (None, None, None)
+        first = C.cast(C.byref(self._pos_reqs, lo * C.sizeof(_lib.SampleReq)), C.POINTER(_lib.SampleReq))
+        check(lib().nfsp_sample_minibatches(first, hi - lo, b, _ptr(self._pos[lo:]), None, _stream(self.device)))
+        if which == "rl":
+            return None
+        if snapshot:  # the sampled slots are rows 0 .. b-1 of the snapshots
+            self._mems = (g_rl, g_sl)
+            return [rows, rows], [rows, rows]
+        self._mems = None
+        return [self._pos[0], self._pos[1]], [self._pos[2], self._pos[3]]
+
+    def _sample_requests(self, snapshot=False, which="both"):
+        """The sampling requests of _sample_positions (self._pos_reqs, rows rl0, rl1, sl0, sl1), their memories' draw
+        counters advanced; nothing is launched.  Returns the range [lo, hi) of the requests `which` names."""
         sp, b = self.sp, self.minibatch
         if not hasattr(self, "_pos"):
             self._pos = torch.empty((4, b), dtype=torch.int64, device=self.device)   # rows: rl0, rl1, sl0, sl1
@@ -131,15 +147,7 @@ class Learner:
                 r.call_idx = mem.sample_calls
                 r.d_rec_out = None if not snapshot else (g_rl[k] if k < 2 else g_sl[k - 2]).data_ptr()
                 mem.sample_calls += 1
-        first = C.cast(C.byref(self._pos_reqs, lo * C.sizeof(_lib.SampleReq)), C.POINTER(_lib.SampleReq))
-        check(lib().nfsp_sample_minibatches(first, hi - lo, b, _ptr(self._pos[lo:]), None, _stream(self.device)))
-        if which == "rl":
-            return None
-        if snapshot:  # the sampled slots are rows 0 .. b-1 of the snapshots
-            self._mems = (g_rl, g_sl)
-            return [rows, rows], [rows, rows]
-        self._mems = None
-        return [self._pos[0], self._pos[1]], [self._pos[2], self._pos[3]]
+        return lo, hi
 
     def presample_rings(self):
         """First half of an update for the pipelined trainer: draw the RL minibatches of both players and snapshot their
@@ -346,9 +354,7 @@ class Learner:
             if weights_out is not None:
                 weights_out.copy_(sp.weights if weights_in is None else weights_in)
             return {"trained": 0}
-        for p in range(2):
-            if (mask >> (2 * p + 1)) & 1:
-                self.iteration[p] += 1          # agent.py:216
+        self._begin_update(mask)
         if presampled_rings and on_gathered is None:
             raise ValueError("presampled_rings belongs to the snapshot path (on_gathered)")
         idx_rl, idx_sl = self._sample_positions(snapshot=on_gathered is not None, which="sl" if presampled_rings else "both")
@@ -368,6 +374,20 @@ class Learner:
                     self._step(idx_rl, idx_sl, row0, min(self.fit_batch, self.minibatch - row0), mask)
                     if stats is None:            # exploitability proxy of the sampled batch, first pass
                         stats = self.flat[GRAD:].clone()
+        return self._finish_update(mask, stats, sync, w_new, pack)
+
+    def _begin_update(self, mask):
+        """First half of update() once the ready mask is known (non-zero): agent.py:216's iteration step.  The sampling
+        and the fit follow; _finish_update() is the second half."""
+        for p in range(2):
+            if (mask >> (2 * p + 1)) & 1:
+                self.iteration[p] += 1          # agent.py:216
+
+    def _finish_update(self, mask, stats, sync, w_new, pack):
+        """Second half of update(), after the fit wrote w_new and its first step's statistics `stats` (a device tensor):
+        the statistics (read back with sync), then each player's schedules -- iteration, temperature, target-net copy,
+        learning-rate decay, epsilon -- and (pack) the acting images rebuilt."""
+        sp = self.sp
         if sync:
             self._loss = stats.cpu().tolist()
         if sync or (self._peers is not None and (self.updates + 1) % self.peer_check_every == 0):

@@ -2,6 +2,7 @@
 
     python -m nfsp_b200.main [--games N] [--episodes E] [--steps-per-call T] [--config ./config.ini]
     python -m torch.distributed.run --nproc-per-node G -m nfsp_b200.main ...     # games sharded over G GPUs
+    python -m nfsp_b200.main --runs R ...     # R independent runs (seeds Seed, Seed + 1, ...) side by side on one GPU
 
 The reference plays one hand at a time: `train(env, player1, player2)` alternates the dealer, draws each
 player's per-hand policy with probability eta, lets the agents `play` until both have seen the terminal
@@ -18,6 +19,7 @@ reads), same seeds, same printed quantities.  `--human` is accepted and ignored,
 from __future__ import annotations
 
 import argparse
+import statistics
 import time
 
 import torch
@@ -27,6 +29,7 @@ from .batched import SelfPlay
 from .config import load_config
 from .exploitability import exploitability
 from .learner import Learner, PipelinedTrainer
+from .runs import RunBatch
 
 
 def sampled_actions(stats, player):
@@ -84,6 +87,48 @@ def train(sp: SelfPlay, learner: Learner, episodes: int, steps_per_call: int = 8
             return rows
 
 
+def train_runs(rb: RunBatch, episodes: int, steps_per_call: int = 8, report_every: int = 100, log=print,
+               true_exploitability: bool = True):
+    """train() for the independent runs of a RunBatch: one batched iteration per call, until every run has played
+    `episodes` hands.  A reported row carries each run's values under "runs" and, with true_exploitability, the mean
+    and standard deviation of the runs' exact exploitability."""
+    rows, calls, t0 = [], 0, time.time()
+    while True:
+        calls += 1
+        report = calls % report_every == 0 or calls == 1
+        sts = rb.step(steps_per_call, sync=report)
+        if not report:
+            continue
+        runs = []
+        for sp, st in zip(rb.sps, sts):
+            stats = sp.read_stats()
+            runs.append({"seed": sp.env.seed, "hands": stats["hands"], "transitions": stats["transitions"],
+                         "exploitability_proxy": st.get("exploitability"),
+                         "actions": [sampled_actions(stats, p) for p in range(2)]})
+        row = {"calls": calls, "runs": runs, "hands": sum(r["hands"] for r in runs),
+               "transitions": sum(r["transitions"] for r in runs)}
+        row["transitions_per_sec"] = row["transitions"] / max(time.time() - t0, 1e-9)
+        if true_exploitability:
+            for run, e in zip(runs, rb.exploitability()):
+                run["exploitability"] = e
+            values = [r["exploitability"]["value"] for r in runs]
+            row["exploitability_mean"] = statistics.fmean(values)
+            row["exploitability_std"] = statistics.stdev(values) if len(values) > 1 else 0.0
+        rows.append(row)
+        log("================ Stats ==================")
+        for k, run in enumerate(runs):
+            line = "run %d (seed %d): hands %d  exploitability proxy %s" % (k, run["seed"], run["hands"], run["exploitability_proxy"])
+            if true_exploitability:
+                line += "  exact exploitability %.4f chips/hand" % run["exploitability"]["value"]
+            log(line)
+        if true_exploitability:
+            log("Exact exploitability over %d runs: mean %.4f  std %.4f chips/hand" %
+                (len(runs), row["exploitability_mean"], row["exploitability_std"]))
+        log("hands %d  transitions %d  (%.3e transitions/s)" % (row["hands"], row["transitions"], row["transitions_per_sec"]))
+        if min(r["hands"] for r in runs) >= episodes:
+            return rows
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(description="NFSP self-play on Leduc Hold'em, B200-native")
     ap.add_argument("--human", action="store_true", help="accepted and ignored, as in the reference (main.py:152-158)")
@@ -104,9 +149,15 @@ def main(argv=None):
                     help="rollout kernel: the nets tabulated over the game's decision states (default) or evaluated per decision")
     ap.add_argument("--updates-per-call", type=int, default=1,
                     help="update_strategy() calls per rollout call (the reference's cadence: games * steps / 256)")
+    ap.add_argument("--runs", type=int, default=1,
+                    help="independent runs with seeds Seed, Seed + 1, ... trained side by side on one GPU, their launches shared")
     args = ap.parse_args(argv)
     cfg = load_config(args.config)
     rank, world, local = sharding.env_rank_world()
+    if args.runs < 1:
+        ap.error("--runs must be at least 1")
+    if args.runs > 1 and (args.pipelined or world > 1):
+        ap.error("--runs > 1 trains on one GPU with the sequential loop: not with --pipelined or more than one rank")
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     if world > 1:
@@ -115,12 +166,21 @@ def main(argv=None):
         dist.init_process_group("nccl", device_id=dev)
     seed = cfg.getint("Utils", "Seed")              # main.py:132-133
     game0, n = sharding.shard_games(args.games, rank, world)
-    sp = SelfPlay(n, seed=seed, game0=game0, device=dev, eta=cfg.getfloat("Agent", "Eta"),
-                  epsilon=cfg.getfloat("Agent", "Epsilon"), rl_capacity=cfg.getint("Agent", "MRLSize"),
-                  sl_capacity=cfg.getint("Agent", "MSLSize"), max_steps_per_call=args.steps_per_call,
-                  deterministic=args.deterministic, direct_rings=False if args.deterministic else "auto", variant=args.variant)
-    learner = Learner(sp, cfg=cfg, terminal_bootstraps=args.terminal_bootstraps, others_to_target=args.others_to_target)
     episodes = args.episodes if args.episodes is not None else cfg.getint("Common", "Episodes")
+
+    def make_run(run_seed):
+        sp_ = SelfPlay(n, seed=run_seed, game0=game0, device=dev, eta=cfg.getfloat("Agent", "Eta"),
+                       epsilon=cfg.getfloat("Agent", "Epsilon"), rl_capacity=cfg.getint("Agent", "MRLSize"),
+                       sl_capacity=cfg.getint("Agent", "MSLSize"), max_steps_per_call=args.steps_per_call,
+                       deterministic=args.deterministic, direct_rings=False if args.deterministic else "auto",
+                       variant=args.variant)
+        return sp_, Learner(sp_, cfg=cfg, terminal_bootstraps=args.terminal_bootstraps, others_to_target=args.others_to_target)
+
+    if args.runs > 1:
+        rb = RunBatch(*zip(*[make_run(seed + r) for r in range(args.runs)]))
+        return train_runs(rb, episodes, args.steps_per_call, args.report_every,
+                          true_exploitability=not args.no_true_exploitability)
+    sp, learner = make_run(seed)
     rows = train(sp, learner, episodes, args.steps_per_call, args.report_every, world,
                  log=print if rank == 0 else (lambda *a, **k: None),
                  true_exploitability=not args.no_true_exploitability, pipelined=args.pipelined,
