@@ -293,7 +293,8 @@ int nfsp_sample_indices(uint64_t seed, uint64_t call_idx, const uint64_t *d_tota
  * one contiguous block: ring (RL)  s[batch][30] a[batch][3] r[batch] s2[batch][30] t[batch]  = 65 * batch floats,
  * reservoir (SL)  s[batch][30] a[batch][3]  = 33 * batch floats.  d_idx int64[n_reqs][batch] (storage slots, -1 beyond
  * the records held) and d_n_out uint32[n_reqs] (rows sampled) may be NULL.  A request with d_out = NULL only reports its
- * positions in d_idx (the learner kernels read the packed records themselves). */
+ * positions in d_idx (the learner kernels read the packed records themselves); with d_rec_out NULL as well it reads no
+ * record and d_mem may be NULL. */
 #define NFSP_MAX_SAMPLE_REQS 128 /* 4 * NFSP_MAX_RUNS: the four memories of every run of a batch */
 typedef struct {
     const void *d_mem;        /* ring (16-byte records) / reservoir (32-byte slots, the record first) storage */
@@ -361,7 +362,12 @@ int nfsp_learner_fit_runs(const nfsp_learner_io *io, int n_runs, int minibatch, 
  * round trip), then sums them in rank order -- so the weights stay bit-identical on every rank.  epoch0 = SGD steps
  * exchanged through these buffers so far (the same on all ranks; add the steps of this call afterwards).  *d_err becomes
  * 1 if a peer did not answer within ~2 s (the kernel then gives up on that net instead of hanging the GPU and writes NaN
- * weights for it: the result is invalid and visibly so).  Every rank must make the same call. */
+ * weights for it: the result is invalid and visibly so).  Every rank must make the same call.
+ * The exchange lives in the row-parallel fit kernel (one warp per sampled row, the weights in shared memory), which holds
+ * at most NFSP_FIT_ROWS_MAX_MINIBATCH sampled rows and NFSP_FIT_ROWS_MAX_STEP rows per SGD step: larger geometries are
+ * refused here.  nfsp_learner_fit and nfsp_learner_fit_runs run them on the register kernel instead. */
+#define NFSP_FIT_ROWS_MAX_MINIBATCH 256
+#define NFSP_FIT_ROWS_MAX_STEP 64
 #define NFSP_MAX_PEERS 8
 #define NFSP_PEER_BUF_FLOATS 279552 /* 2 parities x 4 nets x NFSP_MAX_PEERS senders x 2184 words of 8 bytes */
 typedef struct {

@@ -58,6 +58,7 @@ class Peers(C.Structure):
 
 
 MAX_RUNS, MAX_SAMPLE_REQS = 32, 128  # NFSP_MAX_RUNS, NFSP_MAX_SAMPLE_REQS (= 4 * NFSP_MAX_RUNS)
+FIT_ROWS_MAX_MINIBATCH, FIT_ROWS_MAX_STEP = 256, 64  # NFSP_FIT_ROWS_MAX_MINIBATCH, NFSP_FIT_ROWS_MAX_STEP (row-parallel fit)
 
 
 class SampleReq(C.Structure):

@@ -282,12 +282,22 @@ class _Memory:
         """count saturates at capacity (replay_buffer.py:36-44).  Reads one device word (syncs)."""
         return int(min(int(self.total.item()), self.capacity))
 
+    def sample_req(self, r):
+        """Fills the fields of the nfsp_sample_req r that never change (memory, seed, kind); returns r."""
+        r.d_mem, r.d_total, r.cap = self.store.data_ptr(), self.total.data_ptr(), self.capacity
+        r.seed, r.is_ring = self.seed, int(self.is_ring)
+        return r
+
+    def next_call(self) -> int:
+        """The draw counter (Philox key with the seed) of this memory's next sample_batch, advanced."""
+        self.sample_calls += 1
+        return self.sample_calls - 1
+
     def sample_slots(self, batch: int):
         idx = torch.empty(batch, dtype=torch.int64, device=self.device)
         n = torch.zeros(1, dtype=torch.int32, device=self.device)
-        check(lib().nfsp_sample_indices(self.seed, self.sample_calls, _ptr(self.total), self.capacity,
+        check(lib().nfsp_sample_indices(self.seed, self.next_call(), _ptr(self.total), self.capacity,
                                         int(self.is_ring), batch, _ptr(idx), _ptr(n), _stream(self.device)))
-        self.sample_calls += 1
         return idx, n
 
     def records(self) -> np.ndarray:
@@ -646,18 +656,14 @@ class SelfPlay:
             reqs = (_lib.SampleReq * 4)()
             for p in range(2):
                 for k, mem in ((0, self.rl[p]), (1, self.sl[p])):
-                    r = reqs[2 * p + k]
-                    r.d_mem, r.d_total, r.cap = mem.store.data_ptr(), mem.total.data_ptr(), mem.capacity
-                    r.seed, r.is_ring = mem.seed, int(mem.is_ring)
-                    r.d_out = slab.data_ptr() + 4 * (p * per + k * 65 * b)
+                    mem.sample_req(reqs[2 * p + k]).d_out = slab.data_ptr() + 4 * (p * per + k * 65 * b)
             views = {src is host: [{k: src[o:o + n].view(shape) for k, (o, n, shape) in spec.items()} for spec in layout]
                      for src in (slab, host)}
             cache[lkey] = (reqs, views)
         reqs, views = cache[lkey]
         for p in range(2):
             for k, mem in ((0, self.rl[p]), (1, self.sl[p])):
-                reqs[2 * p + k].call_idx = mem.sample_calls
-                mem.sample_calls += 1
+                reqs[2 * p + k].call_idx = mem.next_call()
         check(lib().nfsp_sample_minibatches(reqs, 4, b, _ptr(idx), _ptr(cnt), st))
         if to_host:
             host.copy_(slab, non_blocking=True)

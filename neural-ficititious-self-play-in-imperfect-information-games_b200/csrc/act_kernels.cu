@@ -54,7 +54,12 @@ __device__ __forceinline__ void pack_images(const float *__restrict__ w, float *
     for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < kImages + 4 * NFSP_NET_PARAMS; e += gridDim.x * blockDim.x)
         pack[e] = e < kPackFloats ? pack_weights_value(w, e) : (e < kImages ? pack_tables_value(w, e - kPackFloats) : w[e - kImages]);
 }
-__global__ void pack_images_kernel(const float *__restrict__ w, float *__restrict__ pack) { pack_images(w, pack); }
+// the images of 1..NFSP_MAX_RUNS handles in one launch: blockIdx.y = handle
+struct ImageRuns {
+    const float *w[NFSP_MAX_RUNS];
+    float *pack[NFSP_MAX_RUNS];
+};
+__global__ void pack_images_kernel(const __grid_constant__ ImageRuns P) { pack_images(P.w[blockIdx.y], P.pack[blockIdx.y]); }
 
 // forward of one net on one observation mask; sw = packed image in shared memory.  The first layer is the sum of the
 // <= 10 weight rows of the set input bits (+ the bias row), accumulated in the thread's ROTATED quad order.
@@ -178,16 +183,36 @@ rollout_kernel(const RolloutArgs A) {
     if (A.stats) c.wide.commit(s_stats, A.stats);
 }
 
-// the images of several handles in one launch (nfsp_rollout_runs): blockIdx.y = run
-struct ImageRuns {
-    const float *w[NFSP_MAX_RUNS];
-    float *pack[NFSP_MAX_RUNS];
-};
-__global__ void pack_images_runs_kernel(const __grid_constant__ ImageRuns P) { pack_images(P.w[blockIdx.y], P.pack[blockIdx.y]); }
-
 }  // namespace nfsp
 
 using namespace nfsp;
+
+// nfsp_act_set_weights of n handles whose buffers exist: handle r's images from w[r], then the default rollout's table of
+// the nets' outputs per decision state from the table image just built -- one launch each, whatever n.  The tensor-core
+// variants' images follow lazily (nfsp_ensure_tc_images).
+static int rebuild_images(const nfsp_env_t *h, const float *const *w, int n, cudaStream_t st) {
+    ImageRuns P;
+    const float *tab[NFSP_MAX_RUNS];
+    for (int r = 0; r < n; ++r) {
+        P.w[r] = w[r];
+        P.pack[r] = h[r]->d_wpack;
+        tab[r] = h[r]->d_wpack + kPackFloats;
+    }
+    pack_images_kernel<<<dim3((kPackFloats + kTabImageFloats + 4 * NFSP_NET_PARAMS + 255) / 256, (unsigned)n), 256, 0, st>>>(P);
+    NFSP_LAUNCH_CHECK();
+    for (int r = 0; r < n; ++r) {
+        h[r]->tc_dirty = h[r]->tq_dirty = h[r]->st_dirty = true;
+        h[r]->has_weights = true;
+    }
+    return nfsp_states_pack(h, tab, n, st);  // clears st_dirty
+}
+
+// the state table alone, when it is older than the table image
+static int states_ensure(nfsp_env_t h, cudaStream_t st) {
+    if (!h->st_dirty) return NFSP_OK;
+    const float *tab = h->d_wpack + kPackFloats;
+    return nfsp_states_pack(&h, &tab, 1, st);
+}
 
 extern "C" int nfsp_act_set_weights(nfsp_env_t h, const float *d_weights, void *stream) {
     NFSP_CHECK_ARG(h != nullptr && d_weights != nullptr, "null argument");
@@ -213,12 +238,7 @@ extern "C" int nfsp_act_set_weights(nfsp_env_t h, const float *d_weights, void *
         rc = nfsp_states_upload_image(h->d_states);
         if (rc != NFSP_OK) return rc;
     }
-    pack_images_kernel<<<(kPackFloats + kTabImageFloats + 4 * NFSP_NET_PARAMS + 255) / 256, 256, 0, (cudaStream_t)stream>>>(d_weights, h->d_wpack);
-    NFSP_LAUNCH_CHECK();
-    h->tc_dirty = h->tq_dirty = h->st_dirty = true;
-    h->has_weights = true;
-    // the default rollout's table of the nets' outputs per decision state, from the table image just built
-    return nfsp_states_ensure(h, h->d_wpack + kPackFloats, h->d_states, (cudaStream_t)stream);
+    return rebuild_images(&h, &d_weights, 1, (cudaStream_t)stream);
 }
 
 int nfsp_ensure_tc_images(nfsp_env_t h, bool tq, cudaStream_t st) {
@@ -329,7 +349,7 @@ extern "C" int nfsp_rollout(nfsp_env_t h, int n_steps, double eta, double epsilo
     DeviceGuard guard(h->device);
     if (!guard.ok) return set_error(NFSP_E_CUDA, "cannot select device %d", h->device);
     if (variant == 6) {
-        int rc = nfsp_states_ensure(h, h->d_wpack + kPackFloats, h->d_states, (cudaStream_t)stream);
+        int rc = states_ensure(h, (cudaStream_t)stream);
         if (rc != NFSP_OK) return rc;
         A.pack = h->d_states;
         rc = nfsp_rollout_states_launch(h, A, io, debug, (cudaStream_t)stream);
@@ -411,24 +431,13 @@ extern "C" int nfsp_rollout_runs(const nfsp_env_t *h, int n_runs, int n_steps, c
     DeviceGuard guard(h[0]->device);
     if (!guard.ok) return set_error(NFSP_E_CUDA, "cannot select device %d", h[0]->device);
     const cudaStream_t st = (cudaStream_t)stream;
-    if (d_weights) {  // nfsp_act_set_weights of every run: the images, then the state tables, one launch each
-        ImageRuns P;
-        const float *tab[NFSP_MAX_RUNS];
-        for (int r = 0; r < n_runs; ++r) {
-            P.w[r] = d_weights[r];
-            P.pack[r] = h[r]->d_wpack;
-            tab[r] = h[r]->d_wpack + kPackFloats;
-        }
-        pack_images_runs_kernel<<<dim3((kPackFloats + kTabImageFloats + 4 * NFSP_NET_PARAMS + 255) / 256, (unsigned)n_runs), 256, 0, st>>>(P);
-        NFSP_LAUNCH_CHECK();
-        for (int r = 0; r < n_runs; ++r) h[r]->tc_dirty = h[r]->tq_dirty = h[r]->st_dirty = true;
-        const int rc = nfsp_states_pack_runs(h, tab, n_runs, st);
+    if (d_weights) {  // nfsp_act_set_weights of every run
+        const int rc = rebuild_images(h, d_weights, n_runs, st);
         if (rc != NFSP_OK) return rc;
-    } else {
-        for (int r = 0; r < n_runs; ++r) {
-            const int rc = nfsp_states_ensure(h[r], h[r]->d_wpack + kPackFloats, h[r]->d_states, st);
-            if (rc != NFSP_OK) return rc;
-        }
+    }
+    for (int r = 0; r < n_runs; ++r) {
+        const int rc = states_ensure(h[r], st);
+        if (rc != NFSP_OK) return rc;
     }
     const int rc = nfsp_rollout_states_runs_launch(h[0], A, n_runs, sms, st);
     if (rc != NFSP_OK) return rc;

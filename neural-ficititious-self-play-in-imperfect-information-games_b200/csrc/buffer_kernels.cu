@@ -351,15 +351,6 @@ __device__ __forceinline__ int floyd_sample(uint64_t seed, uint64_t call_idx, ui
     return b;
 }
 
-__global__ void __launch_bounds__(kBufThreads)
-sample_kernel(uint64_t seed, uint64_t call_idx, const uint64_t *__restrict__ total_p, uint64_t cap, int is_ring,
-              int batch, int64_t *__restrict__ idx_out, uint32_t *__restrict__ n_out) {
-    __shared__ uint64_t draw[kMaxBatch];
-    __shared__ uint64_t pick[kMaxBatch];
-    const int b = floyd_sample(seed, call_idx, *total_p, cap, is_ring, batch, draw, pick, idx_out);
-    if (threadIdx.x == 0 && n_out) *n_out = (uint32_t)b;
-}
-
 // one output element of a sampled RL / SL row (the dense views of replay_buffer.py:46-59 / ReservoirBuffer.py:33-43)
 __device__ __forceinline__ void expand_rl(const uint4 rec, int row, int col, float *__restrict__ s, float *__restrict__ a,
                                           float *__restrict__ r, float *__restrict__ s2, float *__restrict__ t) {
@@ -578,18 +569,16 @@ extern "C" int nfsp_reservoir_insert(void *d_res, int64_t cap, uint64_t *d_total
 
 extern "C" int nfsp_sample_indices(uint64_t seed, uint64_t call_idx, const uint64_t *d_total, int64_t cap,
                                    int is_ring, int batch, int64_t *d_idx, uint32_t *d_n_out, void *stream) {
-    NFSP_CHECK_ARG(d_total && d_idx && cap > 0, "bad arguments");
-    NFSP_CHECK_ARG(batch >= 1 && batch <= kMaxBatch, "batch must be in [1,%d]", kMaxBatch);
-    sample_kernel<<<1, kBufThreads, 0, (cudaStream_t)stream>>>(seed, call_idx, d_total, (uint64_t)cap, is_ring, batch,
-                                                               d_idx, d_n_out);
-    NFSP_LAUNCH_CHECK();
-    return NFSP_OK;
+    nfsp_sample_req r{};  // positions only: no memory is read
+    r.d_total = d_total; r.cap = cap; r.seed = seed; r.call_idx = call_idx; r.is_ring = is_ring;
+    return nfsp_sample_minibatches(&r, 1, batch, d_idx, d_n_out, stream);
 }
 
 template <int kReqs>
 static int fill_sample_table(const nfsp_sample_req *reqs, int n_reqs, const int64_t *d_idx, SampleTable<kReqs> &R) {
     for (int m = 0; m < n_reqs; ++m) {
-        NFSP_CHECK_ARG(reqs[m].d_mem && reqs[m].d_total && reqs[m].cap > 0, "bad request %d", m);
+        const bool reads_mem = reqs[m].d_out || reqs[m].d_rec_out;
+        NFSP_CHECK_ARG((reqs[m].d_mem || !reads_mem) && reqs[m].d_total && reqs[m].cap > 0, "bad request %d", m);
         NFSP_CHECK_ARG(reqs[m].d_out || reqs[m].d_rec_out || d_idx, "request %d has neither an output block nor an index array", m);
         R.mem[m] = (const uint4 *)reqs[m].d_mem;
         R.total[m] = reqs[m].d_total;

@@ -113,7 +113,7 @@ struct NetState {
 // part[0][34][0..4] those of b2, the loss sum and the exploitability-proxy sum.
 // s_rec: the net's sampled records of rows [s_base, s_base + kMaxFitRows) prefetched into shared memory (the two
 // dependent global reads per row -- index, then record -- were most of a row's latency), or nullptr.
-constexpr int kMaxFitRows = 256;
+constexpr int kMaxFitRows = NFSP_FIT_ROWS_MAX_MINIBATCH;
 __device__ __forceinline__ void prefetch_rows(const LearnerArgs &A, int net, int base, int rows, uint4 *s_rec) {
     const int player = net >> 1;
     const uint4 *mem = (net & 1) ? A.rl[player] : A.sl[player];
@@ -274,18 +274,22 @@ learner_grad_kernel(const LearnerArgs A) {
 // [row0_k, row0_k + rows_k) of the sampled minibatch, each step = the sums above, then w -= lr * mean gradient applied
 // to the weights every thread holds in registers (all row groups keep the same copy).  The statistics are those of the
 // first step, as the host-driven sequence reports them.
-struct FitArgs {
-    LearnerArgs A;
-    float *w_out;  // [4][2179], may alias A.w
+// The step schedule (and, with several GPUs, the peers): shared by every run of a launch.
+struct FitSchedule {
     int n_steps, minibatch;
     int row0[NFSP_MAX_FIT_STEPS], rows[NFSP_MAX_FIT_STEPS];
-    float lr[4];
     // several GPUs training together: every rank's exchange buffer as this process sees it (peer memory over NVLink)
     int world, rank;
     float *peer[NFSP_MAX_PEERS];
     uint32_t epoch0;     // SGD steps exchanged through these buffers so far
     uint32_t *err;       // set to 1 if a peer did not answer in time
     float *mc;           // multicast mapping of all ranks' buffers (NVLS), or null
+};
+// What a fit reads per run: the learner's arguments, the output weights and the four learning rates.
+struct FitRun {
+    LearnerArgs A;
+    float *w_out;  // [4][2179], may alias A.w
+    float lr[4];
 };
 
 // Exchange buffer of one rank (the RECEIVER owns it): two parities x four nets x one slot per sending rank of kPeerSlot
@@ -325,17 +329,8 @@ __device__ __forceinline__ float ld_volatile_f32(const float *p) {
     asm volatile("ld.volatile.global.f32 %0, [%1];" : "=f"(v) : "l"(p) : "memory");
     return v;
 }
-// What a fit reads per run: the learner's arguments, the output weights and the four learning rates.  FitArgs carries the
-// same members for the single-run kernels; the step schedule (and the peers) always come from a FitArgs.
-struct FitRun {
-    LearnerArgs A;
-    float *w_out;
-    float lr[4];
-};
-
 // the register kernel's work on net `net` of run P
-template <class Run>
-__device__ __forceinline__ void fit_regs_net(const FitArgs &F, const Run &P, int net) {
+__device__ __forceinline__ void fit_regs_net(const FitSchedule &F, const FitRun &P, int net) {
     __shared__ float red_all[kRowGroups][4][2][4];
     __shared__ float part[kRowGroups][40][64];
     const LearnerArgs &A = P.A;
@@ -376,7 +371,7 @@ __device__ __forceinline__ void fit_regs_net(const FitArgs &F, const Run &P, int
     if (j < 3) w[2176 + j] = N.b2[j];
 }
 __global__ void __launch_bounds__(kLearnThreads)
-learner_fit_kernel(const FitArgs F) { fit_regs_net(F, F, blockIdx.x); }
+learner_fit_kernel(const FitSchedule S, const FitRun P) { fit_regs_net(S, P, blockIdx.x); }
 
 // ---- fit(), the row-parallel formulation ------------------------------------------------------------
 // The register kernel above is bound by instruction latency: a CTA of 256 threads per net, eight rows one after the
@@ -385,7 +380,7 @@ learner_fit_kernel(const FitArgs F) { fit_regs_net(F, F, blockIdx.x); }
 // reference's flat layout, so the hidden layer is one conflict-free LDS per SET input bit (<= 10) in the same order
 // as the register kernel adds them.  A second phase assembles the gradient of each weight from the rows' dh / h / dz in
 // row order and applies the SGD update in place.  Two barriers per SGD step.
-constexpr int kRowThreads = 1024, kRowWarps = kRowThreads / 32, kMaxStepRows = 64;
+constexpr int kRowThreads = 1024, kRowWarps = kRowThreads / 32, kMaxStepRows = NFSP_FIT_ROWS_MAX_STEP;
 struct RowFitSmem {
     float w[2180], wt[2180];          // online net, target net (best response only)
     uint4 rec[kMaxFitRows];           // the sampled records of the minibatch
@@ -402,8 +397,7 @@ __device__ __forceinline__ void warp_sum9(float (&v)[9]) {
     }
 }
 // the row-parallel kernel's work on net `net` of run P
-template <class Run>
-__device__ __forceinline__ void fit_rows_net(const FitArgs &F, const Run &P, int net) {
+__device__ __forceinline__ void fit_rows_net(const FitSchedule &F, const FitRun &P, int net) {
     extern __shared__ __align__(16) unsigned char fit_smem_raw[];
     RowFitSmem &S = *reinterpret_cast<RowFitSmem *>(fit_smem_raw);
     __shared__ int s_peer_lost;  // a peer did not answer within the time limit of the gradient exchange
@@ -605,17 +599,17 @@ __device__ __forceinline__ void fit_rows_net(const FitArgs &F, const Run &P, int
     for (int e = threadIdx.x; e < NFSP_NET_PARAMS; e += kRowThreads) P.w_out[net * NFSP_NET_PARAMS + e] = S.w[e];
 }
 __global__ void __launch_bounds__(kRowThreads, 1)
-learner_fit_rows_kernel(const FitArgs F) { fit_rows_net(F, F, blockIdx.x); }
+learner_fit_rows_kernel(const FitSchedule S, const FitRun P) { fit_rows_net(S, P, blockIdx.x); }
 
 // ---- the fits of independent runs in one launch (nfsp_learner_fit_runs): CTA 4 r + k = net k of run r ------------------
 struct FitRuns {
-    FitArgs F;  // the shared step schedule (world = 1); its A, w_out and lr are not read
-    FitRun run[NFSP_MAX_RUNS];
+    FitRun run[NFSP_MAX_RUNS];  // first: the row-parallel kernel then schedules as it did before the split (sass_check r05)
+    FitSchedule S;              // world = 1
 };
 __global__ void __launch_bounds__(kLearnThreads)
-learner_fit_runs_kernel(const __grid_constant__ FitRuns R) { fit_regs_net(R.F, R.run[blockIdx.x >> 2], blockIdx.x & 3); }
+learner_fit_runs_kernel(const __grid_constant__ FitRuns R) { fit_regs_net(R.S, R.run[blockIdx.x >> 2], blockIdx.x & 3); }
 __global__ void __launch_bounds__(kRowThreads, 1)
-learner_fit_rows_runs_kernel(const __grid_constant__ FitRuns R) { fit_rows_net(R.F, R.run[blockIdx.x >> 2], blockIdx.x & 3); }
+learner_fit_rows_runs_kernel(const __grid_constant__ FitRuns R) { fit_rows_net(R.S, R.run[blockIdx.x >> 2], blockIdx.x & 3); }
 
 // w[k] -= lr[k] * scale * grad[k]   (keras.optimizers.SGD without momentum, agent.py:45-46)
 __global__ void sgd_apply_kernel(float *__restrict__ w, const float *__restrict__ grad, float lr0, float lr1, float lr2,
@@ -657,12 +651,9 @@ extern "C" int nfsp_learner_grads(const nfsp_learner_io *io, void *stream) {
     return NFSP_OK;
 }
 
-static int learner_fit_impl(const nfsp_learner_io *io, int minibatch, int fit_batch, int epochs, const float lr[4],
-                            float *d_weights_out, const nfsp_peers *peers, void *stream);
-
 // the SGD steps of Keras' fit(batch_size = fit_batch, epochs): slices [0, fit_batch), [fit_batch, 2 fit_batch), ... of the
-// minibatch, `epochs` times; one GPU, no peers
-static int fit_schedule(int minibatch, int fit_batch, int epochs, FitArgs &F) {
+// minibatch, `epochs` times; one GPU unless `peers` is given
+static int fit_schedule(int minibatch, int fit_batch, int epochs, const nfsp_peers *peers, FitSchedule &F) {
     NFSP_CHECK_ARG(minibatch >= 1 && fit_batch >= 1 && epochs >= 1, "bad fit geometry");
     F.minibatch = minibatch;
     F.n_steps = 0;
@@ -675,12 +666,46 @@ static int fit_schedule(int minibatch, int fit_batch, int epochs, FitArgs &F) {
         }
     F.world = 1; F.rank = 0; F.epoch0 = 0u; F.err = nullptr; F.mc = nullptr;
     for (int r = 0; r < NFSP_MAX_PEERS; ++r) F.peer[r] = nullptr;
+    if (peers) {
+        F.world = peers->world; F.rank = peers->rank; F.epoch0 = peers->epoch0; F.err = peers->d_err;
+        F.mc = (float *)peers->d_mc;
+        for (int r = 0; r < peers->world; ++r) F.peer[r] = (float *)peers->d_buf[r];
+    }
+    return NFSP_OK;
+}
+
+// The fits of n_runs runs on one schedule, CTA 4 r + k = net k of run r: the row-parallel kernel (one warp per row,
+// weights in shared memory) when the minibatch and a step fit its shared memory, the register kernel otherwise; one run
+// launches the single-run kernels, which read their arguments from the constant bank.
+static int learner_fit(const nfsp_learner_io *io, int n_runs, int minibatch, int fit_batch, int epochs, const float *lr,
+                       float *const *d_weights_out, const nfsp_peers *peers, cudaStream_t st) {
+    NFSP_CHECK_ARG(io && lr && d_weights_out, "null argument");
+    FitRuns R;
+    int rc = fit_schedule(minibatch, fit_batch, epochs, peers, R.S);
+    if (rc != NFSP_OK) return rc;
+    for (int r = 0; r < n_runs; ++r) {
+        NFSP_CHECK_ARG(d_weights_out[r], "null output weights of run %d", r);
+        rc = make_learner_args(io + r, R.run[r].A);
+        if (rc != NFSP_OK) return rc;
+        R.run[r].w_out = d_weights_out[r];
+        for (int k = 0; k < 4; ++k) R.run[r].lr[k] = lr[4 * r + k];
+    }
+    const bool rows = minibatch <= kMaxFitRows && fit_batch <= kMaxStepRows;
+    void (*single)(FitSchedule, FitRun) = rows ? learner_fit_rows_kernel : learner_fit_kernel;
+    void (*batch)(FitRuns) = rows ? learner_fit_rows_runs_kernel : learner_fit_runs_kernel;
+    const int threads = rows ? kRowThreads : kLearnThreads, smem = rows ? (int)sizeof(RowFitSmem) : 0;
+    if (rows)  // per call: the attribute belongs to the current device's context
+        NFSP_CUDA(cudaFuncSetAttribute(n_runs == 1 ? (const void *)single : (const void *)batch,
+                                       cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    if (n_runs == 1) single<<<4, threads, smem, st>>>(R.S, R.run[0]);
+    else batch<<<4 * n_runs, threads, smem, st>>>(R);
+    NFSP_LAUNCH_CHECK();
     return NFSP_OK;
 }
 
 extern "C" int nfsp_learner_fit(const nfsp_learner_io *io, int minibatch, int fit_batch, int epochs, const float lr[4],
                                 float *d_weights_out, void *stream) {
-    return learner_fit_impl(io, minibatch, fit_batch, epochs, lr, d_weights_out, nullptr, stream);
+    return learner_fit(io, 1, minibatch, fit_batch, epochs, lr, &d_weights_out, nullptr, (cudaStream_t)stream);
 }
 
 extern "C" int nfsp_learner_fit_peers(const nfsp_learner_io *io, int minibatch, int fit_batch, int epochs, const float lr[4],
@@ -689,63 +714,16 @@ extern "C" int nfsp_learner_fit_peers(const nfsp_learner_io *io, int minibatch, 
                    "2..%d peers", NFSP_MAX_PEERS);
     NFSP_CHECK_ARG(peers->d_err, "null error word");
     for (int r = 0; r < peers->world; ++r) NFSP_CHECK_ARG(peers->d_buf[r], "null exchange buffer of rank %d", r);
-    NFSP_CHECK_ARG(minibatch <= nfsp::kMaxFitRows && fit_batch <= nfsp::kMaxStepRows,
-                   "the peer exchange lives in the row-parallel kernel: minibatch <= %d, fit_batch <= %d", nfsp::kMaxFitRows,
-                   nfsp::kMaxStepRows);
-    return learner_fit_impl(io, minibatch, fit_batch, epochs, lr, d_weights_out, peers, stream);
-}
-
-static int learner_fit_impl(const nfsp_learner_io *io, int minibatch, int fit_batch, int epochs, const float lr[4],
-                            float *d_weights_out, const nfsp_peers *peers, void *stream) {
-    NFSP_CHECK_ARG(lr && d_weights_out, "null argument");
-    FitArgs F;
-    int rc = fit_schedule(minibatch, fit_batch, epochs, F);
-    if (rc != NFSP_OK) return rc;
-    rc = make_learner_args(io, F.A);
-    if (rc != NFSP_OK) return rc;
-    F.w_out = d_weights_out;
-    for (int k = 0; k < 4; ++k) F.lr[k] = lr[k];
-    if (peers) {
-        F.world = peers->world; F.rank = peers->rank; F.epoch0 = peers->epoch0; F.err = peers->d_err;
-        F.mc = (float *)peers->d_mc;
-        for (int r = 0; r < peers->world; ++r) F.peer[r] = (float *)peers->d_buf[r];
-    }
-    if (minibatch <= kMaxFitRows && fit_batch <= kMaxStepRows) {  // one warp per row, weights in shared memory
-        // per call: the attribute belongs to the current device's context
-        NFSP_CUDA(cudaFuncSetAttribute(learner_fit_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RowFitSmem)));
-        learner_fit_rows_kernel<<<4, kRowThreads, sizeof(RowFitSmem), (cudaStream_t)stream>>>(F);
-    } else {  // large batches: the register kernel
-        learner_fit_kernel<<<4, kLearnThreads, 0, (cudaStream_t)stream>>>(F);
-    }
-    NFSP_LAUNCH_CHECK();
-    return NFSP_OK;
+    NFSP_CHECK_ARG(minibatch <= NFSP_FIT_ROWS_MAX_MINIBATCH && fit_batch <= NFSP_FIT_ROWS_MAX_STEP,
+                   "the peer exchange lives in the row-parallel kernel: minibatch <= %d, fit_batch <= %d",
+                   NFSP_FIT_ROWS_MAX_MINIBATCH, NFSP_FIT_ROWS_MAX_STEP);
+    return learner_fit(io, 1, minibatch, fit_batch, epochs, lr, &d_weights_out, peers, (cudaStream_t)stream);
 }
 
 extern "C" int nfsp_learner_fit_runs(const nfsp_learner_io *io, int n_runs, int minibatch, int fit_batch, int epochs, const float *lr,
                                      float *const *d_weights_out, void *stream) {
-    NFSP_CHECK_ARG(io && lr && d_weights_out, "null argument");
     NFSP_CHECK_ARG(n_runs >= 1 && n_runs <= NFSP_MAX_RUNS, "n_runs must be in [1, %d]", NFSP_MAX_RUNS);
-    FitRuns R;
-    int rc = fit_schedule(minibatch, fit_batch, epochs, R.F);
-    if (rc != NFSP_OK) return rc;
-    R.F.A = LearnerArgs{};
-    R.F.w_out = nullptr;
-    for (int k = 0; k < 4; ++k) R.F.lr[k] = 0.f;
-    for (int r = 0; r < n_runs; ++r) {
-        NFSP_CHECK_ARG(d_weights_out[r], "null output weights of run %d", r);
-        rc = make_learner_args(io + r, R.run[r].A);
-        if (rc != NFSP_OK) return rc;
-        R.run[r].w_out = d_weights_out[r];
-        for (int k = 0; k < 4; ++k) R.run[r].lr[k] = lr[4 * r + k];
-    }
-    if (minibatch <= kMaxFitRows && fit_batch <= kMaxStepRows) {  // the same choice of kernel as nfsp_learner_fit
-        NFSP_CUDA(cudaFuncSetAttribute(learner_fit_rows_runs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RowFitSmem)));
-        learner_fit_rows_runs_kernel<<<4 * n_runs, kRowThreads, sizeof(RowFitSmem), (cudaStream_t)stream>>>(R);
-    } else {
-        learner_fit_runs_kernel<<<4 * n_runs, kLearnThreads, 0, (cudaStream_t)stream>>>(R);
-    }
-    NFSP_LAUNCH_CHECK();
-    return NFSP_OK;
+    return learner_fit(io, n_runs, minibatch, fit_batch, epochs, lr, d_weights_out, nullptr, (cudaStream_t)stream);
 }
 
 extern "C" int nfsp_sgd_apply(float *d_weights, const float *d_grad, const float lr[4], float scale, void *stream) {

@@ -24,14 +24,14 @@ int nfsp_rollout_pairs_configure();
 
 // the rollout over a table of the nets' outputs per decision state (rollout_states.cu)
 int nfsp_rollout_states_launch(nfsp_env_t h, const nfsp::RolloutArgs &A, const nfsp_rollout_io *io, bool debug, cudaStream_t st);
-int nfsp_states_ensure(nfsp_env_t h, const float *d_tab, float *d_states, cudaStream_t st);
+// rebuilds the state tables of n handles (1 <= n <= NFSP_MAX_RUNS) from their table images tab[r] in one launch and clears
+// their st_dirty
+int nfsp_states_pack(const nfsp_env_t *h, const float *const *tab, int n, cudaStream_t st);
 int nfsp_states_floats();
 int nfsp_states_upload_image(float *d_states);
 int nfsp_rollout_states_configure();
 // independent runs of one shape in one launch of the same rollout (nfsp_rollout_runs); A[r].pack = handle r's state table
 int nfsp_rollout_states_runs_launch(nfsp_env_t h, const nfsp::RolloutArgs *A, int n_runs, int sms, cudaStream_t st);
-// rebuilds the state tables of n handles from their table images in one launch and clears their st_dirty
-int nfsp_states_pack_runs(const nfsp_env_t *h, const float *const *tab, int n, cudaStream_t st);
 
 namespace nfsp {
 

@@ -78,14 +78,12 @@ __device__ __forceinline__ void states_pack(const float *__restrict__ tab, float
         states[e] = make_float4(o0, o1, o2, __uint_as_float(score_word(o0, o1, o2)));
     }
 }
-__global__ void states_pack_kernel(const float *__restrict__ tab, float4 *__restrict__ states) { states_pack(tab, states); }
-
-// the tables of several handles in one launch: blockIdx.y = run
+// the tables of 1..NFSP_MAX_RUNS handles in one launch: blockIdx.y = handle
 struct StatesRuns {
     const float *tab[NFSP_MAX_RUNS];
     float4 *states[NFSP_MAX_RUNS];
 };
-__global__ void states_pack_runs_kernel(const __grid_constant__ StatesRuns P) { states_pack(P.tab[blockIdx.y], P.states[blockIdx.y]); }
+__global__ void states_pack_kernel(const __grid_constant__ StatesRuns P) { states_pack(P.tab[blockIdx.y], P.states[blockIdx.y]); }
 
 // 1 024 threads per CTA for launches that keep every warp busy with several blocks of games; 512 (16 warps, 90 registers)
 // when the launch has no more blocks than that gives warps -- a warp then plays one block, and what counts is the latency
@@ -441,15 +439,6 @@ int nfsp_rollout_states_configure() {
     return rc != NFSP_OK ? rc : configure_states<kStatesThreadsSmall>();
 }
 
-// rebuilds the state table from the table image (both live in d_wpack) when the weights have changed since
-int nfsp_states_ensure(nfsp_env_t h, const float *d_tab, float *d_states, cudaStream_t st) {
-    if (!h->st_dirty) return NFSP_OK;
-    states_pack_kernel<<<(4 * kStateQuads + 127) / 128, 128, 0, st>>>(d_tab, reinterpret_cast<float4 *>(d_states));
-    NFSP_LAUNCH_CHECK();
-    h->st_dirty = false;
-    return NFSP_OK;
-}
-
 template <int kThreads>
 static int launch_states(const RolloutArgs &A, int grid, bool debug, bool direct, cudaStream_t st) {
     constexpr int kBytes = states_smem_bytes(kThreads);
@@ -461,14 +450,13 @@ static int launch_states(const RolloutArgs &A, int grid, bool debug, bool direct
     return NFSP_OK;
 }
 
-// the state tables of n handles from their table images (tab[r] = handle r's, in its d_wpack), one launch
-int nfsp_states_pack_runs(const nfsp_env_t *h, const float *const *tab, int n, cudaStream_t st) {
+int nfsp_states_pack(const nfsp_env_t *h, const float *const *tab, int n, cudaStream_t st) {
     StatesRuns P;
     for (int r = 0; r < n; ++r) {
         P.tab[r] = tab[r];
         P.states[r] = reinterpret_cast<float4 *>(h[r]->d_states);
     }
-    states_pack_runs_kernel<<<dim3((4 * kStateQuads + 127) / 128, (unsigned)n), 128, 0, st>>>(P);
+    states_pack_kernel<<<dim3((4 * kStateQuads + 127) / 128, (unsigned)n), 128, 0, st>>>(P);
     NFSP_LAUNCH_CHECK();
     for (int r = 0; r < n; ++r) h[r]->st_dirty = false;
     return NFSP_OK;

@@ -67,7 +67,7 @@ class Learner:
         if peer_transport not in ("auto", "symm", "ipc"):
             raise ValueError("peer_transport must be 'auto', 'symm' or 'ipc'")
         self.peer_transport = peer_transport
-        if self.fused and _world() > 1 and self.minibatch <= 256 and self.fit_batch <= 64:
+        if self.fused and _world() > 1 and self.minibatch <= _lib.FIT_ROWS_MAX_MINIBATCH and self.fit_batch <= _lib.FIT_ROWS_MAX_STEP:
             # every rank must take the same path (a rank in the peer exchange and one in an NCCL all-reduce would wait
             # for each other forever): _setup_peers agrees on every phase collectively
             self._setup_peers()
@@ -108,6 +108,11 @@ class Learner:
         io.d_grad, io.d_stats = self.flat.data_ptr(), self.flat[GRAD:].data_ptr()
         return io
 
+    def _fit_args(self, idx_rl, idx_sl, mask, w_in=None, row0=0, rows=None):
+        """The nfsp_learner_io of sampled rows [row0, row0 + rows) (default: all) and the lrs in net order avg0, br0, avg1, br1."""
+        io = self._io(idx_rl, idx_sl, row0, self.minibatch if rows is None else rows, mask, w_in)
+        return io, (self.lr_ar, self.lr_br[0], self.lr_ar, self.lr_br[1])
+
     def _sample_positions(self, snapshot=False, which="both"):
         """sample_batch positions of the four memories (agent.py:217,260) in one launch; the same draws as four
         sample_slots() calls.  Returns ([rl0, rl1], [sl0, sl1]) index tensors of `minibatch` storage slots.
@@ -131,22 +136,16 @@ class Learner:
         """The sampling requests of _sample_positions (self._pos_reqs, rows rl0, rl1, sl0, sl1), their memories' draw
         counters advanced; nothing is launched.  Returns the range [lo, hi) of the requests `which` names."""
         sp, b = self.sp, self.minibatch
+        mems = (sp.rl[0], sp.rl[1], sp.sl[0], sp.sl[1])
         if not hasattr(self, "_pos"):
             self._pos = torch.empty((4, b), dtype=torch.int64, device=self.device)   # rows: rl0, rl1, sl0, sl1
-            reqs = (_lib.SampleReq * 4)()
-            for k, mem in enumerate((sp.rl[0], sp.rl[1], sp.sl[0], sp.sl[1])):
-                r = reqs[k]
-                r.d_mem, r.d_total, r.cap = mem.store.data_ptr(), mem.total.data_ptr(), mem.capacity
-                r.seed, r.is_ring, r.d_out = mem.seed, int(mem.is_ring), None
-            self._pos_reqs = reqs
+            self._pos_reqs = (_lib.SampleReq * 4)(*(mem.sample_req(_lib.SampleReq()) for mem in mems))
         g_rl, g_sl, rows = self._snapshot_buffers() if snapshot else (None, None, None)
         lo, hi = {"both": (0, 4), "rl": (0, 2), "sl": (2, 4)}[which]
-        for k, mem in enumerate((sp.rl[0], sp.rl[1], sp.sl[0], sp.sl[1])):
-            if lo <= k < hi:
-                r = self._pos_reqs[k]
-                r.call_idx = mem.sample_calls
-                r.d_rec_out = None if not snapshot else (g_rl[k] if k < 2 else g_sl[k - 2]).data_ptr()
-                mem.sample_calls += 1
+        for k in range(lo, hi):
+            r = self._pos_reqs[k]
+            r.call_idx = mems[k].next_call()
+            r.d_rec_out = None if not snapshot else (g_rl[k] if k < 2 else g_sl[k - 2]).data_ptr()
         return lo, hi
 
     def presample_rings(self):
@@ -290,31 +289,26 @@ class Learner:
             raise RuntimeError("a peer GPU did not answer during the gradient exchange: the weights of this update are "
                                "invalid (NaN) and the replicas have diverged")
 
-    def _fit_peers(self, idx_rl, idx_sl, mask, w_in=None, w_out=None):
-        io = self._io(idx_rl, idx_sl, 0, self.minibatch, mask, w_in)
-        lr = (C.c_float * 4)(self.lr_ar, self.lr_br[0], self.lr_ar, self.lr_br[1])
+    # ---- the whole fit() in one launch: one GPU, or several with the all-reduce of every SGD step inside it ----
+    def _fit_one_launch(self, idx_rl, idx_sl, mask, w_in=None, w_out=None):
+        io, lr = self._fit_args(idx_rl, idx_sl, mask, w_in)
+        args = (C.byref(io), self.minibatch, self.fit_batch, self.epochs, (C.c_float * 4)(*lr),
+                _ptr(self.sp.weights if w_out is None else w_out))
+        if self._peers is None:
+            return check(lib().nfsp_learner_fit(*args, _stream(self.device)))
         self._peers.epoch0 = self._epoch & 0xFFFFFFFF
-        check(lib().nfsp_learner_fit_peers(C.byref(io), self.minibatch, self.fit_batch, self.epochs, lr,
-                                           _ptr(self.sp.weights if w_out is None else w_out), C.byref(self._peers),
-                                           _stream(self.device)))
+        check(lib().nfsp_learner_fit_peers(*args, C.byref(self._peers), _stream(self.device)))
         self._epoch += self.epochs * ((self.minibatch + self.fit_batch - 1) // self.fit_batch)
-
-    # ---- the whole fit() in one launch: one GPU, no collective between the SGD steps ---------------
-    def _fit_fused(self, idx_rl, idx_sl, mask, w_in=None, w_out=None):
-        io = self._io(idx_rl, idx_sl, 0, self.minibatch, mask, w_in)
-        lr = (C.c_float * 4)(self.lr_ar, self.lr_br[0], self.lr_ar, self.lr_br[1])
-        check(lib().nfsp_learner_fit(C.byref(io), self.minibatch, self.fit_batch, self.epochs, lr,
-                                     _ptr(self.sp.weights if w_out is None else w_out), _stream(self.device)))
 
     # ---- one SGD step for all four nets -------------------------------------------------------------
     def _step(self, idx_rl, idx_sl, row0, rows, mask):
         sp = self.sp
-        io = self._io(idx_rl, idx_sl, row0, rows, mask)
+        io, lr = self._fit_args(idx_rl, idx_sl, mask, row0=row0, rows=rows)
         check(lib().nfsp_learner_grads(C.byref(io), _stream(self.device)))
         world = _world()
         if world > 1:  # C1 (gradients) + C2 (exploitability stats) in one collective
             dist.all_reduce(self.flat, op=dist.ReduceOp.SUM)
-        lr = (C.c_float * 4)(self.lr_ar, self.lr_br[0], self.lr_ar, self.lr_br[1])
+        lr = (C.c_float * 4)(*lr)
         check(lib().nfsp_sgd_apply(_ptr(sp.weights), _ptr(self.flat), C.byref(lr), 1.0 / world, _stream(self.device)))
 
     def _ready_mask(self):
@@ -361,12 +355,9 @@ class Learner:
         if on_gathered is not None:
             on_gathered()
         stats = None
-        if self.fused and (_world() == 1 or self._peers is not None):
+        if self.one_launch:
             # one launch for the 8 SGD steps; with peers the per-step all-reduce happens inside it over NVLink
-            if _world() == 1:
-                self._fit_fused(idx_rl, idx_sl, mask, weights_in, weights_out)
-            else:
-                self._fit_peers(idx_rl, idx_sl, mask, weights_in, weights_out)
+            self._fit_one_launch(idx_rl, idx_sl, mask, weights_in, weights_out)
             stats = self.flat[GRAD:].clone()     # statistics of the first step, as below
         else:
             for _ in range(self.epochs):         # Keras fit(epochs=2), batch_size 32 (agent.py:243,261)
@@ -431,8 +422,9 @@ class PipelinedTrainer:
 
     def __init__(self, selfplay, learner, reserve_sms=4):
         if not learner.one_launch:
-            raise RuntimeError("PipelinedTrainer needs the one-launch fit: fused=True, minibatch <= 256, fit batch <= 64 and, "
-                               "with several GPUs, peer memory (%s)" % getattr(learner, "_peer_note", "see Learner._setup_peers"))
+            raise RuntimeError("PipelinedTrainer needs the one-launch fit: fused=True and, with several GPUs, minibatch <= %d, fit batch "
+                               "<= %d and peer memory (%s)" % (_lib.FIT_ROWS_MAX_MINIBATCH, _lib.FIT_ROWS_MAX_STEP,
+                                                               getattr(learner, "_peer_note", "see Learner._setup_peers")))
         self.sp, self.learner, self.reserve_sms = selfplay, learner, int(reserve_sms)
         self.w = [selfplay.weights.clone(), selfplay.weights.clone()]  # W_j lives in w[j % 2]
         self.stream = torch.cuda.Stream(selfplay.device)

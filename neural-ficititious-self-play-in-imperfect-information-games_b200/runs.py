@@ -141,8 +141,7 @@ class RunBatch:
         check(lib().nfsp_sample_minibatches(self._sample_reqs, 4 * len(active), b, _ptr(self._pos), None, st))
         for k, r in enumerate(active):
             ln, pos = lns[r], self._pos[k]
-            self._learner_io[k] = ln._io([pos[0], pos[1]], [pos[2], pos[3]], 0, b, masks[r])
-            self._lr[4 * k:4 * k + 4] = [ln.lr_ar, ln.lr_br[0], ln.lr_ar, ln.lr_br[1]]
+            self._learner_io[k], self._lr[4 * k:4 * k + 4] = ln._fit_args([pos[0], pos[1]], [pos[2], pos[3]], masks[r])
             self._w_out[k] = sps[r].weights.data_ptr()
         check(lib().nfsp_learner_fit_runs(self._learner_io, len(active), b, lns[0].fit_batch, lns[0].epochs, self._lr,
                                           self._w_out, st))

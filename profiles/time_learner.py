@@ -27,7 +27,7 @@ for it in range(10):
     marks[0].record()
     idx_rl, idx_sl = L._sample_positions()
     marks.append(ev()); marks[-1].record(); names.append("positions of the 4 minibatches")
-    L._fit_fused(idx_rl, idx_sl, 15)
+    L._fit_one_launch(idx_rl, idx_sl, 15)
     marks.append(ev()); marks[-1].record(); names.append("fit kernel (8 SGD steps)")
     for row0 in range(0, 32, 32):
         L._step(idx_rl, idx_sl, row0, 32, 15)

@@ -77,8 +77,7 @@ def kernel_table(fn, iters):
 
 def short(name):
     for k in ("rollout_states_kernel", "learner_fit_rows_runs_kernel", "learner_fit_rows_kernel", "insert_kernel",
-              "sample_gather_wide_kernel", "sample_gather_kernel", "pack_images_runs_kernel", "pack_images_kernel",
-              "states_pack_runs_kernel", "states_pack_kernel"):
+              "sample_gather_wide_kernel", "sample_gather_kernel", "pack_images_kernel", "states_pack_kernel"):
         if k in name:
             return k + ("<runs>" if k == "rollout_states_kernel" and "RolloutRuns" in name else "")
     return name[:60]

@@ -21,6 +21,9 @@ def test_run_limits_match_the_header():
     assert _define("NFSP_MAX_SAMPLE_REQS") == _lib.MAX_SAMPLE_REQS == 4 * _lib.MAX_RUNS
     # the fit of every run in one wave of 4 CTAs per run on the 148 SMs of a B200
     assert 4 * _lib.MAX_RUNS <= 148
+    # the geometry of the row-parallel fit kernel, which the learner checks before it sets up the peer exchange
+    assert _define("NFSP_FIT_ROWS_MAX_MINIBATCH") == _lib.FIT_ROWS_MAX_MINIBATCH
+    assert _define("NFSP_FIT_ROWS_MAX_STEP") == _lib.FIT_ROWS_MAX_STEP
 
 
 @pytest.mark.parametrize("extra", [["--pipelined"], ["--runs", "0"]])
