@@ -54,6 +54,43 @@ def _as(t, dtype, dev, shape=None):
     return t
 
 
+def check_fields(d, where, **expected):
+    """State-dict validation: raises ValueError naming the first field whose saved value differs from `expected`."""
+    if not isinstance(d, dict):
+        raise ValueError("%s: the state is a %s, not a dict" % (where, type(d).__name__))
+    for k, v in expected.items():
+        if k not in d:
+            raise ValueError("%s: the state has no field %r" % (where, k))
+        if type(d[k]) is not type(v) or d[k] != v:
+            raise ValueError("%s: %s is %r in the state but %r here" % (where, k, d[k], v))
+
+
+def check_tensor(t, name, where, shape, dtype):
+    """State-dict validation: t (the field `name`) is a host tensor of `shape` and `dtype`."""
+    if not (isinstance(t, torch.Tensor) and t.device.type == "cpu" and t.dtype == dtype and tuple(t.shape) == tuple(shape)):
+        got = "%s %s" % (t.dtype, tuple(t.shape)) if isinstance(t, torch.Tensor) else type(t).__name__
+        raise ValueError("%s: %s must be a host %s tensor of shape %s, got %s" % (where, name, dtype, tuple(shape), got))
+
+
+def check_numbers(d, where, **kinds):
+    """State-dict validation of a dict: each named field holds a non-negative int (kind int), a number (kind float) or a
+    list of n of them (kind (int, n) / (float, n))."""
+    for k, kind in kinds.items():
+        kind, n = kind if isinstance(kind, tuple) else (kind, None)
+        v = d.get(k)
+        if n is None:
+            vals = [v]
+        else:
+            vals = v if isinstance(v, list) and len(v) == n else None
+        if kind is int:
+            ok = vals is not None and all(type(x) is int and x >= 0 for x in vals)
+        else:
+            ok = vals is not None and all(type(x) in (int, float) for x in vals)
+        if not ok:
+            raise ValueError("%s: %s must be %s%s, got %r" % (where, k, "a list of %d " % n if n else "a ",
+                                                             "non-negative int" if kind is int else "number", v))
+
+
 def expand_obs(masks: torch.Tensor) -> torch.Tensor:
     """30-bit observation masks -> float32 [n, 30] (the reference's state vector, newenv.py:118-122)."""
     m = masks.contiguous().view(torch.int32).reshape(-1)
@@ -307,6 +344,33 @@ class _Memory:
 
     def clear(self):
         self.total.zero_()
+
+    def _shape(self):
+        return dict(kind="ring" if self.is_ring else "reservoir", capacity=self.capacity, seed=self.seed,
+                    mode=getattr(self, "mode", 0))
+
+    def state_dict(self) -> dict:
+        """Host copy of everything later inserts and draws depend on: the held slots store[:min(total, capacity)]
+        (whole storage slots, a reservoir's stamps included), `total` and the draw counter.  Synchronises the device."""
+        torch.cuda.synchronize(self.device)
+        total = int(self.total.item())
+        return dict(self._shape(), total=total, sample_calls=self.sample_calls,
+                    slots=self.store[:min(total, self.capacity)].cpu())
+
+    def check_state_dict(self, d, where="memory"):
+        """Raises ValueError, naming the field, if load_state_dict(d) would refuse d."""
+        check_fields(d, where, **self._shape())
+        check_numbers(d, where, total=int, sample_calls=int)
+        check_tensor(d.get("slots"), "slots", where, (min(d["total"], self.capacity), self.slot_words), torch.int32)
+
+    def load_state_dict(self, d, where="memory"):
+        """Validates d, then restores it; slots past the held ones are zeroed, as in a memory that never reached them."""
+        self.check_state_dict(d, where)
+        held = d["slots"].shape[0]
+        self.store[:held].copy_(d["slots"])
+        self.store[held:].zero_()
+        self.total.fill_(d["total"])
+        self.sample_calls = d["sample_calls"]
 
 
 class DeviceRing(_Memory):
@@ -672,3 +736,50 @@ class SelfPlay:
     def read_stats(self):
         v = self.stats.cpu().numpy()
         return {k: int(v[i]) for i, k in enumerate(self.STAT_NAMES)}
+
+    def _shape(self):
+        return dict(n_games=self.n, game0=self.env.game0, seed=self.env.seed, variant=self.variant,
+                    direct_rings=self.direct_rings, deterministic=self.deterministic, max_steps=self.max_steps,
+                    n_seg=self.n_seg, rl_capacity=self.rl[0].capacity, sl_capacity=self.sl[0].capacity)
+
+    def state_dict(self) -> dict:
+        """Host copy of what the run's later rollouts, inserts and draws depend on: the four memories, game words, step
+        counter, acting nets, epsilons, eta and rollout counters, with the shape they need.  Synchronises the device;
+        refuses (ValueError) while records are staged but not flushed (rollout(insert=False) without flush())."""
+        if int(self.counts.sum().item()):
+            raise ValueError("SelfPlay: records are staged but not flushed; flush() before state_dict()")
+        torch.cuda.synchronize(self.device)
+        return dict(shape=self._shape(), rl=[m.state_dict() for m in self.rl], sl=[m.state_dict() for m in self.sl],
+                    words=self.env.state_words().cpu(), step=self.env.step_counter, weights=self.weights.cpu(),
+                    epsilons=list(self.epsilons), eta=self.eta, stats=self.stats.cpu())
+
+    def check_state_dict(self, d):
+        """Raises ValueError, naming the field, if load_state_dict(d) would refuse d."""
+        check_fields(d, "SelfPlay")
+        check_fields(d.get("shape"), "SelfPlay", **self._shape())
+        for key, mems in (("rl", self.rl), ("sl", self.sl)):
+            if not (isinstance(d.get(key), list) and len(d[key]) == 2):
+                raise ValueError("SelfPlay: %s must be a list of the two players' memories" % key)
+            for p in range(2):
+                mems[p].check_state_dict(d[key][p], "SelfPlay %s[%d]" % (key, p))
+        check_tensor(d.get("words"), "words", "SelfPlay", (self.n,), torch.int64)
+        check_tensor(d.get("weights"), "weights", "SelfPlay", tuple(self.weights.shape), torch.float32)
+        check_tensor(d.get("stats"), "stats", "SelfPlay", (_lib.STATS_FIELDS,), torch.int64)
+        check_numbers(d, "SelfPlay", step=int, epsilons=(float, 2), eta=float)
+
+    def load_state_dict(self, d):
+        """Validates d, then restores it into this object's own tensors (stats too, which may be a view into the
+        sampling slab); the weight images are rebuilt from the restored nets and nothing stays staged."""
+        self.check_state_dict(d)
+        for key, mems in (("rl", self.rl), ("sl", self.sl)):
+            for p in range(2):
+                mems[p].load_state_dict(d[key][p])
+        self.env.load_state_words(d["words"])
+        self.env.step_counter = d["step"]
+        self.weights.copy_(d["weights"])
+        check(lib().nfsp_act_set_weights(self.env._h, _ptr(self.weights), _stream(self.device)))
+        self.epsilons = [float(e) for e in d["epsilons"]]
+        self.eta = self.env.eta = float(d["eta"])
+        self.stats.copy_(d["stats"])
+        self.counts.zero_()
+        torch.cuda.synchronize(self.device)

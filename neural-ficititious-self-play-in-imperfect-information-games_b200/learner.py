@@ -29,7 +29,7 @@ import torch.distributed as dist
 
 from . import _lib
 from ._lib import check, lib
-from .batched import _ptr, _stream
+from .batched import _ptr, _stream, check_fields, check_numbers, check_tensor
 
 GRAD = 4 * _lib.NET_PARAMS
 N_STATS = 8
@@ -283,11 +283,13 @@ class Learner:
     def check_peers(self):
         """Raises if a peer GPU failed to answer during any gradient exchange so far (the kernel then gave up after ~2 s,
         skipped that net's remaining SGD steps and wrote NaN weights for it, so the failure cannot go unnoticed; the
-        replicas are no longer identical and the run must be restarted from a checkpoint).  Reads one device word (syncs):
+        replicas are no longer identical and the run must be resumed from its last checkpoint, `checkpoint.load` /
+        `main.py --resume DIR`).  Reads one device word (syncs):
         called by update(sync=True), by PipelinedTrainer.finish() and every `peer_check_every` updates."""
         if self._peers is not None and int(self._peer_err.item()):
             raise RuntimeError("a peer GPU did not answer during the gradient exchange: the weights of this update are "
-                               "invalid (NaN) and the replicas have diverged")
+                               "invalid (NaN) and the replicas have diverged; resume the run from its last checkpoint "
+                               "(main.py --resume DIR, with the --checkpoint DIR it was trained with)")
 
     # ---- the whole fit() in one launch: one GPU, or several with the all-reduce of every SGD step inside it ----
     def _fit_one_launch(self, idx_rl, idx_sl, mask, w_in=None, w_out=None):
@@ -404,6 +406,50 @@ class Learner:
         return {"trained": mask, "exploitability": sum(self.exploitability), "loss": s[4:8], "epsilon": sp.epsilon,
                 "lr_br": list(self.lr_br)}
 
+    # ---- checkpoint / resume (the SelfPlay it trains has its own state dict) ----
+    def _shape(self):
+        return dict(minibatch=self.minibatch, fit_batch=self.fit_batch, epochs=self.epochs,
+                    terminal_bootstraps=self.terminal_bootstraps, others_to_target=self.others_to_target, fused=self.fused)
+
+    _SCALARS = dict(gamma=float, lr_br0=float, lr_ar=float, target_update_rate=int, iteration=(int, 2),
+                    target_update_count=(int, 2), temp=(float, 2), lr_br=(float, 2), exploitability=(float, 2), updates=int)
+
+    def state_dict(self) -> dict:
+        """Host copy of the target nets, the schedules and the last read-back statistics, with the learner's shape.
+        Synchronises the device.  The peer exchange's epoch is not part of it: a learner maps fresh, zeroed exchange
+        buffers and starts at epoch 0."""
+        torch.cuda.synchronize(self.device)
+        d = dict(shape=self._shape(), target=self.target.cpu(), loss=list(getattr(self, "_loss", [])) or None)
+        for k in self._SCALARS:
+            v = getattr(self, k)
+            d[k] = list(v) if isinstance(v, list) else v
+        return d
+
+    def check_state_dict(self, d):
+        """Raises ValueError, naming the field, if load_state_dict(d) would refuse d."""
+        check_fields(d, "Learner")
+        check_fields(d.get("shape"), "Learner", **self._shape())
+        check_tensor(d.get("target"), "target", "Learner", tuple(self.target.shape), torch.float32)
+        check_numbers(d, "Learner", **self._SCALARS)
+        if d.get("loss") is not None:
+            check_numbers(d, "Learner", loss=(float, N_STATS))
+        if d["target_update_rate"] < 1:
+            raise ValueError("Learner: target_update_rate must be at least 1")
+
+    def load_state_dict(self, d):
+        """Validates d, then restores it.  Learning rates, gamma and the target update rate come from d."""
+        self.check_state_dict(d)
+        torch.cuda.synchronize(self.device)
+        self.target.copy_(d["target"])
+        for k, kind in self._SCALARS.items():
+            setattr(self, k, list(d[k]) if isinstance(kind, tuple) else d[k])
+        self.gamma, self.lr_br0, self.lr_ar = float(self.gamma), float(self.lr_br0), float(self.lr_ar)
+        self.__dict__.pop("_loss", None)
+        if d["loss"] is not None:
+            self._loss = list(d["loss"])
+        self._all_ready = False  # the memories may hold fewer records now: read their sizes again
+        torch.cuda.synchronize(self.device)
+
 
 class PipelinedTrainer:
     """Self-play with the learner BESIDE the actor: update j runs on its own stream while rollout j+1 plays.
@@ -474,6 +520,32 @@ class PipelinedTrainer:
         self.learner.check_peers()
         self.sp.set_weights(self.w[self.j % 2])
         return self.w[self.j % 2]
+
+    def state_dict(self) -> dict:
+        """Host copies of the two weight tensors (W_j and W_{j-1}: the next step acts with one and trains from the
+        other) and j, once the update in flight has written its result.  The SelfPlay and the Learner have their own
+        state dicts."""
+        torch.cuda.current_stream(self.sp.device).wait_stream(self.stream)
+        torch.cuda.synchronize(self.sp.device)
+        return dict(w=[w.cpu() for w in self.w], j=self.j)
+
+    def check_state_dict(self, d):
+        """Raises ValueError, naming the field, if load_state_dict(d) would refuse d."""
+        check_fields(d, "PipelinedTrainer")
+        check_numbers(d, "PipelinedTrainer", j=int)
+        if not (isinstance(d.get("w"), list) and len(d["w"]) == 2):
+            raise ValueError("PipelinedTrainer: w must be a list of two weight tensors")
+        for k in range(2):
+            check_tensor(d["w"][k], "w[%d]" % k, "PipelinedTrainer", tuple(self.w[k].shape), torch.float32)
+
+    def load_state_dict(self, d):
+        """Validates d, then restores it: the next step() acts with the nets the saved trainer's next step would."""
+        self.check_state_dict(d)
+        torch.cuda.current_stream(self.sp.device).wait_stream(self.stream)
+        for w, src in zip(self.w, d["w"]):
+            w.copy_(src)
+        self.j = d["j"]
+        torch.cuda.synchronize(self.sp.device)
 
 
 # ---- single-game drop-in: agent.Agent.update_*_network ----------------------------------------------------

@@ -157,6 +157,33 @@ class RunBatch:
         self.rollout(n_steps)
         return self.update(sync)
 
+    def state_dict(self) -> dict:
+        """The runs' states in order, each {"selfplay": SelfPlay.state_dict(), "learner": Learner.state_dict()}: the
+        format of a run trained alone, so a run can move between a batch and a standalone SelfPlay / Learner."""
+        return dict(runs=[dict(selfplay=sp.state_dict(), learner=ln.state_dict()) for sp, ln in zip(self.sps, self.learners)])
+
+    def check_state_dict(self, d):
+        """Raises ValueError, naming the run and field, if load_state_dict(d) would refuse d."""
+        runs = d.get("runs") if isinstance(d, dict) else None
+        if not isinstance(runs, list) or len(runs) != self.n_runs:
+            raise ValueError("RunBatch: the state holds %s runs but this batch %d" %
+                             (len(runs) if isinstance(runs, list) else "no", self.n_runs))
+        for r, (run, sp, ln) in enumerate(zip(runs, self.sps, self.learners)):
+            if not (isinstance(run, dict) and {"selfplay", "learner"} <= run.keys()):
+                raise ValueError("RunBatch: run %d must hold a selfplay and a learner state" % r)
+            try:
+                sp.check_state_dict(run["selfplay"])
+                ln.check_state_dict(run["learner"])
+            except ValueError as e:
+                raise ValueError("run %d: %s" % (r, e)) from None
+
+    def load_state_dict(self, d):
+        """Validates every run's state, then loads them all."""
+        self.check_state_dict(d)
+        for run, sp, ln in zip(d["runs"], self.sps, self.learners):
+            sp.load_state_dict(run["selfplay"])
+            ln.load_state_dict(run["learner"])
+
     def exploitability(self):
         """exploitability.exploitability(sp) of every run (exact, of the average policies)."""
         from .exploitability import exploitability
