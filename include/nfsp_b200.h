@@ -50,7 +50,8 @@ int nfsp_device_info(int device, int *sm_count, int *cc_major, int *cc_minor, ch
 /* ------------------------------------------------------------------ lifecycle ------------- */
 /* One packed 64-bit word per game in HBM.  Games are numbered game0 .. game0+n_games-1; all
  * randomness is Philox4x32-10 keyed by (seed; global game id, step counter, purpose), so a
- * game's trace does not depend on how games are sharded over GPUs.
+ * game's trace does not depend on how games are sharded over GPUs.  The Philox counter holds the
+ * low 32 bits of the game id, so game0 + n_games may not exceed 2^32 (NFSP_E_ARG).
  * Replaces Env.__init__ (env.py:13-32, newenv.py:14-55). */
 int nfsp_env_create(int rules, int64_t n_games, uint64_t seed, uint64_t game0, int device, nfsp_env_t *out);
 int nfsp_env_destroy(nfsp_env_t h);

@@ -72,9 +72,14 @@ def check_tensor(t, name, where, shape, dtype):
         raise ValueError("%s: %s must be a host %s tensor of shape %s, got %s" % (where, name, dtype, tuple(shape), got))
 
 
-def check_numbers(d, where, **kinds):
+def check_numbers(d, where, below=None, **kinds):
     """State-dict validation of a dict: each named field holds a non-negative int (kind int), a number (kind float) or a
-    list of n of them (kind (int, n) / (float, n))."""
+    list of n of them (kind (int, n) / (float, n)).  `below` maps an int field to the exclusive bound of what holds it
+    (2**64 for a uint64 counter, 2**63 for an int64 tensor), so a counter that cannot be stored is refused up front."""
+    for k, bound in (below or {}).items():
+        v = d.get(k)
+        if type(v) is int and v >= bound:
+            raise ValueError("%s: %s must be below 2**%d, got %r" % (where, k, bound.bit_length() - 1, v))
     for k, kind in kinds.items():
         kind, n = kind if isinstance(kind, tuple) else (kind, None)
         v = d.get(k)
@@ -360,7 +365,7 @@ class _Memory:
     def check_state_dict(self, d, where="memory"):
         """Raises ValueError, naming the field, if load_state_dict(d) would refuse d."""
         check_fields(d, where, **self._shape())
-        check_numbers(d, where, total=int, sample_calls=int)
+        check_numbers(d, where, below=dict(total=2 ** 63, sample_calls=2 ** 64), total=int, sample_calls=int)
         check_tensor(d.get("slots"), "slots", where, (min(d["total"], self.capacity), self.slot_words), torch.int32)
 
     def load_state_dict(self, d, where="memory"):
@@ -765,7 +770,7 @@ class SelfPlay:
         check_tensor(d.get("words"), "words", "SelfPlay", (self.n,), torch.int64)
         check_tensor(d.get("weights"), "weights", "SelfPlay", tuple(self.weights.shape), torch.float32)
         check_tensor(d.get("stats"), "stats", "SelfPlay", (_lib.STATS_FIELDS,), torch.int64)
-        check_numbers(d, "SelfPlay", step=int, epsilons=(float, 2), eta=float)
+        check_numbers(d, "SelfPlay", below=dict(step=2 ** 64), step=int, epsilons=(float, 2), eta=float)
 
     def load_state_dict(self, d):
         """Validates d, then restores it into this object's own tensors (stats too, which may be a view into the

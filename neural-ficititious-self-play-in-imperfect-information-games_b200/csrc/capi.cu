@@ -42,6 +42,8 @@ extern "C" int nfsp_env_create(int rules, int64_t n_games, uint64_t seed, uint64
     *out = nullptr;
     NFSP_CHECK_ARG(rules == NFSP_RULES_LEGACY || rules == NFSP_RULES_NFSP, "unknown rules %d", rules);
     NFSP_CHECK_ARG(n_games >= 1 && n_games <= (int64_t)1 << 31, "n_games out of range");
+    // Philox counter word 0 holds the low half of the global game id: game 2^32 would replay game 0's deals
+    NFSP_CHECK_ARG(game0 <= ((uint64_t)1 << 32) - (uint64_t)n_games, "game0 + n_games must not exceed 2^32");
     int count = 0;
     // no CPU fallback: without a CUDA device this fails loudly
     NFSP_CUDA(cudaGetDeviceCount(&count));

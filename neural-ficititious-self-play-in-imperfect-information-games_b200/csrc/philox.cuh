@@ -74,9 +74,12 @@ __device__ __forceinline__ Philox4 game_block(const PhiloxKeys &K, uint64_t game
     return philox4x32_10((uint32_t)game, (uint32_t)step, (uint32_t)(step >> 32), stream, K);
 }
 
+// Counter (idx, idx >> 32 | call >> 32, call, stream).  No stream uses both high halves: the reservoir stream draws with
+// call 0, the sample stream with idx = draw index < 1024.  So the whole 64-bit ticket and the whole 64-bit call key the
+// draw, and every draw of a call below 2^32 is the one it always was.
 __device__ __forceinline__ uint64_t buffer_u64(uint64_t seed, uint64_t idx, uint64_t call, uint32_t stream) {
-    const Philox4 o = philox4x32_10((uint32_t)idx, (uint32_t)(idx >> 32), (uint32_t)call, stream, (uint32_t)seed,
-                                    (uint32_t)(seed >> 32));
+    const Philox4 o = philox4x32_10((uint32_t)idx, (uint32_t)(idx >> 32) | (uint32_t)(call >> 32), (uint32_t)call, stream,
+                                    (uint32_t)seed, (uint32_t)(seed >> 32));
     return (uint64_t)o.x | ((uint64_t)o.y << 32);
 }
 

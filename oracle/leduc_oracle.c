@@ -635,9 +635,11 @@ void orc_ring_insert(OrcRing *r, const void *recs, int64_t n) { /* replay_buffer
     }
 }
 
+/* counter (idx, idx >> 32 | call >> 32, call, stream): the reservoir stream draws with call 0, the sample stream with
+   idx < 1024, so the whole 64-bit ticket and the whole 64-bit call key the draw (DESIGN.md "Philox streams") */
 static uint64_t buffer_u64(uint64_t seed, uint64_t idx, uint64_t call, uint32_t stream) {
     uint32_t key[2] = {(uint32_t)seed, (uint32_t)(seed >> 32)};
-    uint32_t ctr[4] = {(uint32_t)idx, (uint32_t)(idx >> 32), (uint32_t)call, stream};
+    uint32_t ctr[4] = {(uint32_t)idx, (uint32_t)(idx >> 32) | (uint32_t)(call >> 32), (uint32_t)call, stream};
     uint32_t o[4];
     orc_philox4x32_10(ctr, key, o);
     return (uint64_t)o[0] | ((uint64_t)o[1] << 32);

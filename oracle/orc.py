@@ -285,10 +285,12 @@ class LegacyBatch:
         return lib().orc_legacy_batch_env(self.h, g).contents
 
 
-def ring_insert_all(recs: np.ndarray, cap: int, chunks=None):
-    """Sequential FIFO ring fed with `recs` (structured array); returns (data[cap], count, total)."""
-    data = np.zeros(cap, recs.dtype)
-    r = Ring(data.ctypes.data, cap, 0, 0, recs.dtype.itemsize)
+def ring_insert_all(recs: np.ndarray, cap: int, total0: int = 0, data=None):
+    """Sequential FIFO ring fed with `recs` (structured array); returns (data[cap], count, total).  A ring mid-life
+    starts at total0 records ever inserted with storage `data` (updated in place)."""
+    if data is None:
+        data = np.zeros(cap, recs.dtype)
+    r = Ring(data.ctypes.data, cap, min(total0, cap), total0, recs.dtype.itemsize)
     recs = np.ascontiguousarray(recs)
     lib().orc_ring_insert(C.byref(r), recs.ctypes.data, len(recs))
     return data, r.count, r.total
@@ -301,6 +303,11 @@ def reservoir_insert_all(recs: np.ndarray, cap: int, seed: int, mode: int = 0, t
     recs = np.ascontiguousarray(recs)
     lib().orc_reservoir_insert(C.byref(r), recs.ctypes.data, len(recs))
     return data, r.count, r.total
+
+
+def reservoir_slot(seed, ticket, cap, mode=0):
+    """Slot the record with this ticket replaces in a reservoir of `cap` slots, -1 if it is dropped."""
+    return int(lib().orc_reservoir_slot(seed, ticket, cap, mode))
 
 
 def sample_indices(seed, call_idx, count, batch):

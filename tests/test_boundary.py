@@ -72,6 +72,9 @@ def test_argument_errors_are_reported(nb):
     assert nb.lib().nfsp_env_create(7, 8, 1, 0, 0, ctypes.byref(h)) == -1
     assert b"rules" in nb.lib().nfsp_last_error()
     assert nb.lib().nfsp_env_create(1, 0, 1, 0, 0, ctypes.byref(h)) == -1
+    # game ids past 2^32 would replay the deals of game id - 2^32 (Philox counter word 0 is the low half)
+    assert nb.lib().nfsp_env_create(1, 8, 1, 2 ** 32 - 7, 0, ctypes.byref(h)) == -1
+    assert b"2^32" in nb.lib().nfsp_last_error()
     assert nb.lib().nfsp_expand_obs(None, 4, None, None) == -1
 
 

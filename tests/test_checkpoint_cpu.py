@@ -47,3 +47,19 @@ def test_a_save_that_fails_part_way_keeps_the_previous_file(tmp_path, monkeypatc
     assert os.listdir(d) == ["rank0-of-1.pt"]
     assert open(os.path.join(d, "rank0-of-1.pt"), "rb").read() == before
     assert checkpoint.load(d) == {"calls": 3}
+
+
+def test_counters_are_bounded_by_what_holds_them():
+    """A memory's total lives in an int64 tensor, the step and draw counters go to the library as uint64: values they
+    cannot hold are refused with the field named, before anything is loaded (torch would refuse total = 2^63 only after
+    the slots were overwritten; ctypes would wrap step 2^64 + 5 to 5)."""
+    from nfsp_b200.batched import check_numbers
+
+    mem = dict(below=dict(total=2 ** 63, sample_calls=2 ** 64), total=int, sample_calls=int)
+    check_numbers(dict(total=2 ** 63 - 1, sample_calls=2 ** 64 - 1), "memory", **mem)
+    for field, d in (("total", dict(total=2 ** 63, sample_calls=0)), ("sample_calls", dict(total=0, sample_calls=2 ** 64))):
+        with pytest.raises(ValueError, match="%s must be below" % field):
+            check_numbers(d, "memory", **mem)
+    check_numbers(dict(step=2 ** 64 - 1), "SelfPlay", below=dict(step=2 ** 64), step=int)
+    with pytest.raises(ValueError, match="step must be below 2\\*\\*64"):
+        check_numbers(dict(step=2 ** 64 + 5), "SelfPlay", below=dict(step=2 ** 64), step=int)

@@ -106,19 +106,25 @@ def test_forward_tensor_core_mixed_nets_ragged(nb):
 
 
 @pytest.mark.parametrize("variant", ["states", "pairs", "sorted", "cuda", "tcgen05", "tcgen05_ws"])
-@pytest.mark.parametrize("n,steps,eta,eps", [(1, 30, 0.5, 0.5), (1000, 12, 0.1, 0.06), (50_000, 8, 0.3, 0.2)])
-def test_fused_rollout_vs_oracle(nb, n, steps, eta, eps, variant):
-    """The fused act+step+remember kernel vs the oracle's restatement of Agent.play/main.train."""
+@pytest.mark.parametrize("n,steps,eta,eps,step0", [
+    pytest.param(1, 30, 0.5, 0.5, 1, id="1-30-0.5-0.5"),
+    pytest.param(1000, 12, 0.1, 0.06, 1, id="1000-12-0.1-0.06"),
+    pytest.param(1000, 12, 0.1, 0.06, 2 ** 32 - 5, id="1000-12-0.1-0.06-step0=4294967291"),
+    pytest.param(50_000, 8, 0.3, 0.2, 1, id="50000-8-0.3-0.2")])
+def test_fused_rollout_vs_oracle(nb, n, steps, eta, eps, step0, variant):
+    """The fused act+step+remember kernel vs the oracle's restatement of Agent.play/main.train, from step counter
+    step0 on (2^32 - 5: the launch crosses 2^32, where the counter's high word enters Philox counter word 2)."""
     seed = 2024
     w = random_nets(5)
     sp = nb.SelfPlay(n, weights=torch.from_numpy(w), seed=seed, eta=eta, epsilon=eps, rl_capacity=1 << 12,
                      sl_capacity=1 << 12, max_steps_per_call=steps, variant=variant)
+    sp.env.step_counter = step0
     out = sp.rollout(steps, insert=False, debug=True)
     rl, sl = sp.staged()
     vec = out["vec"].cpu().numpy()
     b = orc.NfspBatch(n, seed)
     b.reset(0, orc.u32_frac(eta))
-    ref = b.rollout_act(1, steps, oracle_nets(nb, w), orc.u32_frac(eta), orc.u32_frac(eps), forced_vec=vec)
+    ref = b.rollout_act(step0, steps, oracle_nets(nb, w), orc.u32_frac(eta), orc.u32_frac(eps), forced_vec=vec)
     tr = out["raw"].cpu().numpy().view(np.uint32)
     assert np.array_equal(tr[0], ref["trace"]["obs"])
     assert np.array_equal(tr[1].view(np.float32), ref["trace"]["reward"])
@@ -413,7 +419,8 @@ def test_direct_ring_append_equals_the_staged_insert(nb, variant):
     """direct_rings: the rollout kernel writes the RL records into the rings itself (ticket = atomic add on the ring's
     total, slot = ticket % capacity; replay_buffer.py:30-41).  Launch by launch the records are those the staged path
     moves with nfsp_ring_insert (same seed, same games) and those of the oracle; after the rings have wrapped they hold
-    every record of the last launches and the most recent part of the launch the wrap cuts."""
+    every record of the last launches and the most recent part of the launch the wrap cuts.  The rings start a few
+    launches below 2^32 tickets, so the kernel's division-free ticket % capacity meets tickets on both sides of it."""
     from collections import Counter
 
     n, steps, seed, launches = 3000, 4, 21, 11
@@ -421,6 +428,10 @@ def test_direct_ring_append_equals_the_staged_insert(nb, variant):
     mk = lambda direct: nb.SelfPlay(n, seed=seed, eta=0.3, epsilon=0.1, rl_capacity=cap, sl_capacity=1 << 12,  # noqa: E731
                                     max_steps_per_call=steps, variant=variant, direct_rings=direct)
     sd, ss = mk(True), mk(False)
+    T0 = 2 ** 32 - cap - 5  # three to four launches' worth of one player's records below 2^32
+    for sp in (sd, ss):
+        for m in sp.rl:
+            m.total.fill_(T0)
     b = orc.NfspBatch(n, seed)
     b.reset(0, orc.u32_frac(0.3))
     nets = oracle_nets(nb, nb.glorot_nets(seed, "cuda").cpu().numpy())
@@ -437,13 +448,14 @@ def test_direct_ring_append_equals_the_staged_insert(nb, variant):
         sd.rollout(steps)  # production kernel, rings written in place, flush() only moves the SL records
         for p in range(2):
             assert int(sd.rl[p].total.item()) - before[p] == len(rl[p]) and int(sd.rl[p].total.item()) == int(ss.rl[p].total.item())
-            if int(sd.rl[p].total.item()) <= cap:  # not wrapped yet: the same multiset in the same span of slots
-                t = int(sd.rl[p].total.item())
-                assert np.array_equal(canon(sd.rl[p].data[:t].cpu().numpy()), canon(ss.rl[p].data[:t].cpu().numpy()))
+            # the launch's tickets [before, total) land in the same span of slots, ticket % cap, as one multiset
+            span = torch.from_numpy((before[p] % cap + np.arange(len(rl[p]))) % cap)
+            assert np.array_equal(canon(sd.rl[p].data[span].cpu().numpy()), canon(ss.rl[p].data[span].cpu().numpy())), (k, p)
+            assert np.array_equal(canon(sd.rl[p].data[span].cpu().numpy()), canon(rl[p]))
     assert np.array_equal(sd.env.state_words().cpu().numpy(), ss.env.state_words().cpu().numpy())
     assert sd.read_stats() == ss.read_stats() and int(sd.counts.sum().item()) == 0
     for p in range(2):
-        assert int(sd.rl[p].total.item()) > 2 * cap  # wrapped at least twice
+        assert int(sd.rl[p].total.item()) - T0 > 2 * cap and int(sd.rl[p].total.item()) > 2 ** 32 + cap // 2  # wrapped twice
         for q in range(2):  # the reservoirs went through the staged path in both objects, fed in different orders
             assert int(sd.sl[q].total.item()) == int(ss.sl[q].total.item())
         have = Counter(_rows(sd.rl[p].data.cpu().numpy()))

@@ -85,11 +85,16 @@ def _resumed(nb, tmp_path, sp, ln, calls, make):
     return c, lc
 
 
-def _resume_and_compare(nb, tmp_path, make, k, K):
+def _resume_and_compare(nb, tmp_path, make, k, K, age=None):
+    """a runs K iterations; b runs k, is saved and resumed as c, which runs the rest: c must stay equal to a.  age(sp)
+    moves a run's counters before the save (a and b alike)."""
     a, la = make()
     b, lb = make()
     outs = [_iterate(a, la, it) for it in range(k)]
     assert [_iterate(b, lb, it) for it in range(k)] == outs
+    if age is not None:
+        age(a)
+        age(b)
     c, lc = _resumed(nb, tmp_path, b, lb, k, make)
     _assert_same(a, c, la, lc, "resumed")
     for it in range(k, K):
@@ -111,8 +116,19 @@ def test_sequential_resume_with_wrapped_rings_and_replacing_reservoirs(nb, tmp_p
         _iterate(probe, lp, it)
     for m in probe.rl + probe.sl:
         assert int(m.total.item()) > m.capacity   # wrapped / replacing when the checkpoint is taken
-    _, _, outs = _resume_and_compare(nb, tmp_path, lambda: _make(nb, **kw), k, K)
+
+    def age(sp):
+        """A long-lived run: step counter, tickets and draw counters past 2^32 when the checkpoint is taken (the high
+        words are carried by the file and key the draws after the resume)."""
+        sp.env.step_counter = sp.env.step_counter + 2 ** 32 - 7
+        for m in sp.rl + sp.sl:
+            m.total.add_(2 ** 32 + 2 ** 33 * (m in sp.sl) + 12345)
+            m.sample_calls += 2 ** 32 + 5
+
+    a, _, outs = _resume_and_compare(nb, tmp_path, lambda: _make(nb, **kw), k, K, age=age)
     assert all(o["trained"] == 0xF for o in outs[1:])
+    assert a.env.step_counter > 2 ** 32 and all(m.sample_calls > 2 ** 32 and int(m.total.item()) > 2 ** 32
+                                                for m in a.rl + a.sl)
 
 
 def test_sequential_resume_before_every_memory_is_ready(nb, tmp_path):
@@ -305,6 +321,20 @@ def test_refusals_leave_the_target_as_it_was(nb, tmp_path, monkeypatch):
         bad.mkdir()
         torch.save(dict(state, **edit), str(bad / "rank0-of-1.pt"))
         with pytest.raises(ValueError, match=name):
+            checkpoint.load(str(bad), selfplay=t, learner=lt)
+        _same_state(before, (t.state_dict(), lt.state_dict()), name)
+    # counters their holders cannot store: a memory total of 2^63 (an int64 tensor), a step counter or a draw counter of
+    # 2^64 (uint64) -- refused before anything is written, not wrapped or half-loaded
+    sp_state = state["selfplay"]
+    for name, field, edit in (("total", "total", lambda s: s["sl"][1].update(total=2 ** 63)),
+                              ("step", "step", lambda s: s.update(step=2 ** 64)),
+                              ("calls", "sample_calls", lambda s: s["rl"][0].update(sample_calls=2 ** 64))):
+        sp_bad = dict(sp_state, rl=[dict(m) for m in sp_state["rl"]], sl=[dict(m) for m in sp_state["sl"]])
+        edit(sp_bad)
+        bad = tmp_path / name
+        bad.mkdir()
+        torch.save(dict(state, selfplay=sp_bad), str(bad / "rank0-of-1.pt"))
+        with pytest.raises(ValueError, match=field):
             checkpoint.load(str(bad), selfplay=t, learner=lt)
         _same_state(before, (t.state_dict(), lt.state_dict()), name)
     # a single run's file loaded without its learner

@@ -130,22 +130,37 @@ def test_nfsp_do_action_alone_golden(nb, golden_dir):
                 assert np.array_equal(one.last_action[0], g["last_action"][i, c])
 
 
-@pytest.mark.parametrize("n,steps", [(1, 40), (257, 33), (100_000, 24)])
-def test_nfsp_env_seeded_rollout_vs_oracle(nb, n, steps):
-    """Philox deals + uniform-random actions + auto re-deal: trace planes bit-exact vs the oracle."""
+def _with_step0(cases):
+    """Each case at step counters 1 (a fresh run), 2^32 - 5 (the launch crosses 2^32, where the counter's high word
+    enters Philox counter word 2) and 2^40 + 3 (a resumed run of a long life); a fresh run keeps its old test id."""
+    params = []
+    for case in cases:
+        for step0 in (1, 2 ** 32 - 5, 2 ** 40 + 3):
+            tag = "-".join(map(str, case)) + ("" if step0 == 1 else "-step0=%d" % step0)
+            params.append(pytest.param(*case, step0, id=tag))
+    return params
+
+
+@pytest.mark.parametrize("n,steps,step0", _with_step0([(1, 40), (257, 33), (100_000, 24)]))
+def test_nfsp_env_seeded_rollout_vs_oracle(nb, n, steps, step0):
+    """Philox deals + uniform-random actions + auto re-deal: trace planes bit-exact vs the oracle, from step counter
+    step0 on."""
     seed, eta = 1234, 0.1
     env = nb.BatchedNfspEnv(n, seed=seed, eta=eta)
     env.reset()
+    env.step_counter = step0
     tr = env.step(n_steps=steps, trace=True)["raw"].cpu().numpy().view(np.uint32)
+    assert env.step_counter == step0 + steps
     b = orc.NfspBatch(n, seed)
     b.reset(0, orc.u32_frac(eta))
-    ref = b.rollout_env(1, steps, orc.u32_frac(eta))
+    ref = b.rollout_env(step0, steps, orc.u32_frac(eta))
     assert np.array_equal(tr[0], ref["obs"])
     assert np.array_equal(tr[1].view(np.float32), ref["reward"])
     assert np.array_equal(tr[2], ref["misc"])
     # the same rollout, one launch per step, lands in the same packed words
     env2 = nb.BatchedNfspEnv(n, seed=seed, eta=eta)
     env2.reset()
+    env2.step_counter = step0
     for _ in range(steps):
         env2.step(n_steps=1)
     assert torch.equal(env.state_words(), env2.state_words())
@@ -287,15 +302,16 @@ def test_legacy_env_golden_call_order_fuzz(nb, golden_dir):
             assert np.array_equal(st, g["st"][:, c, q]), (c, q)
 
 
-@pytest.mark.parametrize("n,iters", [(1, 30), (1000, 17), (100_000, 12)])
-def test_legacy_seeded_rollout_vs_oracle(nb, n, iters):
+@pytest.mark.parametrize("n,iters,step0", _with_step0([(1, 30), (1000, 17), (100_000, 12)]))
+def test_legacy_seeded_rollout_vs_oracle(nb, n, iters, step0):
     seed = 4321
     env = nb.BatchedLegacyEnv(n, seed=seed)
     env.reset()
+    env.step_counter = step0
     rec = env.rollout(iters, trace=True)["raw"].cpu().numpy()
     b = orc.LegacyBatch(n, seed)
     b.reset(0)
-    ref = b.rollout(1, iters)
+    ref = b.rollout(step0, iters)
     w = rec[0].view(np.uint32)
     sb = lambda x: ((x & 0xFF).astype(np.int16) ^ 0x80) - 0x80  # noqa: E731
     assert np.array_equal(sb(w), ref["card"]) and np.array_equal(sb(w >> 8), ref["pub"])

@@ -225,28 +225,33 @@ UPDATE_SEED = 12   # fit_case seed of the Learner.update() test (gate margin >= 
 def test_learner_update_trains_each_net_with_its_learning_rate(nb):
     """Learner.update() end to end on crafted memories: the host's learning-rate-to-net mapping, its minibatch slicing
     and the sampled positions, against the reference run on the rows the update sampled and the learning rates it had
-    before its decay."""
+    before its decay.  The memories are long-lived (totals past 2^32): a ring's oldest record sits at slot head =
+    total % capacity, so the crafted rows are stored rotated by head and deque position i is crafted row i."""
     from nfsp_b200.learner import GRAD, Learner
 
     c = lo.fit_case(UPDATE_SEED, 128)
     sp = nb.SelfPlay(64, seed=5, rl_capacity=SLOTS, sl_capacity=SLOTS)
     sp.set_weights(torch.tensor(c["w"], dtype=torch.float32, device=sp.device))
     rng = np.random.RandomState(99)
+    total = 2 ** 32 + 3 * SLOTS + 17
+    head = total % SLOTS
+    assert head != 0
     for p in range(2):
         rl, sl = _slot_words(c, p, rng)
-        sp.rl[p].store.copy_(rl)
+        sp.rl[p].store.copy_(torch.roll(rl, head, 0))
         sp.sl[p].store.copy_(sl)
-        sp.rl[p].total.fill_(SLOTS)    # full memories: every net trains and every draw lands on a crafted slot
-        sp.sl[p].total.fill_(SLOTS)
+        sp.rl[p].total.fill_(total)    # full memories: every net trains and every draw lands on a crafted slot
+        sp.sl[p].total.fill_(total + 2 ** 40)
     L = Learner(sp, gamma=GAMMA)
     L.target = torch.tensor(c["w_target"], dtype=torch.float32, device=sp.device)
     L.lr_ar, L.lr_br = 0.01, [0.05, 0.02]
     lr = [L.lr_ar, L.lr_br[0], L.lr_ar, L.lr_br[1]]
     out = L.update()
     assert out["trained"] == 0xF and L.lr_br[0] < 0.05       # the rates decayed after the fit
-    pos = L._pos.cpu().numpy()
-    for k, mem in enumerate((sp.rl[0], sp.rl[1], sp.sl[0], sp.sl[1])):   # full ring: deque position == slot
-        assert np.array_equal(pos[k], orc.sample_indices(mem.seed, 0, SLOTS, 128)), k
+    slots = L._pos.cpu().numpy()
+    pos = [orc.sample_indices(mem.seed, 0, SLOTS, 128) for mem in (sp.rl[0], sp.rl[1], sp.sl[0], sp.sl[1])]
+    for k in range(4):   # a ring's deque position i is slot (head + i) % capacity; a reservoir's is its slot
+        assert np.array_equal(slots[k], (head + pos[k]) % SLOTS if k < 2 else pos[k]), k
     rl = [c["rl_slots"][p][pos[p]] for p in range(2)]
     sl = [c["sl_slots"][p][pos[2 + p]] for p in range(2)]
     ref = _reference(c, (128, 32, 2), rl=rl, sl=sl, lr=lr)

@@ -94,6 +94,44 @@ def test_runs_train_bit_for_bit_like_standalone_runs(nb):
         assert ex[r] == exploitability(solo[r][0]), r
 
 
+def test_runs_at_different_counters_train_like_standalone_runs(nb):
+    """Runs of one batch at their own step counters, ring tickets and draw counters -- a fresh run, one whose counters
+    cross 2^32 during the test and one far past it (a resumed long run): the batched launches take each run's 64-bit
+    counters, so every run still equals the same run driven alone, iteration by iteration."""
+    from nfsp_b200.runs import RunBatch
+
+    ages = [(0, 0, 0), (2 ** 32 - 20, 2 ** 32 - 40_000, 2 ** 32 - 2), (2 ** 40 + 3, 2 ** 62 + 5, 2 ** 40 + 7)]
+    kw = dict(rl_capacity=1 << 16, sl_capacity=1 << 16, max_steps_per_call=8, deterministic=True)
+
+    def aged(r):
+        s, e, ep, lb, la = CONFIGS[r]
+        sp, ln = _run(nb, 4096, s, e, list(ep), lb, la, **kw)
+        step, total, calls = ages[r]
+        sp.env.step_counter = sp.env.step_counter + step
+        for m in sp.rl:
+            m.total.add_(total)
+        for m in sp.rl + sp.sl:
+            m.sample_calls += calls
+        return sp, ln
+
+    solo = [aged(r) for r in range(3)]
+    runs = [aged(r) for r in range(3)]
+    rb = RunBatch([sp for sp, _ in runs], [ln for _, ln in runs])
+    for it in range(6):
+        for sp, ln in solo:
+            sp.rollout(8)
+            if it >= 2:
+                ln.update(sync=False)
+        rb.rollout(8)
+        if it >= 2:
+            rb.update(sync=False)
+        for r in range(3):
+            _assert_same_run(solo[r][0], runs[r][0], solo[r][1], runs[r][1], "iteration %d run %d" % (it, r))
+    sp1 = runs[1][0]
+    assert sp1.env.step_counter > 2 ** 32 and all(int(m.total.item()) > 2 ** 32 and m.sample_calls > 2 ** 32
+                                                  for m in sp1.rl)
+
+
 def _rows(a):
     return [bytes(x) for x in np.ascontiguousarray(a).view(np.uint8).reshape(len(a), -1)]
 
