@@ -1,7 +1,8 @@
 """Checkpoints of training runs: save a run's whole state to a directory and resume it bit for bit.
 
 A checkpoint is a directory with one `torch.save` file per rank, `rank{r}-of-{world}.pt`.  Each file holds the format
-version, the world size and rank, a small driver record (the training loop's `calls` counter) and the `state_dict()` of
+version, the world size and rank, a small driver record (the training loop's `calls` counter; a sweep's also holds its
+run list and world size, main.py --sweep) and the `state_dict()` of
 every object it was given: a SelfPlay and its Learner (plus a PipelinedTrainer), or a RunBatch.  Every random draw of a
 run is Philox keyed by counters those state dicts carry (the env step counter, each memory's `total` and
 `sample_calls`), so a run loaded from a checkpoint continues exactly as the saved one would have, wherever that run is
@@ -18,6 +19,8 @@ import tempfile
 
 import torch
 import torch.distributed as dist
+
+from .sweep import record_difference
 
 FORMAT = 1
 PARTS = ("selfplay", "learner", "trainer", "runs")
@@ -38,12 +41,15 @@ def _given(selfplay, learner, trainer, runs):
     return {k: v for k, v in objs.items() if v is not None}
 
 
-def save(path, calls, selfplay=None, learner=None, trainer=None, runs=None):
+def save(path, calls, selfplay=None, learner=None, trainer=None, runs=None, sweep=None):
     """Writes this rank's file of the checkpoint directory `path` (created if missing): the driver record {"calls":
-    calls} and the state dicts of the objects given.  Every state dict is taken before anything is written, so a refusal
-    (records staged but not flushed) leaves the directory as it was."""
+    calls} (plus {"sweep": sweep}, a sweep.record(), when given) and the state dicts of the objects given.  Every state
+    dict is taken before anything is written, so a refusal (records staged but not flushed) leaves the directory as it
+    was."""
     rank, world = _rank_world()
     state = dict(format=FORMAT, world=world, rank=rank, driver=dict(calls=int(calls)))
+    if sweep is not None:
+        state["driver"]["sweep"] = sweep
     for name, obj in _given(selfplay, learner, trainer, runs).items():
         state[name] = obj.state_dict()
     os.makedirs(path, exist_ok=True)
@@ -68,9 +74,13 @@ def save(path, calls, selfplay=None, learner=None, trainer=None, runs=None):
         os.close(dfd)
 
 
-def _read(path, rank, world, objs):
+def _read(path, rank, world, objs, sweep=None):
     """This rank's file, checked against the objects without changing them; raises ValueError."""
     fname = os.path.join(path, file_name(rank, world))
+    others = sorted(f for f in os.listdir(path) if f.startswith("rank%d-of-" % rank)) if os.path.isdir(path) else []
+    if not os.path.exists(fname) and others:
+        raise ValueError("%s is missing: the checkpoint was saved by another number of ranks (%s) than the %d here" %
+                         (fname, ", ".join(others), world))
     try:
         state = torch.load(fname, map_location="cpu", weights_only=True)
     except Exception as e:  # noqa: BLE001  a missing or unreadable file is a refusal like any other
@@ -84,6 +94,12 @@ def _read(path, rank, world, objs):
     driver = state.get("driver")
     if not (isinstance(driver, dict) and type(driver.get("calls")) is int and driver["calls"] >= 0):
         raise ValueError("%s: no driver record with a calls counter" % fname)
+    if sweep is not None:
+        why = record_difference(driver.get("sweep"), sweep)
+        if why is not None:
+            raise ValueError("%s: %s" % (fname, why))
+    elif "sweep" in driver:
+        raise ValueError("%s: the checkpoint is of a sweep (--sweep)" % fname)
     held = sorted(k for k in PARTS if k in state)
     if held != sorted(objs):
         raise ValueError("%s: the checkpoint holds %s but %s were given" % (fname, held, sorted(objs)))
@@ -92,16 +108,17 @@ def _read(path, rank, world, objs):
     return state
 
 
-def load(path, selfplay=None, learner=None, trainer=None, runs=None) -> dict:
+def load(path, selfplay=None, learner=None, trainer=None, runs=None, sweep=None) -> dict:
     """Loads this rank's file of the checkpoint directory `path` into the objects given and returns the driver record.
-    Everything is validated first -- format, world size, rank, the objects' shapes (n_games, game0, capacities, ...)
-    and, with several ranks, that every rank's file holds the same `calls` -- and all ranks agree on the outcome with
-    one collective, so they refuse together (ValueError) and every object is then left as it was."""
+    Everything is validated first -- format, world size, rank, the objects' shapes (n_games, game0, capacities, ...),
+    the sweep's run list when `sweep` (a sweep.record()) is given, and, with several ranks, that every rank's file holds
+    the same `calls` -- and all ranks agree on the outcome with one collective, so they refuse together (ValueError) and
+    every object is then left as it was."""
     rank, world = _rank_world()
     objs = _given(selfplay, learner, trainer, runs)
     state, why = None, None
     try:
-        state = _read(path, rank, world, objs)
+        state = _read(path, rank, world, objs, sweep)
     except ValueError as e:
         why = str(e)
     if world > 1:

@@ -42,7 +42,7 @@ def _world():
 class Learner:
     def __init__(self, selfplay, cfg=None, minibatch=128, fit_batch=32, epochs=2, lr_br=0.05, lr_ar=0.1, gamma=0.95,
                  target_update_rate=150, terminal_bootstraps=False, fused=True, use_multicast=True, others_to_target=False,
-                 peer_transport="auto"):
+                 peer_transport="auto", data_parallel=True):
         if cfg is not None:
             minibatch = cfg.getint("Agent", "MiniBatchSize")
             lr_br, lr_ar = cfg.getfloat("Agent", "LearningRateBR"), cfg.getfloat("Agent", "LearningRateAR")
@@ -50,6 +50,9 @@ class Learner:
             target_update_rate = cfg.getint("Agent", "TargetModelUpdateRate")
         self.sp = selfplay
         self.device = selfplay.device
+        # data_parallel=False: this learner trains its own run alone and ignores an initialised process group (no peer
+        # exchange, no gradient all-reduce, no agreement on the ready mask) -- a run of a sweep spread over ranks
+        self.data_parallel = bool(data_parallel)
         self.minibatch, self.fit_batch, self.epochs = int(minibatch), int(fit_batch), int(epochs)
         self.lr_br0, self.lr_ar, self.gamma = float(lr_br), float(lr_ar), float(gamma)
         self.lr_br = [self.lr_br0, self.lr_br0]
@@ -67,7 +70,7 @@ class Learner:
         if peer_transport not in ("auto", "symm", "ipc"):
             raise ValueError("peer_transport must be 'auto', 'symm' or 'ipc'")
         self.peer_transport = peer_transport
-        if self.fused and _world() > 1 and self.minibatch <= _lib.FIT_ROWS_MAX_MINIBATCH and self.fit_batch <= _lib.FIT_ROWS_MAX_STEP:
+        if self.fused and self._world() > 1 and self.minibatch <= _lib.FIT_ROWS_MAX_MINIBATCH and self.fit_batch <= _lib.FIT_ROWS_MAX_STEP:
             # every rank must take the same path (a rank in the peer exchange and one in an NCCL all-reduce would wait
             # for each other forever): _setup_peers agrees on every phase collectively
             self._setup_peers()
@@ -77,11 +80,15 @@ class Learner:
         self.exploitability = [0.0, 0.0]
         self.updates = 0
 
+    def _world(self):
+        """The ranks this learner trains over: every rank of the process group, or 1 without data_parallel."""
+        return _world() if self.data_parallel else 1
+
     @property
     def one_launch(self) -> bool:
         """The whole fit runs as one kernel (one GPU, or several with the peer exchange): what weights_in / weights_out
         and PipelinedTrainer need.  The same on every rank (the peer set-up is collective)."""
-        return self.fused and (_world() == 1 or self._peers is not None)
+        return self.fused and (self._world() == 1 or self._peers is not None)
 
     def _snapshot_buffers(self):
         """Where the sampling launch leaves packed copies of the sampled records (4 x minibatch rows, 24 KB): once they
@@ -307,7 +314,7 @@ class Learner:
         sp = self.sp
         io, lr = self._fit_args(idx_rl, idx_sl, mask, row0=row0, rows=rows)
         check(lib().nfsp_learner_grads(C.byref(io), _stream(self.device)))
-        world = _world()
+        world = self._world()
         if world > 1:  # C1 (gradients) + C2 (exploitability stats) in one collective
             dist.all_reduce(self.flat, op=dist.ReduceOp.SUM)
         lr = (C.c_float * 4)(*lr)
@@ -325,7 +332,7 @@ class Learner:
                 mask |= 1 << (2 * p)
             if sp.rl[p].size() > self.minibatch:
                 mask |= 1 << (2 * p + 1)
-        if _world() > 1:  # every rank must take the same decision or the replicas diverge
+        if self._world() > 1:  # every rank must take the same decision or the replicas diverge
             m = torch.tensor([(mask >> k) & 1 for k in range(4)], dtype=torch.int32, device=self.device)
             dist.all_reduce(m, op=dist.ReduceOp.MIN)
             mask = sum(int(v) << k for k, v in enumerate(m.tolist()))

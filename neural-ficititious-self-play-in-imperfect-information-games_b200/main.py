@@ -4,6 +4,15 @@
     python -m torch.distributed.run --nproc-per-node G -m nfsp_b200.main ...     # games sharded over G GPUs
     python -m nfsp_b200.main --runs R ...     # R independent runs (seeds Seed, Seed + 1, ...) side by side on one GPU
     python -m nfsp_b200.main --checkpoint DIR ...   # save the training state; --resume DIR continues it (DESIGN.md 7c)
+    python -m torch.distributed.run --nproc-per-node G -m nfsp_b200.main --sweep Eta=0.05,0.1 --sweep LearningRateBR=0.01,0.05 \
+        --runs R --results FILE ...   # a grid of settings x R seeds, independent runs spread over G ranks (DESIGN.md 7d)
+
+A sweep (`--sweep KEY=V1,V2,...`, repeatable; the keys of sweep.RUN_KEYS, with or without their section) trains the
+Cartesian product of the values given, each grid point with R seeds, as independent runs of `--games` games each.  The
+ranks take contiguous blocks of runs, one RunBatch each, and never shard a run; rank r uses cuda:(LOCAL_RANK % the
+number of visible GPUs), so several ranks may share a GPU.  Every report gathers every run's row on every rank, adds the
+mean and standard deviation of the exact exploitability over each grid point's seeds, and rank 0 prints them and
+appends them to `--results FILE` (JSON Lines).
 
 The reference plays one hand at a time: `train(env, player1, player2)` alternates the dealer, draws each
 player's per-hand policy with probability eta, lets the agents `play` until both have seen the terminal
@@ -20,13 +29,16 @@ reads), same seeds, same printed quantities.  `--human` is accepted and ignored,
 from __future__ import annotations
 
 import argparse
+import json
+import os
 import statistics
 import time
 
 import torch
+import torch.distributed as dist
 
 from . import checkpoint as ckpt
-from . import sharding
+from . import sharding, sweep
 from .batched import SelfPlay
 from .config import load_config
 from .exploitability import exploitability
@@ -179,6 +191,112 @@ def train_runs(rb: RunBatch, episodes: int, steps_per_call: int = 8, report_ever
             return rows
 
 
+def _gather(obj):
+    """[rank 0's obj, rank 1's obj, ...] over the process group (one all_gather_object), or [obj] without one."""
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size() == 1:
+        return [obj]
+    out = [None] * dist.get_world_size()
+    dist.all_gather_object(out, obj)
+    return out
+
+
+def _keep_results(path, calls):
+    """The results file as a run resumed at `calls` continues it: the lines of later reports dropped."""
+    lines = []
+    if os.path.exists(path):
+        with open(path) as f:
+            lines = [ln for ln in f if ln.strip() and json.loads(ln)["calls"] <= calls]
+    with open(path, "w") as f:
+        f.writelines(lines)
+
+
+def _point_rows(run_rows, calls, true_exploitability):
+    """One row per grid point: its runs and seeds and, with the exact exploitability, its mean and standard deviation
+    over the seeds."""
+    out = []
+    for p in sorted({r["point"] for r in run_rows}):
+        rs = [r for r in run_rows if r["point"] == p]
+        row = {"kind": "point", "calls": calls, "point": p, "hparams": rs[0]["hparams"], "runs": [r["run"] for r in rs],
+               "seeds": [r["seed"] for r in rs], "hands": min(r["hands"] for r in rs)}
+        if true_exploitability:
+            values = [r["exploitability"]["value"] for r in rs]
+            row["exploitability_mean"] = statistics.fmean(values)
+            row["exploitability_std"] = statistics.stdev(values) if len(values) > 1 else 0.0
+        out.append(row)
+    return out
+
+
+def train_sweep(rb: RunBatch, runs, record, episodes: int, steps_per_call: int = 8, report_every: int = 100, log=print,
+                true_exploitability: bool = True, results=None, checkpoint=None, checkpoint_every: int = CHECKPOINT_EVERY,
+                resume=None):
+    """train_runs() for one rank's block of a sweep.  `runs` are the definitions (sweep.expand) of rb's runs in order,
+    `record` the whole sweep's checkpoint record (sweep.record).  At a report call every rank evaluates its own runs
+    (counters, the proxy, the exact exploitability) and one all_gather_object gives every rank every run's row, in run
+    order, followed by one row per grid point (_point_rows); every rank returns the same rows and stops at the same call,
+    once every run of the sweep has played `episodes` hands.  results: a file rank 0 writes those rows to as JSON Lines
+    (on resume, first without the lines of reports after the checkpoint).  checkpoint / checkpoint_every / resume: as in
+    train(); the file also holds `record`, and a resume of another sweep or world size is refused on every rank."""
+    rank = dist.get_rank() if dist.is_available() and dist.is_initialized() else 0
+    rows, calls, tr0 = [], 0, [0] * rb.n_runs
+    if resume is not None:
+        calls = ckpt.load(resume, runs=rb, sweep=record)["calls"]
+        saved = [sp.read_stats() for sp in rb.sps]
+        tr0 = [s["transitions"] for s in saved]
+        if results is not None and rank == 0:
+            _keep_results(results, calls)
+        if _stopped(calls, report_every, min(h for hs in _gather([s["hands"] for s in saved]) for h in hs), episodes):
+            return rows
+    elif results is not None and rank == 0:
+        open(results, "w").close()
+    t0 = time.time()
+    while True:
+        calls += 1
+        report = _is_report(calls, report_every)
+        sts = rb.step(steps_per_call, sync=report)
+        if not report:
+            if checkpoint is not None and calls % checkpoint_every == 0:
+                ckpt.save(checkpoint, calls, runs=rb, sweep=record)
+            continue
+        dt = max(time.time() - t0, 1e-9)
+        ex = rb.exploitability() if true_exploitability else None
+        mine = []
+        for k, (run, sp, st) in enumerate(zip(runs, rb.sps, sts)):
+            stats = sp.read_stats()
+            row = {"kind": "run", "calls": calls, "run": run["run"], "rank": rank, "point": run["point"], "seed": run["seed"],
+                   "hparams": dict(run["hparams"]), "hands": stats["hands"], "transitions": stats["transitions"],
+                   "exploitability_proxy": st.get("exploitability"),
+                   "actions": [sampled_actions(stats, p) for p in range(2)],
+                   "transitions_per_sec": (stats["transitions"] - tr0[k]) / dt}
+            if true_exploitability:
+                row["exploitability"] = ex[k]
+            mine.append(row)
+        run_rows = [r for part in _gather(mine) for r in part]
+        new = run_rows + _point_rows(run_rows, calls, true_exploitability)
+        rows.extend(new)
+        log("================ Stats ==================")
+        for r in new:
+            hp = " ".join("%s=%s" % kv for kv in r["hparams"].items())
+            if r["kind"] == "run":
+                line = "run %d (rank %d, seed %d, %s): hands %d  exploitability proxy %s" % (
+                    r["run"], r["rank"], r["seed"], hp, r["hands"], r["exploitability_proxy"])
+                if true_exploitability:
+                    line += "  exact exploitability %.4f chips/hand" % r["exploitability"]["value"]
+            else:
+                line = "point %d (%s): %d seeds" % (r["point"], hp, len(r["seeds"]))
+                if true_exploitability:
+                    line += "  exact exploitability mean %.4f  std %.4f chips/hand" % (r["exploitability_mean"],
+                                                                                      r["exploitability_std"])
+            log(line)
+        if results is not None and rank == 0:
+            with open(results, "a") as f:
+                f.writelines(json.dumps(r) + "\n" for r in new)
+        done = min(r["hands"] for r in run_rows) >= episodes
+        if checkpoint is not None and (done or calls % checkpoint_every == 0):
+            ckpt.save(checkpoint, calls, runs=rb, sweep=record)
+        if done:
+            return rows
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(description="NFSP self-play on Leduc Hold'em, B200-native")
     ap.add_argument("--human", action="store_true", help="accepted and ignored, as in the reference (main.py:152-158)")
@@ -200,7 +318,13 @@ def main(argv=None):
     ap.add_argument("--updates-per-call", type=int, default=1,
                     help="update_strategy() calls per rollout call (the reference's cadence: games * steps / 256)")
     ap.add_argument("--runs", type=int, default=1,
-                    help="independent runs with seeds Seed, Seed + 1, ... trained side by side on one GPU, their launches shared")
+                    help="independent runs with seeds Seed, Seed + 1, ... trained side by side on one GPU, their launches shared; "
+                         "with --sweep, the seeds of every grid point")
+    ap.add_argument("--sweep", action="append", default=None, metavar="KEY=V1,V2,...",
+                    help="train every combination of the values given (repeatable; keys: %s, with or without their "
+                         "section), --runs seeds each, as independent runs spread over all ranks" % ", ".join(sweep.RUN_KEYS))
+    ap.add_argument("--results", metavar="FILE", default=None,
+                    help="with --sweep: write every reported row of every run and grid point to FILE as JSON Lines")
     ap.add_argument("--checkpoint", metavar="DIR", default=None,
                     help="save the training state to DIR every --checkpoint-every rollout calls and when training ends")
     ap.add_argument("--checkpoint-every", type=int, default=CHECKPOINT_EVERY, metavar="CALLS",
@@ -212,34 +336,64 @@ def main(argv=None):
     rank, world, local = sharding.env_rank_world()
     if args.runs < 1:
         ap.error("--runs must be at least 1")
-    if args.runs > 1 and (args.pipelined or world > 1):
+    runs = None
+    if args.sweep is not None:
+        if args.pipelined:
+            ap.error("--sweep trains with the sequential loop: not with --pipelined")
+        if args.updates_per_call != 1:
+            ap.error("--sweep runs one update per rollout call: not --updates-per-call %d" % args.updates_per_call)
+        if args.variant not in ("default", "states"):
+            ap.error("--sweep plays the state-table rollout (--variant default / states): not --variant %s" % args.variant)
+        try:
+            runs = sweep.expand(sweep.parse_axes(args.sweep), args.runs, cfg)
+            sweep.check_layout(len(runs), world)
+        except ValueError as e:
+            ap.error(str(e))
+    elif args.runs > 1 and (args.pipelined or world > 1):
         ap.error("--runs > 1 trains on one GPU with the sequential loop: not with --pipelined or more than one rank")
+    if args.results is not None and runs is None:
+        ap.error("--results needs --sweep")
     if args.checkpoint_every < 1:
         ap.error("--checkpoint-every must be at least 1")
     saving = dict(checkpoint=args.checkpoint, checkpoint_every=args.checkpoint_every, resume=args.resume)
+    if runs is not None:   # several ranks may share a GPU: a sweep's ranks exchange nothing on the device
+        local %= max(torch.cuda.device_count(), 1)
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
-    if world > 1:
-        import torch.distributed as dist
-
+    if world > 1 and runs is not None:   # host-side collectives only: the report gather, the stop, the checkpoint agreement
+        dist.init_process_group("gloo")
+    elif world > 1:
         dist.init_process_group("nccl", device_id=dev)
     seed = cfg.getint("Utils", "Seed")              # main.py:132-133
     game0, n = sharding.shard_games(args.games, rank, world)
     episodes = args.episodes if args.episodes is not None else cfg.getint("Common", "Episodes")
 
-    def make_run(run_seed):
-        sp_ = SelfPlay(n, seed=run_seed, game0=game0, device=dev, eta=cfg.getfloat("Agent", "Eta"),
-                       epsilon=cfg.getfloat("Agent", "Epsilon"), rl_capacity=cfg.getint("Agent", "MRLSize"),
+    def make_run(run_seed, hp, n=n, game0=game0, data_parallel=True):
+        sp_ = SelfPlay(n, seed=run_seed, game0=game0, device=dev, eta=hp["Eta"], epsilon=hp["Epsilon"],
+                       rl_capacity=cfg.getint("Agent", "MRLSize"),
                        sl_capacity=cfg.getint("Agent", "MSLSize"), max_steps_per_call=args.steps_per_call,
                        deterministic=args.deterministic, direct_rings=False if args.deterministic else "auto",
                        variant=args.variant)
-        return sp_, Learner(sp_, cfg=cfg, terminal_bootstraps=args.terminal_bootstraps, others_to_target=args.others_to_target)
+        return sp_, Learner(sp_, minibatch=cfg.getint("Agent", "MiniBatchSize"), lr_br=hp["LearningRateBR"],
+                            lr_ar=hp["LearningRateAR"], gamma=hp["Gamma"], target_update_rate=hp["TargetModelUpdateRate"],
+                            terminal_bootstraps=args.terminal_bootstraps, others_to_target=args.others_to_target,
+                            data_parallel=data_parallel)
 
+    if runs is not None:   # no run is sharded: run i plays games 0 .. --games - 1 whatever the world size
+        mine = [runs[i] for i in sweep.rank_runs(len(runs), rank, world)]
+        rb = RunBatch(*zip(*[make_run(r["seed"], r["hparams"], args.games, 0, False) for r in mine]))
+        rows = train_sweep(rb, mine, sweep.record(runs, world), episodes, args.steps_per_call, args.report_every,
+                           log=print if rank == 0 else (lambda *a, **k: None),
+                           true_exploitability=not args.no_true_exploitability, results=args.results, **saving)
+        if world > 1:
+            dist.destroy_process_group()
+        return rows
+    hp = sweep.config_hparams(cfg)
     if args.runs > 1:
-        rb = RunBatch(*zip(*[make_run(seed + r) for r in range(args.runs)]))
+        rb = RunBatch(*zip(*[make_run(seed + r, hp) for r in range(args.runs)]))
         return train_runs(rb, episodes, args.steps_per_call, args.report_every,
                           true_exploitability=not args.no_true_exploitability, **saving)
-    sp, learner = make_run(seed)
+    sp, learner = make_run(seed, hp)
     rows = train(sp, learner, episodes, args.steps_per_call, args.report_every, world,
                  log=print if rank == 0 else (lambda *a, **k: None),
                  true_exploitability=not args.no_true_exploitability, pipelined=args.pipelined,

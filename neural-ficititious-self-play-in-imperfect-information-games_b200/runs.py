@@ -38,7 +38,8 @@ class RunBatch:
 
     selfplays[r] is trained by learners[r].  The runs must share device, n_games, max_steps_per_call, the default
     ("states") rollout variant, direct_rings, deterministic, the memories' capacities and the learner's minibatch, fit
-    batch, epochs and flags; seeds, eta, epsilons and learning rates are each run's own.  One GPU only."""
+    batch, epochs and flags; seeds, eta, epsilons and learning rates are each run's own.  One GPU only; with a process
+    group of several ranks (a sweep, sweep.py) every learner must train alone (Learner(data_parallel=False))."""
 
     def __init__(self, selfplays, learners):
         sps, lns = list(selfplays), list(learners)
@@ -46,8 +47,9 @@ class RunBatch:
             raise ValueError("one learner per self-play, at least one run")
         if len(sps) > _lib.MAX_RUNS:
             raise ValueError("at most %d runs per batch" % _lib.MAX_RUNS)
-        if _world() > 1:
-            raise ValueError("a RunBatch trains its runs on one GPU: world > 1 is not supported")
+        if _world() > 1 and any(ln.data_parallel for ln in lns):
+            raise ValueError("a RunBatch trains its runs on one GPU: world > 1 needs learners that train alone "
+                             "(Learner(data_parallel=False))")
         if len({id(sp) for sp in sps}) != len(sps):
             raise ValueError("a self-play appears twice")
         for r, (sp, ln) in enumerate(zip(sps, lns)):
