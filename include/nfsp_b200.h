@@ -393,6 +393,28 @@ int nfsp_peer_buffer_destroy(int device, void *d_buf);
  * all-reduce.  lr is a HOST array of 4 floats. */
 int nfsp_sgd_apply(float *d_weights, const float *d_grad, const float lr[4], float scale, void *stream);
 
+/* ---- Adam instead of SGD: Keras 2's keras.optimizers.Adam, beta1 = 0.9, beta2 = 0.999, epsilon = 1e-7 (fixed).
+ * Step t (t = 1, 2, ... per net) on the mean gradient g, which is the gradient the SGD entries apply:
+ *   m = beta1 m + (1 - beta1) g;  v = beta2 v + (1 - beta2) g^2;  w -= lr sqrt(1 - beta2^t) / (1 - beta1^t) m / (sqrt(v) + eps)
+ * The state of one run: the moments of its four nets (device, zero at the start, updated in place) and the steps each
+ * net has taken so far.  A net outside net_mask takes no step: its weights and moments are left alone, and the caller
+ * leaves its t0 as it was; a net inside it takes the call's steps, t0[k] + 1 ... t0[k] + steps. */
+typedef struct {
+    float *d_m;      /* [4][NFSP_NET_PARAMS] first moments, index player*2 + policy */
+    float *d_v;      /* [4][NFSP_NET_PARAMS] second moments                          */
+    int64_t t0[4];   /* steps of each net before this call, in [0, 2^62]             */
+} nfsp_adam_state;
+/* nfsp_learner_fit, nfsp_learner_fit_runs (adam[r] = run r's state) and nfsp_learner_fit_peers with Adam steps. */
+int nfsp_learner_fit_adam(const nfsp_learner_io *io, int minibatch, int fit_batch, int epochs, const float lr[4],
+                          float *d_weights_out, const nfsp_adam_state *adam, void *stream);
+int nfsp_learner_fit_runs_adam(const nfsp_learner_io *io, int n_runs, int minibatch, int fit_batch, int epochs, const float *lr,
+                               float *const *d_weights_out, const nfsp_adam_state *adam, void *stream);
+int nfsp_learner_fit_peers_adam(const nfsp_learner_io *io, int minibatch, int fit_batch, int epochs, const float lr[4],
+                                float *d_weights_out, const nfsp_peers *peers, const nfsp_adam_state *adam, void *stream);
+/* nfsp_sgd_apply's counterpart: step t0[k] + 1 of each net k in net_mask on the mean gradient scale * grad[k]. */
+int nfsp_adam_apply(float *d_weights, const float *d_grad, const float lr[4], float scale, int net_mask,
+                    const nfsp_adam_state *adam, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

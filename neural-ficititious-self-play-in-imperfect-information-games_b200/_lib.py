@@ -28,6 +28,7 @@ SYMBOLS = [
     "nfsp_act_set_weights", "nfsp_act_set_weights_from_host", "nfsp_act_forward", "nfsp_act_forward_tc", "nfsp_rollout", "nfsp_rollout_with_weights", "nfsp_rollout_runs", "nfsp_rollout_tune", "nfsp_rollout_profile",
     "nfsp_ring_insert", "nfsp_reservoir_insert", "nfsp_insert_multi", "nfsp_ring_insert_multi", "nfsp_reservoir_insert_multi", "nfsp_sample_indices", "nfsp_sample_minibatches", "nfsp_gather_rl", "nfsp_gather_sl",
     "nfsp_learner_grads", "nfsp_learner_fit", "nfsp_learner_fit_runs", "nfsp_learner_fit_peers", "nfsp_sgd_apply",
+    "nfsp_learner_fit_adam", "nfsp_learner_fit_runs_adam", "nfsp_learner_fit_peers_adam", "nfsp_adam_apply",
     "nfsp_peer_buffer_create", "nfsp_peer_buffer_open", "nfsp_peer_buffer_close", "nfsp_peer_buffer_destroy",
 ]
 
@@ -71,6 +72,10 @@ class LearnerIO(C.Structure):
                 ("d_rl_idx", C.c_void_p * 2), ("d_sl", C.c_void_p * 2), ("d_sl_idx", C.c_void_p * 2),
                 ("row0", C.c_int32), ("rows", C.c_int32), ("gamma", C.c_float), ("net_mask", C.c_int32),
                 ("terminal_bootstraps", C.c_int32), ("others_to_target", C.c_int32), ("d_grad", C.c_void_p), ("d_stats", C.c_void_p)]
+
+
+class AdamState(C.Structure):
+    _fields_ = [("d_m", C.c_void_p), ("d_v", C.c_void_p), ("t0", C.c_int64 * 4)]
 
 
 class NfspError(RuntimeError):
@@ -149,6 +154,13 @@ def lib():
     L.nfsp_learner_fit_peers.argtypes = [C.POINTER(LearnerIO), C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float), vp,
                                          C.POINTER(Peers), vp]
     L.nfsp_sgd_apply.argtypes = [vp, vp, C.POINTER(C.c_float * 4), C.c_float, vp]
+    L.nfsp_learner_fit_adam.argtypes = [C.POINTER(LearnerIO), C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float), vp,
+                                        C.POINTER(AdamState), vp]
+    L.nfsp_learner_fit_runs_adam.argtypes = [C.POINTER(LearnerIO), C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float),
+                                             C.POINTER(vp), C.POINTER(AdamState), vp]
+    L.nfsp_learner_fit_peers_adam.argtypes = [C.POINTER(LearnerIO), C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float), vp,
+                                              C.POINTER(Peers), C.POINTER(AdamState), vp]
+    L.nfsp_adam_apply.argtypes = [vp, vp, C.POINTER(C.c_float * 4), C.c_float, C.c_int, C.POINTER(AdamState), vp]
     L.nfsp_peer_buffer_create.argtypes = [C.c_int, C.POINTER(vp), C.c_char_p]
     L.nfsp_peer_buffer_open.argtypes = [C.c_int, C.c_char_p, C.POINTER(vp)]
     L.nfsp_peer_buffer_close.argtypes = [C.c_int, vp]

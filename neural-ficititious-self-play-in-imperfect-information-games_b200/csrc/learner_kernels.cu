@@ -292,6 +292,30 @@ struct FitRun {
     float lr[4];
 };
 
+// ---- Adam (Keras 2's keras.optimizers.Adam with its fixed constants), the optimizer a fit may use instead of SGD ----
+// One run's state: the moments of its four nets, updated in place, and the steps each net has taken before this call.
+struct AdamRun {
+    float *m, *v;        // [4][2179]
+    long long t0[4];
+    // step k (0, 1, ...) of this call for net `net`, without a local copy of t0 (net is not a compile-time index)
+    __device__ __forceinline__ long long t(int net, int k) const {
+        return (net == 0 ? t0[0] : (net == 1 ? t0[1] : (net == 2 ? t0[2] : t0[3]))) + k + 1;
+    }
+};
+constexpr float kAdamBeta1 = 0.9f, kAdamBeta2 = 0.999f, kAdamEps = 1e-7f;
+constexpr float kAdamLog2Beta1 = -0.15200309344504997f, kAdamLog2Beta2 = -0.0014434168696687186f;  // log2 of the betas
+// Step t (1, 2, ...) of one weight on the mean gradient g: every Adam path calls this, so they differ only in where
+// g comes from.  lr_t = lr * sqrt(1 - beta2^t) / (1 - beta1^t) is the same for every weight of a net and step (the
+// register kernel computes it once per step; a thread of the row kernel updates at most three weights).  beta^t is
+// exp2(t log2 beta): a few instructions where powf takes a hundred, within 2 ulp of it.
+__device__ __forceinline__ void adam_step(float &w, float &m, float &v, float g, float lr, long long t) {
+    const float tf = (float)t;
+    const float lr_t = lr * sqrtf(1.0f - exp2f(tf * kAdamLog2Beta2)) / (1.0f - exp2f(tf * kAdamLog2Beta1));
+    m = kAdamBeta1 * m + (1.0f - kAdamBeta1) * g;
+    v = kAdamBeta2 * v + (1.0f - kAdamBeta2) * (g * g);
+    w -= lr_t * m / (sqrtf(v) + kAdamEps);
+}
+
 // Exchange buffer of one rank (the RECEIVER owns it): two parities x four nets x one slot per sending rank of kPeerSlot
 // 8-byte words {value, epoch} -- 2179 mean gradients, then loss sum, exploitability sum, rows.  A sender PUSHES its values
 // into the slot it has in every rank's buffer (its own included); a receiver polls its own memory until a word carries
@@ -329,8 +353,14 @@ __device__ __forceinline__ float ld_volatile_f32(const float *p) {
     asm volatile("ld.volatile.global.f32 %0, [%1];" : "=f"(v) : "l"(p) : "memory");
     return v;
 }
-// the register kernel's work on net `net` of run P
-__device__ __forceinline__ void fit_regs_net(const FitSchedule &F, const FitRun &P, int net) {
+// the register kernel's work on net `net` of run P; kAdam: Adam steps on the state M, else SGD steps (M is not read).
+// The moments live in dynamic shared memory, laid out as part[0] (row i < 34: the weights of hidden unit j; row 34: b2):
+// loaded once, stored once.  In registers beside the weights they would be live through every row of the step sums,
+// and at 255 registers the kernel spills.  Every group updates its copy of the weights from the same moments; after a
+// barrier, group 0 writes the new moments back.
+constexpr int kRegsAdamSmem = 2 * 35 * 64 * (int)sizeof(float);
+template <bool kAdam>
+__device__ __forceinline__ void fit_regs_net(const FitSchedule &F, const FitRun &P, const AdamRun &M, int net) {
     __shared__ float red_all[kRowGroups][4][2][4];
     __shared__ float part[kRowGroups][40][64];
     const LearnerArgs &A = P.A;
@@ -345,21 +375,70 @@ __device__ __forceinline__ void fit_regs_net(const FitSchedule &F, const FitRun 
     if (pre) prefetch_rows(A, net, 0, F.minibatch, s_rec);
     NetState N;
     N.load(A, net, j);
+    extern __shared__ float regs_adam_smem[];
+    float (*mom)[35][64] = reinterpret_cast<float (*)[35][64]>(regs_adam_smem);  // [m, v][row][hidden unit]
+    // the flat index of row i, hidden unit j (b2: row 34, j < 3)
+    auto flat = [](int i, int jj) { return i < 30 ? i * 64 + jj : (i == 30 ? 1920 + jj : (i < 34 ? 1984 + jj * 3 + (i - 31) : 2176 + jj)); };
+    if constexpr (kAdam) {
+        // the first step's barriers order these stores before any read
+        for (int e = threadIdx.x; e < 35 * 64; e += kLearnThreads) {
+            const int i = e >> 6, jj = e & 63;
+            if (i < 34 || jj < 3) {
+                mom[0][i][jj] = M.m[net * NFSP_NET_PARAMS + flat(i, jj)];
+                mom[1][i][jj] = M.v[net * NFSP_NET_PARAMS + flat(i, jj)];
+            }
+        }
+    }
     const float lr = P.lr[net];
     for (int k = 0; k < F.n_steps; ++k) {
         step_sums(A, N, net, F.row0[k], F.rows[k], red_all, part, pre ? s_rec : nullptr, 0);
         if (k == 0) write_stats(A.stats, net, F.rows[k], part);
         const float inv_rows = 1.0f / (float)F.rows[k];
-        // the same arithmetic as sgd_apply_kernel on the stored mean gradient: w -= lr * 1.0f * (sum * inv_rows)
+        if constexpr (kAdam) {
+            const long long t = M.t(net, k);
+            float mw[34], vw[34], mb2[3], vb2[3];
 #pragma unroll
-        for (int i = 0; i < 30; ++i) N.W.w1[i] -= lr * 1.0f * (part[0][i][j] * inv_rows);
-        N.W.b1 -= lr * 1.0f * (part[0][30][j] * inv_rows);
+            for (int i = 0; i < 34; ++i) { mw[i] = mom[0][i][j]; vw[i] = mom[1][i][j]; }
 #pragma unroll
-        for (int c = 0; c < 3; ++c) {
-            N.W.w2[c] -= lr * 1.0f * (part[0][31 + c][j] * inv_rows);
-            N.b2[c] -= lr * 1.0f * (part[0][34][c] * inv_rows);
+            for (int c = 0; c < 3; ++c) { mb2[c] = mom[0][34][c]; vb2[c] = mom[1][34][c]; }
+#pragma unroll
+            for (int i = 0; i < 30; ++i) adam_step(N.W.w1[i], mw[i], vw[i], part[0][i][j] * inv_rows, lr, t);
+            adam_step(N.W.b1, mw[30], vw[30], part[0][30][j] * inv_rows, lr, t);
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+                adam_step(N.W.w2[c], mw[31 + c], vw[31 + c], part[0][31 + c][j] * inv_rows, lr, t);
+                adam_step(N.b2[c], mb2[c], vb2[c], part[0][34][c] * inv_rows, lr, t);
+            }
+            __syncthreads();  // every group has read this step's moments
+            if (threadIdx.x < 64) {
+#pragma unroll
+                for (int i = 0; i < 34; ++i) { mom[0][i][j] = mw[i]; mom[1][i][j] = vw[i]; }
+                if (j == 0) {
+#pragma unroll
+                    for (int c = 0; c < 3; ++c) { mom[0][34][c] = mb2[c]; mom[1][34][c] = vb2[c]; }
+                }
+            }
+        } else {
+            // the same arithmetic as sgd_apply_kernel on the stored mean gradient: w -= lr * 1.0f * (sum * inv_rows)
+#pragma unroll
+            for (int i = 0; i < 30; ++i) N.W.w1[i] -= lr * 1.0f * (part[0][i][j] * inv_rows);
+            N.W.b1 -= lr * 1.0f * (part[0][30][j] * inv_rows);
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+                N.W.w2[c] -= lr * 1.0f * (part[0][31 + c][j] * inv_rows);
+                N.b2[c] -= lr * 1.0f * (part[0][34][c] * inv_rows);
+            }
         }
         __syncthreads();  // part[] is rewritten by the next step
+    }
+    if constexpr (kAdam) {  // after the last step's barrier: group 0's moments are complete
+        for (int e = threadIdx.x; e < 35 * 64; e += kLearnThreads) {
+            const int i = e >> 6, jj = e & 63;
+            if (i < 34 || jj < 3) {
+                M.m[net * NFSP_NET_PARAMS + flat(i, jj)] = mom[0][i][jj];
+                M.v[net * NFSP_NET_PARAMS + flat(i, jj)] = mom[1][i][jj];
+            }
+        }
     }
     if (threadIdx.x >= 64) return;
     float *w = P.w_out + net * NFSP_NET_PARAMS;
@@ -371,7 +450,9 @@ __device__ __forceinline__ void fit_regs_net(const FitSchedule &F, const FitRun 
     if (j < 3) w[2176 + j] = N.b2[j];
 }
 __global__ void __launch_bounds__(kLearnThreads)
-learner_fit_kernel(const FitSchedule S, const FitRun P) { fit_regs_net(S, P, blockIdx.x); }
+learner_fit_kernel(const FitSchedule S, const FitRun P) { fit_regs_net<false>(S, P, AdamRun{}, blockIdx.x); }
+__global__ void __launch_bounds__(kLearnThreads)
+learner_fit_adam_kernel(const FitSchedule S, const FitRun P, const AdamRun M) { fit_regs_net<true>(S, P, M, blockIdx.x); }
 
 // ---- fit(), the row-parallel formulation ------------------------------------------------------------
 // The register kernel above is bound by instruction latency: a CTA of 256 threads per net, eight rows one after the
@@ -396,10 +477,18 @@ __device__ __forceinline__ void warp_sum9(float (&v)[9]) {
         for (int k = 0; k < 9; ++k) v[k] += __shfl_xor_sync(0xFFFFFFFFu, v[k], o);
     }
 }
-// the row-parallel kernel's work on net `net` of run P
-__device__ __forceinline__ void fit_rows_net(const FitSchedule &F, const FitRun &P, int net) {
+// Adam: the moments of the net, behind RowFitSmem in the dynamic shared memory of the row-parallel kernel
+struct RowFitMoments {
+    float m[2180], v[2180];
+};
+constexpr int kRowFitAdamSmem = (int)(sizeof(RowFitSmem) + sizeof(RowFitMoments));
+// the row-parallel kernel's work on net `net` of run P; kAdam: Adam steps on the state M (its moments in shared memory
+// from the first step to the last), else SGD steps (M is not read)
+template <bool kAdam>
+__device__ __forceinline__ void fit_rows_net(const FitSchedule &F, const FitRun &P, const AdamRun &M, int net) {
     extern __shared__ __align__(16) unsigned char fit_smem_raw[];
     RowFitSmem &S = *reinterpret_cast<RowFitSmem *>(fit_smem_raw);
+    RowFitMoments &SM = *reinterpret_cast<RowFitMoments *>(fit_smem_raw + sizeof(RowFitSmem));
     __shared__ int s_peer_lost;  // a peer did not answer within the time limit of the gradient exchange
     const LearnerArgs &A = P.A;
     const int player = net >> 1, is_br = net & 1, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -412,6 +501,10 @@ __device__ __forceinline__ void fit_rows_net(const FitSchedule &F, const FitRun 
     for (int e = threadIdx.x; e < NFSP_NET_PARAMS; e += kRowThreads) {
         S.w[e] = A.w[net * NFSP_NET_PARAMS + e];
         if (is_br) S.wt[e] = A.w_target[player * NFSP_NET_PARAMS + e];
+        if constexpr (kAdam) {
+            SM.m[e] = M.m[net * NFSP_NET_PARAMS + e];
+            SM.v[e] = M.v[net * NFSP_NET_PARAMS + e];
+        }
     }
     prefetch_rows(A, net, 0, F.minibatch, S.rec);  // ends with a CTA barrier
     const float lr = P.lr[net];
@@ -506,6 +599,8 @@ __device__ __forceinline__ void fit_rows_net(const FitSchedule &F, const FitRun 
                 if (F.mc) ll_store(F.mc, ll_index(parity, net, F.rank, e), v, epoch);
                 else
                     for (int r = 0; r < F.world; ++r) ll_store(F.peer[r], ll_index(parity, net, F.rank, e), v, epoch);
+            } else if constexpr (kAdam) {
+                adam_step(S.w[e], SM.m[e], SM.v[e], g * inv_rows, lr, M.t(net, k));
             } else {
                 S.w[e] -= lr * 1.0f * (g * inv_rows);
             }
@@ -569,7 +664,8 @@ __device__ __forceinline__ void fit_rows_net(const FitSchedule &F, const FitRun 
             for (int e = threadIdx.x; e < NFSP_NET_PARAMS; e += kRowThreads) {
                 float g = 0.f;
                 for (int r = 0; r < F.world; ++r) g += ll_wait(mybuf, ll_index(parity, net, r, e), epoch, &lost);
-                S.w[e] -= lr * scale * g;
+                if constexpr (kAdam) adam_step(S.w[e], SM.m[e], SM.v[e], scale * g, lr, M.t(net, k));
+                else S.w[e] -= lr * scale * g;
             }
             if (k == 0 && threadIdx.x == 0) {
                 float ls = 0.f, ex = 0.f, rw = 0.f;
@@ -596,10 +692,18 @@ __device__ __forceinline__ void fit_rows_net(const FitSchedule &F, const FitRun 
         }
         __syncthreads();
     }
-    for (int e = threadIdx.x; e < NFSP_NET_PARAMS; e += kRowThreads) P.w_out[net * NFSP_NET_PARAMS + e] = S.w[e];
+    for (int e = threadIdx.x; e < NFSP_NET_PARAMS; e += kRowThreads) {
+        P.w_out[net * NFSP_NET_PARAMS + e] = S.w[e];
+        if constexpr (kAdam) {
+            M.m[net * NFSP_NET_PARAMS + e] = SM.m[e];
+            M.v[net * NFSP_NET_PARAMS + e] = SM.v[e];
+        }
+    }
 }
 __global__ void __launch_bounds__(kRowThreads, 1)
-learner_fit_rows_kernel(const FitSchedule S, const FitRun P) { fit_rows_net(S, P, blockIdx.x); }
+learner_fit_rows_kernel(const FitSchedule S, const FitRun P) { fit_rows_net<false>(S, P, AdamRun{}, blockIdx.x); }
+__global__ void __launch_bounds__(kRowThreads, 1)
+learner_fit_rows_adam_kernel(const FitSchedule S, const FitRun P, const AdamRun M) { fit_rows_net<true>(S, P, M, blockIdx.x); }
 
 // ---- the fits of independent runs in one launch (nfsp_learner_fit_runs): CTA 4 r + k = net k of run r ------------------
 struct FitRuns {
@@ -607,9 +711,26 @@ struct FitRuns {
     FitSchedule S;              // world = 1
 };
 __global__ void __launch_bounds__(kLearnThreads)
-learner_fit_runs_kernel(const __grid_constant__ FitRuns R) { fit_regs_net(R.S, R.run[blockIdx.x >> 2], blockIdx.x & 3); }
+learner_fit_runs_kernel(const __grid_constant__ FitRuns R) {
+    fit_regs_net<false>(R.S, R.run[blockIdx.x >> 2], AdamRun{}, blockIdx.x & 3);
+}
 __global__ void __launch_bounds__(kRowThreads, 1)
-learner_fit_rows_runs_kernel(const __grid_constant__ FitRuns R) { fit_rows_net(R.S, R.run[blockIdx.x >> 2], blockIdx.x & 3); }
+learner_fit_rows_runs_kernel(const __grid_constant__ FitRuns R) {
+    fit_rows_net<false>(R.S, R.run[blockIdx.x >> 2], AdamRun{}, blockIdx.x & 3);
+}
+// the same with each run's Adam state
+struct FitRunsAdam {
+    FitRuns R;
+    AdamRun adam[NFSP_MAX_RUNS];
+};
+__global__ void __launch_bounds__(kLearnThreads)
+learner_fit_runs_adam_kernel(const __grid_constant__ FitRunsAdam R) {
+    fit_regs_net<true>(R.R.S, R.R.run[blockIdx.x >> 2], R.adam[blockIdx.x >> 2], blockIdx.x & 3);
+}
+__global__ void __launch_bounds__(kRowThreads, 1)
+learner_fit_rows_runs_adam_kernel(const __grid_constant__ FitRunsAdam R) {
+    fit_rows_net<true>(R.R.S, R.R.run[blockIdx.x >> 2], R.adam[blockIdx.x >> 2], blockIdx.x & 3);
+}
 
 // w[k] -= lr[k] * scale * grad[k]   (keras.optimizers.SGD without momentum, agent.py:45-46)
 __global__ void sgd_apply_kernel(float *__restrict__ w, const float *__restrict__ grad, float lr0, float lr1, float lr2,
@@ -619,6 +740,18 @@ __global__ void sgd_apply_kernel(float *__restrict__ w, const float *__restrict_
     const int net = e / NFSP_NET_PARAMS;
     const float lr = net == 0 ? lr0 : (net == 1 ? lr1 : (net == 2 ? lr2 : lr3));
     w[e] -= lr * scale * grad[e];
+}
+
+// the Adam counterpart: step t0[k] + 1 of the nets k in net_mask on the mean gradient scale * grad[k]; the other nets'
+// weights and moments are left alone (a zero gradient would still move them under Adam)
+__global__ void adam_apply_kernel(float *__restrict__ w, const float *__restrict__ grad, const AdamRun M, float lr0, float lr1,
+                                  float lr2, float lr3, float scale, int net_mask) {
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= kGradFloats) return;
+    const int net = e / NFSP_NET_PARAMS;
+    if (!((net_mask >> net) & 1)) return;
+    const float lr = net == 0 ? lr0 : (net == 1 ? lr1 : (net == 2 ? lr2 : lr3));
+    adam_step(w[e], M.m[e], M.v[e], scale * grad[e], lr, M.t(net, 0));
 }
 
 }  // namespace nfsp
@@ -674,13 +807,26 @@ static int fit_schedule(int minibatch, int fit_batch, int epochs, const nfsp_pee
     return NFSP_OK;
 }
 
+static int make_adam_run(const nfsp_adam_state *s, AdamRun &M) {
+    NFSP_CHECK_ARG(s != nullptr && s->d_m && s->d_v, "null Adam state");
+    NFSP_CHECK_ARG(s->d_m != s->d_v, "the Adam moments m and v must be separate buffers");
+    M.m = s->d_m; M.v = s->d_v;
+    for (int k = 0; k < 4; ++k) {
+        NFSP_CHECK_ARG(s->t0[k] >= 0 && s->t0[k] <= (int64_t)1 << 62, "Adam step count t0[%d] out of range", k);
+        M.t0[k] = (long long)s->t0[k];
+    }
+    return NFSP_OK;
+}
+
 // The fits of n_runs runs on one schedule, CTA 4 r + k = net k of run r: the row-parallel kernel (one warp per row,
 // weights in shared memory) when the minibatch and a step fit its shared memory, the register kernel otherwise; one run
-// launches the single-run kernels, which read their arguments from the constant bank.
+// launches the single-run kernels, which read their arguments from the constant bank.  adam: one Adam state per run, or
+// null for SGD.
 static int learner_fit(const nfsp_learner_io *io, int n_runs, int minibatch, int fit_batch, int epochs, const float *lr,
-                       float *const *d_weights_out, const nfsp_peers *peers, cudaStream_t st) {
+                       float *const *d_weights_out, const nfsp_peers *peers, const nfsp_adam_state *adam, cudaStream_t st) {
     NFSP_CHECK_ARG(io && lr && d_weights_out, "null argument");
-    FitRuns R;
+    FitRunsAdam RA;
+    FitRuns &R = RA.R;
     int rc = fit_schedule(minibatch, fit_batch, epochs, peers, R.S);
     if (rc != NFSP_OK) return rc;
     for (int r = 0; r < n_runs; ++r) {
@@ -689,8 +835,23 @@ static int learner_fit(const nfsp_learner_io *io, int n_runs, int minibatch, int
         if (rc != NFSP_OK) return rc;
         R.run[r].w_out = d_weights_out[r];
         for (int k = 0; k < 4; ++k) R.run[r].lr[k] = lr[4 * r + k];
+        if (adam) {
+            rc = make_adam_run(adam + r, RA.adam[r]);
+            if (rc != NFSP_OK) return rc;
+        }
     }
     const bool rows = minibatch <= kMaxFitRows && fit_batch <= kMaxStepRows;
+    if (adam) {
+        void (*single)(FitSchedule, FitRun, AdamRun) = rows ? learner_fit_rows_adam_kernel : learner_fit_adam_kernel;
+        void (*batch)(FitRunsAdam) = rows ? learner_fit_rows_runs_adam_kernel : learner_fit_runs_adam_kernel;
+        const int threads = rows ? kRowThreads : kLearnThreads, smem = rows ? kRowFitAdamSmem : kRegsAdamSmem;
+        NFSP_CUDA(cudaFuncSetAttribute(n_runs == 1 ? (const void *)single : (const void *)batch,
+                                           cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        if (n_runs == 1) single<<<4, threads, smem, st>>>(R.S, R.run[0], RA.adam[0]);
+        else batch<<<4 * n_runs, threads, smem, st>>>(RA);
+        NFSP_LAUNCH_CHECK();
+        return NFSP_OK;
+    }
     void (*single)(FitSchedule, FitRun) = rows ? learner_fit_rows_kernel : learner_fit_kernel;
     void (*batch)(FitRuns) = rows ? learner_fit_rows_runs_kernel : learner_fit_runs_kernel;
     const int threads = rows ? kRowThreads : kLearnThreads, smem = rows ? (int)sizeof(RowFitSmem) : 0;
@@ -705,11 +866,16 @@ static int learner_fit(const nfsp_learner_io *io, int n_runs, int minibatch, int
 
 extern "C" int nfsp_learner_fit(const nfsp_learner_io *io, int minibatch, int fit_batch, int epochs, const float lr[4],
                                 float *d_weights_out, void *stream) {
-    return learner_fit(io, 1, minibatch, fit_batch, epochs, lr, &d_weights_out, nullptr, (cudaStream_t)stream);
+    return learner_fit(io, 1, minibatch, fit_batch, epochs, lr, &d_weights_out, nullptr, nullptr, (cudaStream_t)stream);
 }
 
-extern "C" int nfsp_learner_fit_peers(const nfsp_learner_io *io, int minibatch, int fit_batch, int epochs, const float lr[4],
-                                      float *d_weights_out, const nfsp_peers *peers, void *stream) {
+extern "C" int nfsp_learner_fit_adam(const nfsp_learner_io *io, int minibatch, int fit_batch, int epochs, const float lr[4],
+                                     float *d_weights_out, const nfsp_adam_state *adam, void *stream) {
+    NFSP_CHECK_ARG(adam, "null Adam state");
+    return learner_fit(io, 1, minibatch, fit_batch, epochs, lr, &d_weights_out, nullptr, adam, (cudaStream_t)stream);
+}
+
+static int check_peers(const nfsp_peers *peers, int minibatch, int fit_batch) {
     NFSP_CHECK_ARG(peers && peers->world >= 2 && peers->world <= NFSP_MAX_PEERS && peers->rank >= 0 && peers->rank < peers->world,
                    "2..%d peers", NFSP_MAX_PEERS);
     NFSP_CHECK_ARG(peers->d_err, "null error word");
@@ -717,19 +883,56 @@ extern "C" int nfsp_learner_fit_peers(const nfsp_learner_io *io, int minibatch, 
     NFSP_CHECK_ARG(minibatch <= NFSP_FIT_ROWS_MAX_MINIBATCH && fit_batch <= NFSP_FIT_ROWS_MAX_STEP,
                    "the peer exchange lives in the row-parallel kernel: minibatch <= %d, fit_batch <= %d",
                    NFSP_FIT_ROWS_MAX_MINIBATCH, NFSP_FIT_ROWS_MAX_STEP);
-    return learner_fit(io, 1, minibatch, fit_batch, epochs, lr, &d_weights_out, peers, (cudaStream_t)stream);
+    return NFSP_OK;
+}
+
+extern "C" int nfsp_learner_fit_peers(const nfsp_learner_io *io, int minibatch, int fit_batch, int epochs, const float lr[4],
+                                      float *d_weights_out, const nfsp_peers *peers, void *stream) {
+    const int rc = check_peers(peers, minibatch, fit_batch);
+    if (rc != NFSP_OK) return rc;
+    return learner_fit(io, 1, minibatch, fit_batch, epochs, lr, &d_weights_out, peers, nullptr, (cudaStream_t)stream);
+}
+
+extern "C" int nfsp_learner_fit_peers_adam(const nfsp_learner_io *io, int minibatch, int fit_batch, int epochs,
+                                           const float lr[4], float *d_weights_out, const nfsp_peers *peers,
+                                           const nfsp_adam_state *adam, void *stream) {
+    NFSP_CHECK_ARG(adam, "null Adam state");
+    const int rc = check_peers(peers, minibatch, fit_batch);
+    if (rc != NFSP_OK) return rc;
+    return learner_fit(io, 1, minibatch, fit_batch, epochs, lr, &d_weights_out, peers, adam, (cudaStream_t)stream);
 }
 
 extern "C" int nfsp_learner_fit_runs(const nfsp_learner_io *io, int n_runs, int minibatch, int fit_batch, int epochs, const float *lr,
                                      float *const *d_weights_out, void *stream) {
     NFSP_CHECK_ARG(n_runs >= 1 && n_runs <= NFSP_MAX_RUNS, "n_runs must be in [1, %d]", NFSP_MAX_RUNS);
-    return learner_fit(io, n_runs, minibatch, fit_batch, epochs, lr, d_weights_out, nullptr, (cudaStream_t)stream);
+    return learner_fit(io, n_runs, minibatch, fit_batch, epochs, lr, d_weights_out, nullptr, nullptr, (cudaStream_t)stream);
+}
+
+extern "C" int nfsp_learner_fit_runs_adam(const nfsp_learner_io *io, int n_runs, int minibatch, int fit_batch, int epochs,
+                                          const float *lr, float *const *d_weights_out, const nfsp_adam_state *adam,
+                                          void *stream) {
+    NFSP_CHECK_ARG(n_runs >= 1 && n_runs <= NFSP_MAX_RUNS, "n_runs must be in [1, %d]", NFSP_MAX_RUNS);
+    NFSP_CHECK_ARG(adam, "null Adam state");
+    return learner_fit(io, n_runs, minibatch, fit_batch, epochs, lr, d_weights_out, nullptr, adam, (cudaStream_t)stream);
 }
 
 extern "C" int nfsp_sgd_apply(float *d_weights, const float *d_grad, const float lr[4], float scale, void *stream) {
     NFSP_CHECK_ARG(d_weights && d_grad && lr, "null argument");
     sgd_apply_kernel<<<(kGradFloats + 255) / 256, 256, 0, (cudaStream_t)stream>>>(d_weights, d_grad, lr[0], lr[1], lr[2],
                                                                                   lr[3], scale);
+    NFSP_LAUNCH_CHECK();
+    return NFSP_OK;
+}
+
+extern "C" int nfsp_adam_apply(float *d_weights, const float *d_grad, const float lr[4], float scale, int net_mask,
+                               const nfsp_adam_state *adam, void *stream) {
+    NFSP_CHECK_ARG(d_weights && d_grad && lr, "null argument");
+    NFSP_CHECK_ARG(net_mask >= 0 && net_mask <= 15, "net_mask must be in [0, 15]");
+    AdamRun M;
+    const int rc = make_adam_run(adam, M);
+    if (rc != NFSP_OK) return rc;
+    adam_apply_kernel<<<(kGradFloats + 255) / 256, 256, 0, (cudaStream_t)stream>>>(d_weights, d_grad, M, lr[0], lr[1], lr[2],
+                                                                                   lr[3], scale, net_mask);
     NFSP_LAUNCH_CHECK();
     return NFSP_OK;
 }

@@ -8,6 +8,9 @@ nets, gradients into one flat fp32 buffer with the exploitability statistics beh
 all-reduce of that buffer over the GPUs (NCCL; C1 + C2 of SURVEY 2a), one `nfsp_sgd_apply` launch.
 Weights therefore stay bit-identical on every rank.
 
+`optimizer="adam"` trains with Keras 2's Adam (beta1 0.9, beta2 0.999, epsilon 1e-7) instead of the reference's plain SGD,
+through the same paths: the `_adam` entries of the fit kernels and `nfsp_adam_apply` in place of `nfsp_sgd_apply`.
+
 What follows the reference literally (host arithmetic): the schedules of agent.py:245-253 per player
 (`iteration` advanced twice per update, temperature, BR learning-rate decay, each agent's own
 `epsilon ** 1/iteration` == epsilon/iteration by operator precedence) and the target-net copy every
@@ -33,6 +36,7 @@ from .batched import _ptr, _stream, check_fields, check_numbers, check_tensor
 
 GRAD = 4 * _lib.NET_PARAMS
 N_STATS = 8
+OPTIMIZERS = ("sgd", "adam")
 
 
 def _world():
@@ -42,7 +46,7 @@ def _world():
 class Learner:
     def __init__(self, selfplay, cfg=None, minibatch=128, fit_batch=32, epochs=2, lr_br=0.05, lr_ar=0.1, gamma=0.95,
                  target_update_rate=150, terminal_bootstraps=False, fused=True, use_multicast=True, others_to_target=False,
-                 peer_transport="auto", data_parallel=True):
+                 peer_transport="auto", data_parallel=True, optimizer="sgd"):
         if cfg is not None:
             minibatch = cfg.getint("Agent", "MiniBatchSize")
             lr_br, lr_ar = cfg.getfloat("Agent", "LearningRateBR"), cfg.getfloat("Agent", "LearningRateAR")
@@ -62,6 +66,15 @@ class Learner:
         # reference's `target = target_br_model.predict(s_batch)` does (agent.py:220,243)
         self.others_to_target = bool(others_to_target)
         self.fused = bool(fused)  # single GPU: the whole fit() as one kernel; False = one launch pair per SGD step
+        if optimizer not in OPTIMIZERS:
+            raise ValueError("optimizer must be one of %s, not %r" % (", ".join(OPTIMIZERS), optimizer))
+        self.optimizer = optimizer
+        if optimizer == "adam":
+            # Adam's state, per net as each Keras model has its own optimizer: the moments on the device (the kernels
+            # update them in place) and the steps taken (on the host, which knows every fit's mask and step count)
+            self.adam_m = torch.zeros((4, _lib.NET_PARAMS), dtype=torch.float32, device=self.device)
+            self.adam_v = torch.zeros((4, _lib.NET_PARAMS), dtype=torch.float32, device=self.device)
+            self.adam_t = [0, 0, 0, 0]
         self.target = selfplay.weights[[1, 3]].clone().contiguous()   # agent.py:70-72
         self.flat = torch.zeros(GRAD + N_STATS, dtype=torch.float32, device=self.device)
         self._peers = None
@@ -298,16 +311,48 @@ class Learner:
                                "invalid (NaN) and the replicas have diverged; resume the run from its last checkpoint "
                                "(main.py --resume DIR, with the --checkpoint DIR it was trained with)")
 
+    @property
+    def fit_steps(self) -> int:
+        """SGD (or Adam) steps of one fit: `epochs` passes over the minibatch in slices of `fit_batch` rows."""
+        return self.epochs * ((self.minibatch + self.fit_batch - 1) // self.fit_batch)
+
+    # ---- Adam's state ----
+    def adam_state(self, out=None):
+        """The nfsp_adam_state of this learner (moments and steps so far), written into `out` if given."""
+        s = _lib.AdamState() if out is None else out
+        s.d_m, s.d_v = self.adam_m.data_ptr(), self.adam_v.data_ptr()
+        for k in range(4):
+            s.t0[k] = self.adam_t[k]
+        return s
+
+    def _adam_advance(self, mask, steps):
+        """The nets in `mask` have taken `steps` more Adam steps (the others none: they did not move)."""
+        for k in range(4):
+            if (mask >> k) & 1:
+                self.adam_t[k] += steps
+
     # ---- the whole fit() in one launch: one GPU, or several with the all-reduce of every SGD step inside it ----
     def _fit_one_launch(self, idx_rl, idx_sl, mask, w_in=None, w_out=None):
         io, lr = self._fit_args(idx_rl, idx_sl, mask, w_in)
         args = (C.byref(io), self.minibatch, self.fit_batch, self.epochs, (C.c_float * 4)(*lr),
                 _ptr(self.sp.weights if w_out is None else w_out))
+        adam = self.optimizer == "adam"
         if self._peers is None:
+            if adam:
+                # the moments are updated in place on this stream.  Beside the pipelined trainer's next rollout that is
+                # safe: a rollout reads the acting images and the memories, never the learner's moments
+                check(lib().nfsp_learner_fit_adam(*args, C.byref(self.adam_state()), _stream(self.device)))
+                self._adam_advance(mask, self.fit_steps)
+                return
             return check(lib().nfsp_learner_fit(*args, _stream(self.device)))
         self._peers.epoch0 = self._epoch & 0xFFFFFFFF
-        check(lib().nfsp_learner_fit_peers(*args, C.byref(self._peers), _stream(self.device)))
-        self._epoch += self.epochs * ((self.minibatch + self.fit_batch - 1) // self.fit_batch)
+        if adam:
+            check(lib().nfsp_learner_fit_peers_adam(*args, C.byref(self._peers), C.byref(self.adam_state()),
+                                                    _stream(self.device)))
+            self._adam_advance(mask, self.fit_steps)
+        else:
+            check(lib().nfsp_learner_fit_peers(*args, C.byref(self._peers), _stream(self.device)))
+        self._epoch += self.fit_steps
 
     # ---- one SGD step for all four nets -------------------------------------------------------------
     def _step(self, idx_rl, idx_sl, row0, rows, mask):
@@ -318,6 +363,11 @@ class Learner:
         if world > 1:  # C1 (gradients) + C2 (exploitability stats) in one collective
             dist.all_reduce(self.flat, op=dist.ReduceOp.SUM)
         lr = (C.c_float * 4)(*lr)
+        if self.optimizer == "adam":
+            check(lib().nfsp_adam_apply(_ptr(sp.weights), _ptr(self.flat), C.byref(lr), 1.0 / world, mask,
+                                        C.byref(self.adam_state()), _stream(self.device)))
+            self._adam_advance(mask, 1)
+            return
         check(lib().nfsp_sgd_apply(_ptr(sp.weights), _ptr(self.flat), C.byref(lr), 1.0 / world, _stream(self.device)))
 
     def _ready_mask(self):
@@ -415,8 +465,11 @@ class Learner:
 
     # ---- checkpoint / resume (the SelfPlay it trains has its own state dict) ----
     def _shape(self):
-        return dict(minibatch=self.minibatch, fit_batch=self.fit_batch, epochs=self.epochs,
-                    terminal_bootstraps=self.terminal_bootstraps, others_to_target=self.others_to_target, fused=self.fused)
+        d = dict(minibatch=self.minibatch, fit_batch=self.fit_batch, epochs=self.epochs,
+                 terminal_bootstraps=self.terminal_bootstraps, others_to_target=self.others_to_target, fused=self.fused)
+        if self.optimizer != "sgd":  # an SGD learner's state is what it was before Adam existed: old checkpoints load
+            d["optimizer"] = self.optimizer
+        return d
 
     _SCALARS = dict(gamma=float, lr_br0=float, lr_ar=float, target_update_rate=int, iteration=(int, 2),
                     target_update_count=(int, 2), temp=(float, 2), lr_br=(float, 2), exploitability=(float, 2), updates=int)
@@ -430,12 +483,23 @@ class Learner:
         for k in self._SCALARS:
             v = getattr(self, k)
             d[k] = list(v) if isinstance(v, list) else v
+        if self.optimizer == "adam":
+            d.update(adam_m=self.adam_m.cpu(), adam_v=self.adam_v.cpu(), adam_t=list(self.adam_t))
         return d
 
     def check_state_dict(self, d):
         """Raises ValueError, naming the field, if load_state_dict(d) would refuse d."""
         check_fields(d, "Learner")
         check_fields(d.get("shape"), "Learner", **self._shape())
+        saved = d["shape"].get("optimizer", "sgd")
+        if saved != self.optimizer:  # check_fields does not see a shape key this learner lacks
+            raise ValueError("Learner: optimizer is %r in the state but %r here" % (saved, self.optimizer))
+        if self.optimizer == "adam":
+            for k in ("adam_m", "adam_v"):
+                check_tensor(d.get(k), k, "Learner", tuple(self.adam_m.shape), torch.float32)
+            check_numbers(d, "Learner", adam_t=(int, 4))
+            if any(t > 2 ** 62 for t in d["adam_t"]):  # nfsp_adam_state.t0 holds at most 2^62
+                raise ValueError("Learner: adam_t must be at most 2**62, got %r" % (d["adam_t"],))
         check_tensor(d.get("target"), "target", "Learner", tuple(self.target.shape), torch.float32)
         check_numbers(d, "Learner", **self._SCALARS)
         if d.get("loss") is not None:
@@ -448,6 +512,10 @@ class Learner:
         self.check_state_dict(d)
         torch.cuda.synchronize(self.device)
         self.target.copy_(d["target"])
+        if self.optimizer == "adam":
+            self.adam_m.copy_(d["adam_m"])
+            self.adam_v.copy_(d["adam_v"])
+            self.adam_t = list(d["adam_t"])
         for k, kind in self._SCALARS.items():
             setattr(self, k, list(d[k]) if isinstance(kind, tuple) else d[k])
         self.gamma, self.lr_br0, self.lr_ar = float(self.gamma), float(self.lr_br0), float(self.lr_ar)

@@ -42,7 +42,7 @@ from . import sharding, sweep
 from .batched import SelfPlay
 from .config import load_config
 from .exploitability import exploitability
-from .learner import Learner, PipelinedTrainer
+from .learner import OPTIMIZERS, Learner, PipelinedTrainer
 from .runs import RunBatch
 
 
@@ -58,6 +58,12 @@ def _is_report(calls, report_every):
 def _stopped(calls, report_every, hands, episodes):
     """Whether a run resumed at `calls` with `hands` played had stopped there: the loop ends at a report call."""
     return calls > 0 and _is_report(calls, report_every) and hands >= episodes
+
+
+def _mark_optimizer(row, learner):
+    """A reported row names the optimizer when it is not the reference's SGD (SGD rows stay as they always were)."""
+    if learner.optimizer != "sgd":
+        row["optimizer"] = learner.optimizer
 
 
 def sampled_actions(stats, player):
@@ -121,6 +127,7 @@ def train(sp: SelfPlay, learner: Learner, episodes: int, steps_per_call: int = 8
                "transitions_per_sec": (stats["transitions"] - tr0) / max(time.time() - t0, 1e-9)}
         if true_exploitability:
             row["exploitability"] = exploitability(sp)  # exact best response to the average policies (SURVEY 8 f-2)
+        _mark_optimizer(row, learner)
         rows.append(row)
         log("================ Stats ==================")
         for p in range(2):
@@ -173,6 +180,7 @@ def train_runs(rb: RunBatch, episodes: int, steps_per_call: int = 8, report_ever
             values = [r["exploitability"]["value"] for r in runs]
             row["exploitability_mean"] = statistics.fmean(values)
             row["exploitability_std"] = statistics.stdev(values) if len(values) > 1 else 0.0
+        _mark_optimizer(row, rb.learners[0])
         rows.append(row)
         log("================ Stats ==================")
         for k, run in enumerate(runs):
@@ -222,6 +230,8 @@ def _point_rows(run_rows, calls, true_exploitability):
             values = [r["exploitability"]["value"] for r in rs]
             row["exploitability_mean"] = statistics.fmean(values)
             row["exploitability_std"] = statistics.stdev(values) if len(values) > 1 else 0.0
+        if "optimizer" in rs[0]:
+            row["optimizer"] = rs[0]["optimizer"]
         out.append(row)
     return out
 
@@ -269,6 +279,7 @@ def train_sweep(rb: RunBatch, runs, record, episodes: int, steps_per_call: int =
                    "transitions_per_sec": (stats["transitions"] - tr0[k]) / dt}
             if true_exploitability:
                 row["exploitability"] = ex[k]
+            _mark_optimizer(row, rb.learners[k])
             mine.append(row)
         run_rows = [r for part in _gather(mine) for r in part]
         new = run_rows + _point_rows(run_rows, calls, true_exploitability)
@@ -325,6 +336,9 @@ def main(argv=None):
                          "section), --runs seeds each, as independent runs spread over all ranks" % ", ".join(sweep.RUN_KEYS))
     ap.add_argument("--results", metavar="FILE", default=None,
                     help="with --sweep: write every reported row of every run and grid point to FILE as JSON Lines")
+    ap.add_argument("--optimizer", default="sgd", choices=list(OPTIMIZERS),
+                    help="the learner's optimizer: the reference's plain SGD (default) or Keras 2's Adam, with the "
+                         "configured learning rates; every run of a sweep uses the same one")
     ap.add_argument("--checkpoint", metavar="DIR", default=None,
                     help="save the training state to DIR every --checkpoint-every rollout calls and when training ends")
     ap.add_argument("--checkpoint-every", type=int, default=CHECKPOINT_EVERY, metavar="CALLS",
@@ -377,7 +391,7 @@ def main(argv=None):
         return sp_, Learner(sp_, minibatch=cfg.getint("Agent", "MiniBatchSize"), lr_br=hp["LearningRateBR"],
                             lr_ar=hp["LearningRateAR"], gamma=hp["Gamma"], target_update_rate=hp["TargetModelUpdateRate"],
                             terminal_bootstraps=args.terminal_bootstraps, others_to_target=args.others_to_target,
-                            data_parallel=data_parallel)
+                            data_parallel=data_parallel, optimizer=args.optimizer)
 
     if runs is not None:   # no run is sharded: run i plays games 0 .. --games - 1 whatever the world size
         mine = [runs[i] for i in sweep.rank_runs(len(runs), rank, world)]

@@ -7,8 +7,9 @@ own env handle, memories, counters) plus the `Learner` that trains it -- and iss
 
     rollout(T)   one nfsp_rollout_runs launch for all runs (plus one image and one state-table launch when learners have
                  updated), then the inserts in groups of up to four memories (nfsp_insert_multi)
-    update()     one sampling launch for the 4R memories, one nfsp_learner_fit_runs launch (4R CTAs), then each learner's
-                 own host schedules (Learner._finish_update)
+    update()     one sampling launch for the 4R memories, one nfsp_learner_fit_runs launch (4R CTAs; with Adam learners
+                 nfsp_learner_fit_runs_adam, each run's moments and steps its own), then each learner's own host
+                 schedules (Learner._finish_update)
 
 Run r does exactly what it would do alone, bit for bit: games, records, memories, weights, schedules.
 """
@@ -30,7 +31,7 @@ def _selfplay_shape(sp):
 
 
 def _learner_shape(ln):
-    return (ln.minibatch, ln.fit_batch, ln.epochs, ln.terminal_bootstraps, ln.others_to_target, ln.fused)
+    return (ln.minibatch, ln.fit_batch, ln.epochs, ln.terminal_bootstraps, ln.others_to_target, ln.fused, ln.optimizer)
 
 
 class RunBatch:
@@ -38,7 +39,7 @@ class RunBatch:
 
     selfplays[r] is trained by learners[r].  The runs must share device, n_games, max_steps_per_call, the default
     ("states") rollout variant, direct_rings, deterministic, the memories' capacities and the learner's minibatch, fit
-    batch, epochs and flags; seeds, eta, epsilons and learning rates are each run's own.  One GPU only; with a process
+    batch, epochs, flags and optimizer; seeds, eta, epsilons and learning rates are each run's own.  One GPU only; with a process
     group of several ranks (a sweep, sweep.py) every learner must train alone (Learner(data_parallel=False))."""
 
     def __init__(self, selfplays, learners):
@@ -61,7 +62,7 @@ class RunBatch:
                 raise ValueError("run %d differs from run 0 in shape (device, games, steps per call, record mode, "
                                  "capacities)" % r)
             if _learner_shape(ln) != _learner_shape(lns[0]):
-                raise ValueError("run %d's learner differs from run 0's (minibatch, fit batch, epochs, flags)" % r)
+                raise ValueError("run %d's learner differs from run 0's (minibatch, fit batch, epochs, flags, optimizer)" % r)
             if not ln.fused:
                 raise ValueError("run %d: the batched update is the one-launch fit (fused=True)" % r)
         self.sps, self.learners = sps, lns
@@ -90,6 +91,7 @@ class RunBatch:
         self._learner_io = (_lib.LearnerIO * R)()
         self._lr = (C.c_float * (4 * R))()
         self._w_out = (C.c_void_p * R)()
+        self._adam = (_lib.AdamState * R)() if lns[0].optimizer == "adam" else None
 
     def rollout(self, n_steps=8):
         """SelfPlay.rollout(n_steps) of every run: one nfsp_rollout_runs call (rebuilding the weight images of the runs
@@ -145,8 +147,15 @@ class RunBatch:
             ln, pos = lns[r], self._pos[k]
             self._learner_io[k], self._lr[4 * k:4 * k + 4] = ln._fit_args([pos[0], pos[1]], [pos[2], pos[3]], masks[r])
             self._w_out[k] = sps[r].weights.data_ptr()
-        check(lib().nfsp_learner_fit_runs(self._learner_io, len(active), b, lns[0].fit_batch, lns[0].epochs, self._lr,
-                                          self._w_out, st))
+        fit = (self._learner_io, len(active), b, lns[0].fit_batch, lns[0].epochs, self._lr, self._w_out)
+        if self._adam is None:
+            check(lib().nfsp_learner_fit_runs(*fit, st))
+        else:
+            for k, r in enumerate(active):
+                lns[r].adam_state(self._adam[k])
+            check(lib().nfsp_learner_fit_runs_adam(*fit, self._adam, st))
+            for r in active:
+                lns[r]._adam_advance(masks[r], lns[r].fit_steps)
         out = list(out)
         for r in active:
             ln = lns[r]
